@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W            our arm  (libs3d_b200.so, hand-written sm_100a kernels)
     python bench.py --impl reference --gpus N --steps K ...  reference arm (the CPU oracle, -O3 -march=native, all host threads)
     python bench.py --workload c3 | c4 [...]                 BASELINE.json configs[2] / configs[3] as the headline line
+    python bench.py ... --dump-outputs DIR                   also writes what the last timed step returned as DIR/<name>.npy
 
 One "step" of the default workload (c2) = one call of s3d_gicp_align_batch on `--pairs` independent scan pairs
 (consecutive-scan odometry: voxel filter 0.1 m x2, NN grids, kNN-20 covariances x2, GICP loop, fitness, gates — the whole align()).
@@ -44,6 +45,29 @@ def make_pairs(n_distinct, seed0=SEED0, loop=False):
 def params():
     from slam3d_b200._abi import RegistrationParameters
     return RegistrationParameters.defaults(point_cloud_density=VOXEL)  # 2.5 m corr. distance, 50 iterations, default epsilons
+
+
+def dump_results(out_dir, results, prefix=""):
+    """--dump-outputs: the fields of the Result structs a caller of the timed call receives, one float64 array per field
+    (pose: (n, 4, 4), the others: (n,)), in the order of the pairs."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"pose": np.array([r.pose() for r in results], np.float64).reshape(-1, 4, 4)}
+    for name in ("fitness", "status", "converged", "outer_iterations", "inner_iterations", "n_source", "n_target", "n_correspondences"):
+        arrays[name] = np.array([getattr(r, name) for r in results], np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
+
+
+DUMP_MAX_ROWS = 1 << 20  # per dumped cloud: 16 MB of float32 xyzw
+
+
+def dump_cloud(out_dir, name, cloud):
+    """--dump-outputs for a point cloud: all rows up to DUMP_MAX_ROWS, beyond that a fixed, seeded sample of them (in order)."""
+    os.makedirs(out_dir, exist_ok=True)
+    cloud = np.asarray(cloud, np.float32)
+    if cloud.shape[0] > DUMP_MAX_ROWS:
+        cloud = cloud[np.sort(np.random.default_rng(0).choice(cloud.shape[0], DUMP_MAX_ROWS, replace=False))]
+    np.save(os.path.join(out_dir, name + ".npy"), cloud)
 
 
 def loop_params():
@@ -111,7 +135,7 @@ class ClockSampler:
 def _oracle_native():
     import oracle
     oracle.build()
-    how = oracle.use_native()  # compiles oracle/_native/ on this machine when missing; falls back to the portable build
+    how = oracle.use_native()  # compiles a -march=native build in a private temporary directory; falls back to the portable build
     return oracle, how
 
 
@@ -139,13 +163,13 @@ def run_reference(args, rank, world):
         step()
     t0 = time.perf_counter()
     done = 0
-    steps = max(1, args.steps)
-    for i in range(steps):
-        done += len(step())
-        if time.perf_counter() - t0 > 120:
-            steps = i + 1
-            break
+    steps = args.steps
+    for _ in range(steps):
+        last = step()
+        done += len(last)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_results(args.dump_outputs, last, "fine_" if loop else "")
     value = done / dt
     metric, unit = (METRIC, UNIT) if not loop else ("loop_closure_constraints_per_s_256_pairs", "constraints/s")
     wl = ("256 synthetic loop-closure candidate pairs (131072 points), coarse 0.5 m / 5 m then fine 0.1 m GICP (BASELINE.json configs[3])" if loop
@@ -201,7 +225,12 @@ def main():
     ap.add_argument("--no-chain", action="store_true", help="skip the supplementary odometry-chain measurement (device cache)")
     ap.add_argument("--no-extras", action="store_true", help="skip the supplementary config 3 / config 4 / latency / in-process measurements")
     ap.add_argument("--scene-rank", type=int, default=-1, help="experiment: another set of scenes (seed offset 1000 R), to see the cost spread between scene sets")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (rank 0; inputs are seeded, so two builds compare output for output). "
+                         "--impl reference runs min(host threads, 64) pairs per step, not --pairs: compare its dumps with reference dumps")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -319,6 +348,8 @@ def main():
         for _ in range(max(args.warmup, 3)):
             ctx.gicp_align_batch(dev_src, dev_tgt, None, p)
         ev_ms, wall_ms, cnt, last = timed(dev_src, dev_tgt, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_results(args.dump_outputs, last)
     value = world * B * args.steps / (wall_ms / 1e3)
     rank_ms_value = list(rank_ms)  # of the device-resident timed region (later timed() calls overwrite rank_ms)
     ok = sum(1 for r in last if r.status == _abi.S3D_OK)
@@ -507,7 +538,7 @@ def bench_c3(ctx, peak, peak_src, args, headline):
     was = True
     ctx.set_profiling(True)
     res = {}
-    n = 10
+    n = args.steps if headline else 10
     for leaf in (0.05, 0.1, 0.2):
         for _ in range(3):
             out, _, _ = ctx.voxel_downsample(dev, leaf, want_leaf_index=False)
@@ -515,6 +546,8 @@ def bench_c3(ctx, peak, peak_src, args, headline):
         for _ in range(n):
             out, _, _ = ctx.voxel_downsample(dev, leaf, want_leaf_index=False)
         st = ctx.stage_times(reset=True)
+        if headline and args.dump_outputs:
+            dump_cloud(args.dump_outputs, f"voxel_leaf_{leaf}", out)
         ms = st["voxel"]["ms"] / n
         m = out.shape[0]
         algo = 16.0 * cloud.shape[0] + 16.0 * m   # SURVEY 8d: 16 B per input point read + 16 B per voxel written
@@ -567,13 +600,16 @@ def bench_c4(ctx, args, rank, world, n_dev, headline, barrier):
     truth = [pinned[i % len(pinned)][2] for i in range(lo, hi)]
     coarse, fine = loop_params()
     ctx.gicp_align_loop_batch(srcs, tgts, None, coarse, fine)
-    steps = max(1, min(args.steps, 3))
+    steps = args.steps if headline else max(1, min(args.steps, 3))
     barrier()
     t0 = time.perf_counter()
     for _ in range(steps):
         rc, rf = ctx.gicp_align_loop_batch(srcs, tgts, None, coarse, fine)
     barrier()
     dt = sharding.max_over_ranks(time.perf_counter() - t0, device="cuda") / steps
+    if headline and args.dump_outputs and rank == 0:
+        dump_results(args.dump_outputs, rc, "coarse_")
+        dump_results(args.dump_outputs, rf, "fine_")
     okf = [r.status == _abi.S3D_OK for r in rf]
     err = [float(np.linalg.norm((np.linalg.inv(T) @ r.pose())[:3, 3])) for r, T, good in zip(rf, truth, okf) if good]
     res = {"constraints_per_s": total / dt, "aligns_per_s": 2 * total / dt, "ms_per_256_pairs": 1e3 * dt, "pairs_this_rank": hi - lo,

@@ -1,7 +1,7 @@
 """CPU prototype (numpy + cKDTree): what a warp-cooperative TILE kNN would have to scan on the bench clouds — group sizes, shared
 candidate-set sizes and the share of queries whose k-th neighbour such a tile cannot certify.  Result: profiles/r02_summary.md."""
-import sys, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import oracle
 from slam3d_b200 import synth
 from scipy.spatial import cKDTree

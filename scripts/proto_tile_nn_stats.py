@@ -1,7 +1,7 @@
 """CPU prototype: bounding boxes of 32 Morton-consecutive transformed queries in the fixed cloud's grid — what a shared-candidate 1-NN
 tile would have to load.  Result: profiles/r02_summary.md."""
-import sys, numpy as np
-sys.path.insert(0, '/root/repo')
+import os, sys, numpy as np
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import oracle
 from slam3d_b200 import synth
 from scipy.spatial import cKDTree

@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Regenerates tests/golden/ from the reference's test data (run in the build container only).
+"""Regenerates tests/golden/ from the reference's test data:  python make_golden.py <slam3d checkout>/test
 
-Inputs : /root/reference/test/cloud{1..4}.bin  (KITTI-format float32 x,y,z,intensity; SURVEY Appendix B).
-Outputs: tests/golden/cloud{1..4}.xyz.f32.xz   xyz float32, lzma — the reference DATA travels with the repo
-                                               because /root/reference does not exist on the GPU box;
+Inputs : <dir>/cloud{1..4}.bin                 (KITTI-format float32 x,y,z,intensity; SURVEY Appendix B).
+Outputs: tests/golden/cloud{1..4}.xyz.f32.xz   xyz float32, lzma — the reference DATA travels with the repo,
+                                               so that the tests need nothing outside it;
          tests/golden/golden.json              frozen outputs of the CPU oracle (oracle/s3d_oracle.cpp) on them.
 
 The reference has no expected outputs for this path (SURVEY 8c), so golden.json pins the ORACLE (regression) and
@@ -22,17 +22,15 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
 import oracle  # noqa: E402
 from slam3d_b200._abi import RegistrationParameters  # noqa: E402
 
-REF = "/root/reference/test"
-
 
 def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-def main():
+def main(ref):
     clouds = []
     for i in range(1, 5):
-        raw = np.fromfile(os.path.join(REF, f"cloud{i}.bin"), np.float32).reshape(-1, 4)
+        raw = np.fromfile(os.path.join(ref, f"cloud{i}.bin"), np.float32).reshape(-1, 4)
         xyz = np.ascontiguousarray(raw[:, :3])
         with open(os.path.join(HERE, f"cloud{i}.xyz.f32.xz"), "wb") as f:
             f.write(lzma.compress(xyz.tobytes(), preset=9))
@@ -106,4 +104,9 @@ def add_map_only():
 
 
 if __name__ == "__main__":
-    add_map_only() if "--map" in sys.argv else main()
+    if "--map" in sys.argv:
+        add_map_only()
+    elif len(sys.argv) == 2:
+        main(sys.argv[1])
+    else:
+        sys.exit(__doc__)
