@@ -145,6 +145,18 @@ int s3d_gicp_align_loop_batch(s3d_context* ctx, const s3d_cloud* sources, const 
                               const s3d_registration_parameters* coarse, const s3d_registration_parameters* fine, int n_pairs,
                               s3d_result* out_coarse, s3d_result* out_fine);
 
+/* Inner optimiser of PCL's GICP (estimateRigidTransformation*), the one step in which PCL versions differ:
+ *   S3D_GICP_NEWTON  estimateRigidTransformationNewton, PCL >= 1.14's default (back-tracking Newton; the default here)
+ *   S3D_GICP_BFGS    estimateRigidTransformationBFGS, the only optimiser of PCL 1.8.1 ... 1.13 (pcl/registration/bfgs.h, GSL's
+ *                    vector_bfgs2 with Fletcher's line search).  About 10x the evaluation passes of Newton (DESIGN.md 4).
+ * The setting belongs to the context, not to s3d_registration_parameters (which mirrors slam3d's struct field for field): it is a
+ * property of the PCL a build replaces.  It applies to every GICP (and GICP_OMP) entry point — s3d_gicp_align, _batch,
+ * _loop_batch (coarse and fine), _prepared, _prepared_batch — and NDT ignores it; prepared clouds serve both.  Calls that start
+ * after it returns use the new setting: change it while no call is running on the context.  `previous` (may be NULL) receives the
+ * setting it replaces.  Any other value returns S3D_INVALID_ARGUMENT and changes nothing. */
+enum { S3D_GICP_NEWTON = 0, S3D_GICP_BFGS = 1 };
+int s3d_set_gicp_optimizer(s3d_context* ctx, int optimizer, int* previous);
+
 /* ---- stage-level entry points (used by the parity tests and the bench; same kernels as align) ---------- */
 
 /* GICP computeCovariances (SURVEY A.3): exact kNN (k neighbours, self included, ascending (d2, index)),

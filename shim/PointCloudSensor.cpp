@@ -35,6 +35,9 @@ s3d_context* gpu() {
   static s3d_context* ctx = [] {
     s3d_context* c = nullptr;
     if (s3d_create_context(nullptr, 0, &c) != S3D_OK) throw std::runtime_error(s3d_last_error());
+#ifdef S3D_GICP_USE_BFGS  // built against PCL < 1.14 (shim/CMakeLists.txt): GICP runs that PCL's BFGS inner optimiser
+    if (s3d_set_gicp_optimizer(c, S3D_GICP_BFGS, nullptr) != S3D_OK) throw std::runtime_error(s3d_last_error());
+#endif
     return c;
   }();
   return ctx;

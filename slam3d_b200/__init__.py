@@ -38,6 +38,7 @@ def lib():
         L.s3d_set_input_stream.argtypes = [C.c_void_p, C.c_void_p, C.c_int]
         L.s3d_get_loop_stats.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]
         L.s3d_set_profiling.argtypes = [C.c_void_p, C.c_int]
+        L.s3d_set_gicp_optimizer.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.s3d_get_stage_times.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.s3d_voxel_downsample.argtypes = [C.c_void_p, Cloud, C.c_float, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p, C.POINTER(C.c_int32)]
         L.s3d_knn_covariances.argtypes = [C.c_void_p, Cloud, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -140,6 +141,16 @@ class Context:
         n = (C.c_uint64 * 6)()
         lib().s3d_get_stage_times(self._h, ms, n, int(reset))
         return {k: {"ms": ms[i], "launches": int(n[i])} for i, k in enumerate(self.STAGES)}
+
+    def set_gicp_optimizer(self, which):
+        """Inner optimiser of every GICP registration on this context: "newton" (estimateRigidTransformationNewton, PCL >= 1.14's
+        default; the default here) or "bfgs" (estimateRigidTransformationBFGS, the only one of PCL 1.8.1 ... 1.13).  NDT ignores
+        it.  Change it while no call is running on the context.  Returns the previous setting."""
+        if which not in _abi.GICP_OPTIMIZERS:
+            raise ValueError(f"GICP optimizer must be one of {sorted(_abi.GICP_OPTIMIZERS)}, not {which!r}")
+        prev = C.c_int(0)
+        self._check(lib().s3d_set_gicp_optimizer(self._h, _abi.GICP_OPTIMIZERS[which], C.byref(prev)), "s3d_set_gicp_optimizer")
+        return "bfgs" if prev.value == _abi.GICP_BFGS else "newton"
 
     def loop_stats(self, reset=False):
         t, c = C.c_uint64(0), C.c_uint64(0)

@@ -11,6 +11,10 @@ S3D_INVALID_ARGUMENT = 6
 
 ALG_ICP, ALG_GICP, ALG_GICP_OMP, ALG_NDT, ALG_NDT_OMP = range(5)
 
+# s3d_set_gicp_optimizer: the inner optimiser of PCL's GICP (PCL >= 1.14 default / PCL <= 1.13)
+GICP_NEWTON, GICP_BFGS = 0, 1
+GICP_OPTIMIZERS = {"newton": GICP_NEWTON, "bfgs": GICP_BFGS}
+
 
 class RegistrationParameters(C.Structure):
     """slam3d::RegistrationParameters (RegistrationParameters.hpp:36-97), field for field."""

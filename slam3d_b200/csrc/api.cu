@@ -107,6 +107,7 @@ struct s3d_context {
   int streams_small = 3;
   cudaStream_t input_stream = nullptr;  // s3d_set_input_stream: device-pointer inputs are produced on this stream
   bool have_input_stream = false;
+  std::atomic<int> gicp_optimizer{S3D_GICP_NEWTON};  // s3d_set_gicp_optimizer
   s3d::WorkerPool pool;
   // n workers through the pool, or through threads of the call's own when another batch call holds the pool
   void parallel(int n, const std::function<void(int)>& f) {
@@ -145,6 +146,7 @@ struct WsLease {
     }
     if (!ws) { ws.reset(new Workspace()); ws->init(dc->device); std::lock_guard<std::mutex> g(dc->mu); dc->all.push_back(ws.get()); }
     ws->profiling = ctx->profiling;
+    ws->gicp_optimizer = ctx->gicp_optimizer.load();
     static const bool gate_enabled = [] { const char* e = getenv("S3D_GATE_UPLOADS"); return !e || atoi(e) != 0; }();  // 0: A/B measurements
     ws->upload_gate = (t_gate_uploads && gate_enabled) ? &dc->upload_mu : nullptr;
     static const bool blocking_enabled = [] { const char* e = getenv("S3D_BLOCKING_SYNC"); return !e || atoi(e) != 0; }();  // 0: A/B measurements
@@ -406,6 +408,17 @@ int s3d_set_input_stream(s3d_context* ctx, void* stream, int enabled) {
   std::lock_guard<std::mutex> g(ctx->mu);
   ctx->input_stream = static_cast<cudaStream_t>(stream);
   ctx->have_input_stream = enabled != 0;
+  return S3D_OK;
+}
+
+int s3d_set_gicp_optimizer(s3d_context* ctx, int optimizer, int* previous) {
+  if (!ctx) return S3D_INVALID_ARGUMENT;
+  if (optimizer != S3D_GICP_NEWTON && optimizer != S3D_GICP_BFGS) {
+    set_error("GICP optimizer must be S3D_GICP_NEWTON (0) or S3D_GICP_BFGS (1)");
+    return S3D_INVALID_ARGUMENT;
+  }
+  const int old = ctx->gicp_optimizer.exchange(optimizer);
+  if (previous) *previous = old;
   return S3D_OK;
 }
 

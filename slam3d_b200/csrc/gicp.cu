@@ -11,9 +11,10 @@
 //                                 (FP64, stored) -> the 74 sums of gicp_math.h per tile in a fixed order: 60 x-independent sums
 //                                 that give the whole Hessian, and the 13 residual sums + count of PCL's first objective evaluation
 //   control step  (ctrl_step)     fixed-order sum of the tile partials, then ONE thread advances PCL's inner optimiser
-//                                 (estimateRigidTransformationNewton as a resumable state machine, pair state staged in shared
-//                                 memory) to its next objective evaluation, or finishes the outer iteration (convergence test)
-//   trial pass    (eval_tile)     f at the pending back-tracking trial(s): one pass over the stored correspondences with the
+//                                 (estimateRigidTransformationNewton, or per context the BFGS one of PCL <= 1.13, as a resumable
+//                                 state machine, pair state staged in shared memory) to its next objective evaluation, or
+//                                 finishes the outer iteration (convergence test)
+//   trial pass    (eval_tile)     f (and its gradient) at the pending back-tracking / line-search trial(s): one pass over the stored correspondences with the
 //                                 residual formed exactly as PCL forms it (float32 T(x)*p, float subtraction) -> 13 sums per tile
 //   fitness pass  (fitness_tile)  getFitnessScore once the outer loop has ended; its last tile closes the pair
 // While one pair sits in its (serial, ~10 us) control step the CTAs work on tiles of the other pairs; a CTA that finds nothing
@@ -89,10 +90,19 @@ __device__ void mat4f_mul(const float* A, const float* B, float* C) {
                                __fmul_rn(A[12 + r], B[c * 4 + 3]));
 }
 
+__device__ __noinline__ void bfgs_begin_outer(PairState& ps) {  // out of line: the Newton path does not carry it
+  bfgs_begin(ps.bst, ps.T);
+  matrix_from_state(ps.bst.xc, ps.T_eval);
+}
+
 // start of an outer iteration: x0 from transformation_, the float matrix PCL's first evaluation uses, and R for the Mahalanobis matrices
 __device__ void begin_outer(PairState& ps) {
-  newton_begin(ps.nst, ps.T);
-  matrix_from_state(ps.nst.xc, ps.T_eval);
+  if (ps.optimizer == S3D_GICP_BFGS) {
+    bfgs_begin_outer(ps);
+  } else {
+    newton_begin(ps.nst, ps.T);
+    matrix_from_state(ps.nst.xc, ps.T_eval);
+  }
   update_rotation(ps);
   ps.phase = kPhaseNeedNN;
 }
@@ -353,14 +363,15 @@ __device__ __forceinline__ void fitness_tile(const GicpArgs& a, const PairState&
 }
 
 // End of an outer iteration (computeTransformation, SURVEY A.4): convergence test, counters, next iteration or final transform.
-__device__ void finish_outer(PairState& ps, bool optimiser_failed) {
+// x, inner: the inner optimiser's result state and iteration count.
+__device__ void finish_outer(PairState& ps, bool optimiser_failed, const double* x, int inner) {
   bool stop = false;
   if (optimiser_failed) {
     ps.failed = 1; ps.converged = 0; stop = true;  // optimiser exception: loop breaks, converged_ stays false, final = previous * guess
   } else {
     float T[16];
-    matrix_from_state(ps.nst.x, T);  // transformation_matrix.setIdentity(); applyState(transformation_matrix, x)
-    ps.inner_iterations += ps.nst.it;
+    matrix_from_state(x, T);  // transformation_matrix.setIdentity(); applyState(transformation_matrix, x)
+    ps.inner_iterations += inner;
     double delta = 0.0;
     for (int r = 0; r < 4; ++r)
       for (int c = 0; c < 4; ++c) {
@@ -411,6 +422,22 @@ __device__ void euler_derivs_cta(const double* x, Euler& E, double (*fac)[3][3][
 // Control step of pair p, run by the CTA that delivered the last tile of a search or trial pass: ordered reduction of the tile
 // partials, then the optimiser advances.  The pair state is staged in shared memory (the serial part is one thread's dependent
 // chain; on global memory every step of it was an L2 round trip: 29 us per control launch in round 1).
+// BFGS mode (PCL <= 1.13): f and the gradient at the pending state (sums 60..73, gradient entries gH[0..5]) advance the line
+// search to its next trial, which becomes the single trial T_trial[0] of the next pass, or end the solve.  Out of line: the
+// Newton path of the loop kernel does not carry its registers.
+__device__ __noinline__ void bfgs_ctrl(PairState& ps, const double* gH) {
+  double g[6];
+  for (int i = 0; i < 6; ++i) g[i] = gH[i];
+  if (bfgs_advance(ps.bst, ps.sums[72] / ps.sums[73], g, ps.max_inner)) {
+    matrix_from_state(ps.bst.xc, ps.T_trial[0]);
+    ps.trial_first = 0; ps.trial_count = 1;
+    ps.phase = kPhaseEval;
+  } else {
+    if (ps.bst.failed) ps.inner_iterations += ps.bst.it;  // estimateRigidTransformationBFGS has counted them before it throws
+    finish_outer(ps, ps.bst.failed != 0, ps.bst.x, ps.bst.it);
+  }
+}
+
 struct CtrlShared {
   PairState ps;
   double part[3][kLineSearchTrials * kEvalSums];
@@ -467,7 +494,9 @@ __device__ __forceinline__ void ctrl_step_body(const GicpArgs& a, uint32_t p, in
       for (int i = 0; i < kNumMoments; ++i) ps.sums[i] = sh.red[i];
       ps.n_corr = (uint32_t)ps.sums[73];
       for (int i = 0; i < 16; ++i) { ps.prev[i] = ps.T[i]; ps.T_search[i] = ps.T[i]; }  // previous_transformation_ = transformation_
-      if (ps.sums[73] < 4.0) { finish_outer(ps, true); sh.mode = 0; }  // min_number_correspondences_: PCL throws
+      if (ps.sums[73] < 4.0) { finish_outer(ps, true, ps.nst.x, 0); sh.mode = 0; }  // min_number_correspondences_: PCL throws
+    } else if (ps.optimizer == S3D_GICP_BFGS) {
+      for (int i = 0; i < kEvalSums; ++i) ps.sums[60 + i] = sh.red[i];  // the single pending line-search trial
     } else {
       double f_trial[kLineSearchTrials];
       for (int j = 0; j < ps.trial_count; ++j) f_trial[ps.trial_first + j] = sh.red[j * kEvalSums + 12] / ps.sums[73];
@@ -480,18 +509,20 @@ __device__ __forceinline__ void ctrl_step_body(const GicpArgs& a, uint32_t p, in
         sh.mode = 0;
       } else {
         ps.nst.phase = 2;  // no improvement found
-        finish_outer(ps, false);
+        finish_outer(ps, false, ps.nst.x, ps.nst.it);
         sh.mode = 0;
       }
     }
   }
   __syncthreads();
   if (sh.mode) {
-    euler_derivs_cta(ps.nst.xc, sh.E, sh.fac);
+    euler_derivs_cta(ps.optimizer == S3D_GICP_BFGS ? ps.bst.xc : ps.nst.xc, sh.E, sh.fac);
     // objective at the evaluated state: 42 threads contract one gradient / Hessian entry each
     if (threadIdx.x < 42) sh.gH[threadIdx.x] = objective_entry(ps.sums, sh.E, threadIdx.x);
     __syncthreads();
-    if (threadIdx.x == 0) {
+    if (threadIdx.x == 0 && ps.optimizer == S3D_GICP_BFGS) {
+      bfgs_ctrl(ps, sh.gH);
+    } else if (threadIdx.x == 0) {
       double g[6], H[6][6];
       for (int i = 0; i < 6; ++i) { g[i] = sh.gH[i]; for (int j = 0; j < 6; ++j) H[i][j] = sh.gH[6 + 6 * i + j]; }
       if (newton_advance_pre(ps.nst, ps.sums[72] / ps.sums[73], g, H, ps.max_inner)) {
@@ -499,7 +530,7 @@ __device__ __forceinline__ void ctrl_step_body(const GicpArgs& a, uint32_t p, in
         ps.phase = kPhaseEval;
         sh.newstep = 1;
       } else {
-        finish_outer(ps, false);
+        finish_outer(ps, false, ps.nst.x, ps.nst.it);
       }
     }
     __syncthreads();
@@ -893,6 +924,7 @@ void run_gicp(Workspace& ws, const std::vector<s3d_registration_parameters>& par
     ps.fit_range = cfg.max_correspondence_distance;
     ps.pt_off = ws.pair_off[p];
     ps.max_iter = cfg.maximum_iterations; ps.max_inner = cfg.maximum_optimizer_iterations; ps.k = cfg.correspondence_randomness;
+    ps.optimizer = ws.gicp_optimizer;
   }
   S3D_CUDA(cudaMemcpyAsync(ws.pairs.p, hp, sizeof(PairState) * np, cudaMemcpyHostToDevice, st));
   const SlotInfo* slots = ws.slots.as<SlotInfo>();

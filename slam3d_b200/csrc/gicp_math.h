@@ -5,7 +5,8 @@
 //     Newton step of estimateRigidTransformationNewton;
 //   * the GICP objective f(x) = 1/m sum d^T M d, d = T(x) p - q, its exact gradient and Hessian in the
 //     (t, ZYX-Euler) parametrisation, assembled from 74 sums of one pass over the correspondences, and PCL's inner
-//     Newton optimiser as a resumable state machine (one yield per objective evaluation).
+//     optimisers as resumable state machines (one yield per objective evaluation): the Newton one of PCL >= 1.14 here, the
+//     BFGS one of PCL <= 1.13 in gicp_bfgs.h (included at the end).
 //
 // B200-first design note: of the 74 sums, 60 (sum M (x) phi phi^T, phi = (p,1)) do not depend on x and give the whole
 // Hessian except its second-derivative term; an evaluation pass only adds the 13 sums that contain the residual d.
@@ -308,3 +309,5 @@ S3D_HD void mahalanobis6(const double (&RRt)[3][3], const double a[3], const dou
 }
 
 }  // namespace s3d
+
+#include "gicp_bfgs.h"

@@ -72,10 +72,15 @@ struct PairState {
   double fit_sum;
   uint32_t fit_n;
   int32_t max_iter, max_inner, k;
-  NewtonState nst;         // resumable inner optimiser (gicp_math.h)
+  int32_t optimizer;       // S3D_GICP_NEWTON / S3D_GICP_BFGS: which inner optimiser runs (the context's setting)
+  union {                  // resumable inner optimiser: one at a time, so they share storage
+    NewtonState nst;       // PCL >= 1.14 estimateRigidTransformationNewton (gicp_math.h)
+    BfgsState bst;         // PCL <= 1.13 estimateRigidTransformationBFGS (gicp_bfgs.h)
+  };
   float  T_eval[16];       // float matrix of the outer iteration's start state x0 (PCL applyState), evaluated by the search pass
   float  T_trial[kLineSearchTrials][16];  // float matrices of the back-tracking trials x - 2^-j delta of the current Newton step
-  int32_t trial_first, trial_count;       // trials the next evaluation pass has to cover (0,1 first; 1,9 if trial 0 failed)
+                                          // (BFGS: T_trial[0] is the one pending line-search trial x0 + alpha p)
+  int32_t trial_first, trial_count;       // trials the next evaluation pass has to cover (0,1 first; 1,9 if trial 0 failed; BFGS: 0,1)
   double sums[kNumMoments];// reduced sums of the current correspondence set (static part) + last evaluation (residual part)
   int32_t phase;           // kPhaseNeedNN / kPhaseEval / kPhaseFitness / kPhaseFinished
   int32_t active;          // 1 while the outer loop runs
@@ -141,6 +146,7 @@ struct Workspace {
   std::map<float, float> learned_frac;        // leaf size -> what the last raw-cloud batch with that leaf showed (+ margin)
   float batch_leaf = 0.f;                     // leaf size of the current batch (set by run_voxel)
   float grid_frac = 1.f;                      // what the current batch uses (1 for prepared clouds: their sizes are exact)
+  int gicp_optimizer = S3D_GICP_NEWTON;       // inner optimiser of the GICP loop: the context's setting at the time the workspace was leased
   // after a batch: `hs` = the slot table read back from the device
   void learn_grid_frac(const SlotInfo* hs, uint32_t ns) {
     if (!(batch_leaf > 0.f)) return;

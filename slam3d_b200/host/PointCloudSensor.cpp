@@ -14,6 +14,9 @@ s3d_context* defaultContext() {
   static std::string err;
   std::call_once(once, [] {
     status = s3d_create_context(nullptr, 0, &ctx);
+#ifdef S3D_GICP_USE_BFGS  // built against PCL < 1.14 (shim/CMakeLists.txt): GICP runs that PCL's BFGS inner optimiser
+    if (status == S3D_OK) status = s3d_set_gicp_optimizer(ctx, S3D_GICP_BFGS, nullptr);
+#endif
     if (status != S3D_OK) err = s3d_last_error();
   });
   if (!ctx) throw std::runtime_error("slam3d_b200: cannot create CUDA context: " + err);
