@@ -196,16 +196,35 @@ int s3d_get_loop_stats(s3d_context* ctx, uint64_t* tiles, uint64_t* control_step
  * (H2D, voxel filter at `density`, NN grid, kNN-k covariances) and keeps the result on the device;
  * s3d_gicp_align_prepared(_batch) then runs only the GICP loop + fitness + gates.  Results are bit-identical to
  * s3d_gicp_align on the raw clouds with point_cloud_density == density and correspondence_randomness == k
- * (status 6 if the handle was prepared with other values).  Handles are immutable and may be shared by threads. */
+ * (status 6 if the handle was prepared with other values).  Handles are immutable and may be shared by threads.
+ * s3d_prepare_cloud_ndt does the same for the NDT branch: voxel filter, NN grid and the VoxelGridCovariance at `resolution`
+ * that doNDT builds for its target (PointCloudSensor.cpp:84-117); the handle holds no normals. */
 typedef struct s3d_prepared_cloud s3d_prepared_cloud;
 int s3d_prepare_cloud(s3d_context* ctx, int device_slot, s3d_cloud cloud, double density, int k, s3d_prepared_cloud** out);
 /* n clouds in one pass (same result as n calls of s3d_prepare_cloud; out receives n handles, all-or-nothing). */
 int s3d_prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k,
                        s3d_prepared_cloud** out);
+/* n clouds in one pass: voxel filter at `density`, NN grid, and the NDT VoxelGridCovariance at `resolution`.  All-or-nothing like
+ * s3d_prepare_clouds.  resolution <= 0 or not finite, a NaN density or a bad device slot: S3D_INVALID_ARGUMENT and no handle.
+ * A cloud whose grid is not searchable (no finite point, PCL's int32 voxel-count guard) still gets a handle; an align on it
+ * ends like the raw call ("Voxel grid is not searchable": not converged, identity pose). */
+int s3d_prepare_clouds_ndt(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, float resolution,
+                           s3d_prepared_cloud** out);
+int s3d_prepare_cloud_ndt(s3d_context* ctx, int device_slot, s3d_cloud cloud, double density, float resolution,
+                          s3d_prepared_cloud** out);
 int s3d_release_cloud(s3d_context* ctx, s3d_prepared_cloud* cloud);
 uint64_t s3d_prepared_cloud_size(const s3d_prepared_cloud* cloud); /* points after filtering */
-/* Prepared clouds carry GICP data (Morton-sorted points, normals, NN grid); an NDT request on them returns
- * S3D_UNKNOWN_ALGORITHM with a message pointing at s3d_gicp_align(_batch), which voxelises the filtered source itself. */
+/* Device blocks of prepared clouds since context creation, over all devices: obtained from cudaMalloc, and reused from
+ * released handles (s3d_release_cloud hands a block back to its device; a later prepare takes it when it fits). */
+int s3d_get_prepared_block_stats(s3d_context* ctx, uint64_t* allocated, uint64_t* reused);
+/* Align on prepared clouds; the algorithm comes from params->registration_algorithm as in s3d_gicp_align.
+ *   GICP / GICP_OMP  both handles from s3d_prepare_cloud(s) with k == correspondence_randomness (an NDT handle: status 6).
+ *   NDT / NDT_OMP    the source (the scan whose grid NDT matches against) from s3d_prepare_cloud(s)_ndt with
+ *                    resolution == params->resolution (compared as floats; another value: status 6).  The target is read as
+ *                    points only, so a GICP handle of the same density serves too.  A pair whose source is a GICP handle ends
+ *                    with S3D_UNKNOWN_ALGORITHM (S3D_TOO_FEW_POINTS under 100 points), as before NDT handles existed.
+ * Every handle must match point_cloud_density (status 6 otherwise).  Results are bit-identical to s3d_gicp_align(_batch) on the
+ * raw clouds with the same parameters. */
 int s3d_gicp_align_prepared(s3d_context* ctx, const s3d_prepared_cloud* source, const s3d_prepared_cloud* target,
                             const double guess[16], const s3d_registration_parameters* params, s3d_result* out);
 int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* const* sources,

@@ -55,8 +55,11 @@ def lib():
         L.s3d_create_combined_measurement.argtypes = [C.c_void_p, C.POINTER(Cloud), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]
         L.s3d_prepare_cloud.argtypes = [C.c_void_p, C.c_int, Cloud, C.c_double, C.c_int, C.POINTER(C.c_void_p)]
         L.s3d_prepare_clouds.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.c_double, C.c_int, C.POINTER(C.c_void_p)]
+        L.s3d_prepare_cloud_ndt.argtypes = [C.c_void_p, C.c_int, Cloud, C.c_double, C.c_float, C.POINTER(C.c_void_p)]
+        L.s3d_prepare_clouds_ndt.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.c_double, C.c_float, C.POINTER(C.c_void_p)]
         L.s3d_release_cloud.argtypes = [C.c_void_p, C.c_void_p]
         L.s3d_prepared_cloud_size.restype = C.c_uint64
+        L.s3d_get_prepared_block_stats.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64)]
         L.s3d_prepared_cloud_size.argtypes = [C.c_void_p]
         L.s3d_gicp_align_prepared.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RegistrationParameters), C.POINTER(Result)]
         L.s3d_gicp_align_prepared_batch.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_void_p,
@@ -157,6 +160,12 @@ class Context:
         lib().s3d_get_loop_stats(self._h, C.byref(t), C.byref(c), int(reset))
         return {"tiles": t.value, "control_steps": c.value}
 
+    def prepared_block_stats(self):
+        """Device blocks of prepared clouds since context creation: from cudaMalloc, and reused from released handles."""
+        a, r = C.c_uint64(0), C.c_uint64(0)
+        self._check(lib().s3d_get_prepared_block_stats(self._h, C.byref(a), C.byref(r)), "s3d_get_prepared_block_stats")
+        return {"allocated": a.value, "reused": r.value}
+
     def counters(self):
         c = Counters()
         lib().s3d_get_counters(self._h, C.byref(c))
@@ -239,10 +248,11 @@ class Context:
 
 
 class PreparedCloud:
-    """Device-resident, preprocessed scan (s3d_prepare_cloud): voxel filter + NN grid + covariances done once."""
+    """Device-resident, preprocessed scan: voxel filter + NN grid + covariances (s3d_prepare_cloud, `k` set, `resolution` None)
+    or + NDT voxel Gaussians (s3d_prepare_cloud_ndt, `k` 0, `resolution` the grid's) done once."""
 
-    def __init__(self, ctx, handle, density, k):
-        self._ctx, self._h, self.density, self.k = ctx, handle, density, k
+    def __init__(self, ctx, handle, density, k, resolution=None):
+        self._ctx, self._h, self.density, self.k, self.resolution = ctx, handle, density, k, resolution
 
     @property
     def size(self):
@@ -279,6 +289,28 @@ def _prepare_clouds(self, clouds, density, k=20, device_slot=0):
     st = lib().s3d_prepare_clouds(self._h, device_slot, cc, n, float(density), int(k), hh)
     self._check(st, "s3d_prepare_clouds")
     return [PreparedCloud(self, C.c_void_p(hh[i]), float(density), int(k)) for i in range(n)]
+
+
+def _prepare_cloud_ndt(self, cloud, density, resolution, device_slot=0):
+    """NDT handle: voxel filter at `density`, NN grid and the VoxelGridCovariance at `resolution` (what doNDT builds for its target)."""
+    a, c = _cloud(self, cloud)
+    h = C.c_void_p()
+    st = lib().s3d_prepare_cloud_ndt(self._h, device_slot, c, float(density), float(resolution), C.byref(h))
+    self._check(st, "s3d_prepare_cloud_ndt")
+    return PreparedCloud(self, h, float(density), 0, float(C.c_float(resolution).value))
+
+
+def _prepare_clouds_ndt(self, clouds, density, resolution, device_slot=0):
+    n = len(clouds)
+    keep = []
+    cc = (Cloud * n)()
+    for i in range(n):
+        a, c = _cloud(self, clouds[i]); keep.append(a); cc[i] = c
+    hh = (C.c_void_p * n)()
+    st = lib().s3d_prepare_clouds_ndt(self._h, device_slot, cc, n, float(density), float(resolution), hh)
+    self._check(st, "s3d_prepare_clouds_ndt")
+    r = float(C.c_float(resolution).value)
+    return [PreparedCloud(self, C.c_void_p(hh[i]), float(density), 0, r) for i in range(n)]
 
 
 def _gicp_align_prepared(self, source, target, guess=None, params=None):
@@ -358,6 +390,8 @@ Context.remove_outliers = _remove_outliers
 Context.build_map = _build_map
 Context.prepare_cloud = _prepare_cloud
 Context.prepare_clouds = _prepare_clouds
+Context.prepare_cloud_ndt = _prepare_cloud_ndt
+Context.prepare_clouds_ndt = _prepare_clouds_ndt
 Context.gicp_align_prepared = _gicp_align_prepared
 Context.gicp_align_prepared_batch = _gicp_align_prepared_batch
 

@@ -18,6 +18,7 @@
 #include <thread>
 
 #include "internal.h"
+#include "ndt_math.h"
 
 namespace s3d {
 
@@ -29,6 +30,7 @@ struct DeviceCtx {
   std::mutex mu;
   std::mutex upload_mu;  // one chunk uploads at a time (Workspace::upload_gate)
   std::vector<std::pair<void*, size_t>> free_blocks;  // recycled allocations of released prepared clouds
+  uint64_t blocks_allocated = 0, blocks_reused = 0;   // prepared-cloud blocks from cudaMalloc / from free_blocks (under mu)
   std::vector<std::unique_ptr<Workspace>> pool;  // idle workspaces
   std::vector<Workspace*> all;
 };
@@ -84,10 +86,12 @@ class WorkerPool {
 struct s3d_prepared_cloud {
   int device_slot = 0;
   s3d::SlotInfo info;        // host copy; gpts / normals / table point into `block`
-  void* block = nullptr;     // one device allocation: [gpts | normals | hash table]
+  void* block = nullptr;     // one device allocation: GICP [gpts | normals | hash table], NDT [gpts | hash table | NDT leaves | NDT hash]
   size_t block_bytes = 0;
   double density = 0;
-  int k = 0;
+  int k = 0;                 // kNN of the covariances (GICP handles); 0 for NDT handles
+  float resolution = 0.f;    // NDT handles: resolution of `grid`; 0 for GICP handles
+  s3d::NdtGrid grid{};       // NDT handles: the VoxelGridCovariance; leaves / table point into `block`
 };
 
 struct s3d_context {
@@ -553,36 +557,56 @@ static void* block_alloc(DeviceCtx* dc, size_t bytes, size_t* got) {
       if (dc->free_blocks[i].second >= bytes && dc->free_blocks[i].second <= 2 * bytes + 4096) {
         void* p = dc->free_blocks[i].first; *got = dc->free_blocks[i].second;
         dc->free_blocks.erase(dc->free_blocks.begin() + i);
+        ++dc->blocks_reused;
         return p;
       }
   }
   void* p = nullptr;
   S3D_CUDA(cudaMalloc(&p, bytes));
   *got = bytes;
+  std::lock_guard<std::mutex> g(dc->mu);
+  ++dc->blocks_allocated;
   return p;
 }
 
 namespace s3d {
-// Per-cloud stages for `n` clouds in one workspace pass, then one device block per cloud.
-static void prepare_chunk(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k, s3d_prepared_cloud** out) {
+// Per-cloud stages for `n` clouds in one workspace pass, then one device block per cloud.  resolution > 0 builds NDT handles
+// (VoxelGridCovariance at `resolution`), otherwise GICP handles (kNN-k covariances and normals).
+static void prepare_chunk(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k, float resolution,
+                          s3d_prepared_cloud** out) {
   WsLease lease(ctx, device_slot);
   Workspace& ws = *lease;
+  const bool ndt = resolution > 0.f;
   const float leaf = density > 0 ? (float)density : 0.f;
   std::vector<const float*> ptrs(n);
   std::vector<uint64_t> sizes(n);
   uint64_t total = 0;
   for (int i = 0; i < n; ++i) { ptrs[i] = clouds[i].xyzw; sizes[i] = clouds[i].n; total += clouds[i].n; }
   SlotInfo* hs = nullptr;
+  NdtGrid* hg = nullptr;
   with_arena_retry(ws, [&] {
     setup_batch(ws, ptrs, sizes, 0);
     run_voxel(ws, leaf);
-    if (total) { run_grid(ws, leaf); run_knn_covariances(ws, k, nullptr, nullptr); }
+    if (total) {
+      run_grid(ws, leaf);
+      if (ndt) {
+        const std::vector<float> res(n, resolution);
+        run_ndt_grids(ws, kNdtEverySlot, (uint32_t)n, res.data());
+      } else {
+        run_knn_covariances(ws, k, nullptr, nullptr);
+      }
+    }
     hs = ws.h_slots.as<SlotInfo>();
     int32_t* hf = ws.h_small.as<int32_t>();
     S3D_CUDA(cudaMemcpyAsync(hs, ws.slots.p, sizeof(SlotInfo) * n, cudaMemcpyDeviceToHost, ws.stream));
     S3D_CUDA(cudaMemcpyAsync(hf, ws.flags.p, 16, cudaMemcpyDeviceToHost, ws.stream));
-    ws.sync();
     ws.d2h += sizeof(SlotInfo) * n + 16;
+    if (ndt && total) {  // the grid sizes, which size the blocks, arrive with the same synchronise
+      hg = ws.h_grids.as<NdtGrid>();
+      S3D_CUDA(cudaMemcpyAsync(hg, ws.ndt_grids.p, sizeof(NdtGrid) * n, cudaMemcpyDeviceToHost, ws.stream));
+      ws.d2h += sizeof(NdtGrid) * n;
+    }
+    ws.sync();
     ws.collect_spans();
     check_arena(ws, hf);
     ws.learn_grid_frac(hs, (uint32_t)n);
@@ -600,20 +624,35 @@ static void prepare_chunk(s3d_context* ctx, int device_slot, const s3d_cloud* cl
   for (int i = 0; i < n; ++i) {
     std::unique_ptr<s3d_prepared_cloud>& h = hh[i];
     h.reset(new s3d_prepared_cloud());
-    h->device_slot = device_slot; h->density = density; h->k = k;
+    h->device_slot = device_slot; h->density = density; h->k = ndt ? 0 : k; h->resolution = ndt ? resolution : 0.f;
     h->info = hs[i];
     const size_t np = h->info.n_pts;
-    const size_t b_pts = up(16 * np), b_nrm = up(32 * np), b_tab = up(sizeof(HashEntry) * (size_t)h->info.hash_cap);
+    if (ndt) {  // a cloud without a searchable grid (no finite point, int32 guard) keeps an empty one: its align ends at once
+      if (hg) h->grid = hg[i];
+      h->grid.resolution = resolution;
+      h->grid.leaves = nullptr; h->grid.table = nullptr;
+    }
+    const size_t b_pts = up(16 * np), b_nrm = ndt ? 0 : up(32 * np), b_tab = up(sizeof(HashEntry) * (size_t)h->info.hash_cap);
+    const bool ndt_arrays = ndt && h->grid.searchable;
+    const size_t b_leaf = ndt_arrays ? up(sizeof(NdtLeaf) * (size_t)h->grid.n_voxels) : 0;
+    const size_t b_ndt_tab = ndt_arrays ? up(sizeof(uint2) * ((size_t)h->grid.hash_mask + 1)) : 0;
     if (np) {
-      h->block = block_alloc(ctx->devs[device_slot].get(), b_pts + b_nrm + b_tab, &h->block_bytes);
+      h->block = block_alloc(ctx->devs[device_slot].get(), b_pts + b_nrm + b_tab + b_leaf + b_ndt_tab, &h->block_bytes);
       char* base = static_cast<char*>(h->block);
       S3D_CUDA(cudaMemcpyAsync(base, ws.gpts.as<float4>() + hs[i].off, 16 * np, cudaMemcpyDeviceToDevice, ws.stream));
-      S3D_CUDA(cudaMemcpyAsync(base + b_pts, ws.normals.as<double4>() + hs[i].off, 32 * np, cudaMemcpyDeviceToDevice, ws.stream));
+      if (!ndt) S3D_CUDA(cudaMemcpyAsync(base + b_pts, ws.normals.as<double4>() + hs[i].off, 32 * np, cudaMemcpyDeviceToDevice, ws.stream));
       S3D_CUDA(cudaMemcpyAsync(base + b_pts + b_nrm, ws.hash.as<HashEntry>() + hs[i].hash_off, sizeof(HashEntry) * (size_t)h->info.hash_cap,
                                cudaMemcpyDeviceToDevice, ws.stream));
       h->info.gpts = reinterpret_cast<const float4*>(base);
-      h->info.normals = reinterpret_cast<const double4*>(base + b_pts);
+      h->info.normals = ndt ? nullptr : reinterpret_cast<const double4*>(base + b_pts);
       h->info.table = reinterpret_cast<const HashEntry*>(base + b_pts + b_nrm);
+      if (ndt_arrays) {  // leaf ranks in the hash are relative to the leaf array: copying both keeps them valid
+        char* leaves = base + b_pts + b_tab;
+        S3D_CUDA(cudaMemcpyAsync(leaves, hg[i].leaves, sizeof(NdtLeaf) * (size_t)h->grid.n_voxels, cudaMemcpyDeviceToDevice, ws.stream));
+        S3D_CUDA(cudaMemcpyAsync(leaves + b_leaf, hg[i].table, sizeof(uint2) * ((size_t)h->grid.hash_mask + 1), cudaMemcpyDeviceToDevice, ws.stream));
+        h->grid.leaves = reinterpret_cast<NdtLeaf*>(leaves);
+        h->grid.table = reinterpret_cast<uint2*>(leaves + b_leaf);
+      }
     } else {
       h->info.gpts = nullptr; h->info.normals = nullptr; h->info.table = nullptr; h->info.hash_cap = 0;
     }
@@ -623,13 +662,10 @@ static void prepare_chunk(s3d_context* ctx, int device_slot, const s3d_cloud* cl
   guard.armed = false;
   for (int i = 0; i < n; ++i) out[i] = hh[i].release();
 }
-}  // namespace s3d
 
-int s3d_prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k, s3d_prepared_cloud** out) {
-  if (!ctx || !out || n < 0 || (n > 0 && !clouds) || device_slot < 0 || device_slot >= (int)ctx->devs.size()) return S3D_INVALID_ARGUMENT;
-  for (int i = 0; i < n; ++i) out[i] = nullptr;
-  if (k < 1 || k > kMaxK) { set_error("correspondence_randomness must be in [1, 4096]"); return S3D_INVALID_ARGUMENT; }
-  if (n == 0) return S3D_OK;
+// s3d_prepare_clouds / s3d_prepare_clouds_ndt: chunks of the n clouds on `streams_small` worker threads, all-or-nothing
+static int prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k, float resolution,
+                          s3d_prepared_cloud** out) {
   const int W = std::max(1, ctx->streams_small);
   const int chunk = balanced_chunk(n, W, 2 * ctx->max_pairs_per_launch);
   std::vector<int> st(W, S3D_OK);
@@ -643,7 +679,7 @@ int s3d_prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* cloud
       for (;;) {
         const int b = next.fetch_add(1) * chunk;
         if (b >= n) break;
-        prepare_chunk(ctx, device_slot, clouds + b, std::min(chunk, n - b), density, k, out + b);
+        prepare_chunk(ctx, device_slot, clouds + b, std::min(chunk, n - b), density, k, resolution, out + b);
       }
       return S3D_OK;
     });
@@ -660,10 +696,35 @@ int s3d_prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* cloud
     }
   return S3D_OK;
 }
+}  // namespace s3d
+
+int s3d_prepare_clouds(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, int k, s3d_prepared_cloud** out) {
+  if (!ctx || !out || n < 0 || (n > 0 && !clouds) || device_slot < 0 || device_slot >= (int)ctx->devs.size()) return S3D_INVALID_ARGUMENT;
+  for (int i = 0; i < n; ++i) out[i] = nullptr;
+  if (k < 1 || k > kMaxK) { set_error("correspondence_randomness must be in [1, 4096]"); return S3D_INVALID_ARGUMENT; }
+  if (n == 0) return S3D_OK;
+  return prepare_clouds(ctx, device_slot, clouds, n, density, k, 0.f, out);
+}
 
 int s3d_prepare_cloud(s3d_context* ctx, int device_slot, s3d_cloud cloud, double density, int k, s3d_prepared_cloud** out) {
   if (!out) return S3D_INVALID_ARGUMENT;
   return s3d_prepare_clouds(ctx, device_slot, &cloud, 1, density, k, out);
+}
+
+int s3d_prepare_clouds_ndt(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, double density, float resolution,
+                           s3d_prepared_cloud** out) {
+  if (!ctx || !out || n < 0 || (n > 0 && !clouds)) return S3D_INVALID_ARGUMENT;
+  for (int i = 0; i < n; ++i) out[i] = nullptr;
+  if (device_slot < 0 || device_slot >= (int)ctx->devs.size()) { set_error("bad device slot"); return S3D_INVALID_ARGUMENT; }
+  if (!(resolution > 0.f) || !std::isfinite(resolution)) { set_error("NDT resolution must be positive and finite"); return S3D_INVALID_ARGUMENT; }
+  if (std::isnan(density)) { set_error("point_cloud_density must not be NaN"); return S3D_INVALID_ARGUMENT; }
+  if (n == 0) return S3D_OK;
+  return prepare_clouds(ctx, device_slot, clouds, n, density, 0, resolution, out);
+}
+
+int s3d_prepare_cloud_ndt(s3d_context* ctx, int device_slot, s3d_cloud cloud, double density, float resolution, s3d_prepared_cloud** out) {
+  if (!out) return S3D_INVALID_ARGUMENT;
+  return s3d_prepare_clouds_ndt(ctx, device_slot, &cloud, 1, density, resolution, out);
 }
 
 int s3d_release_cloud(s3d_context* ctx, s3d_prepared_cloud* cloud) {
@@ -680,53 +741,76 @@ int s3d_release_cloud(s3d_context* ctx, s3d_prepared_cloud* cloud) {
 
 uint64_t s3d_prepared_cloud_size(const s3d_prepared_cloud* cloud) { return cloud ? cloud->info.n_pts : 0; }
 
+int s3d_get_prepared_block_stats(s3d_context* ctx, uint64_t* allocated, uint64_t* reused) {
+  if (!ctx) return S3D_INVALID_ARGUMENT;
+  uint64_t a = 0, r = 0;
+  for (auto& dc : ctx->devs) { std::lock_guard<std::mutex> g(dc->mu); a += dc->blocks_allocated; r += dc->blocks_reused; }
+  if (allocated) *allocated = a;
+  if (reused) *reused = r;
+  return S3D_OK;
+}
+
 namespace s3d {
-// One sub-batch of align() calls on prepared clouds (all on device slot `slot`).
+// One sub-batch of align() calls on prepared clouds (all on device slot `slot`).  GICP runs every pair; NDT runs the pairs whose
+// fixed cloud (the source, slot 2p) is an NDT handle, and the others end as align() ends for an algorithm without its data.
 static void align_prepared_chunk(s3d_context* ctx, int slot, const s3d_prepared_cloud* const* sources, const s3d_prepared_cloud* const* targets,
                                  const double* guesses, const s3d_registration_parameters& cfg_in, int n, s3d_result* out) {
   s3d_registration_parameters cfg = cfg_in;
   cfg.registration_algorithm = effective_algorithm(cfg_in.registration_algorithm);
+  const bool gicp = cfg.registration_algorithm == S3D_ALG_GICP, ndt = cfg.registration_algorithm == S3D_ALG_NDT;
+  std::vector<int> run;  // pairs that reach the optimiser, in batch order
+  for (int i = 0; i < n; ++i) {
+    if (gicp || (ndt && sources[i]->resolution > 0.f)) { run.push_back(i); continue; }
+    // same order as align(): <100 gate first, then the algorithm switch
+    memset(&out[i], 0, sizeof out[i]);
+    for (int j = 0; j < 16; ++j) out[i].T[j] = (j % 5 == 0) ? 1.0 : 0.0;
+    out[i].n_source = sources[i]->info.n_pts; out[i].n_target = targets[i]->info.n_pts;
+    out[i].status = (out[i].n_source < 100 || out[i].n_target < 100) ? S3D_TOO_FEW_POINTS : S3D_UNKNOWN_ALGORITHM;
+  }
+  if ((int)run.size() < n) {
+    if (cfg.registration_algorithm == S3D_ALG_GICP_OMP || cfg.registration_algorithm == S3D_ALG_NDT_OMP)
+      set_error("OMP is not available, you need to rebuild SLAM3D with OMP or use another matching algorithm.");
+    else if (ndt)
+      set_error("NDT on prepared clouds needs the source scan prepared with s3d_prepare_clouds_ndt / s3d_prepare_cloud_ndt "
+                "(this handle holds GICP data); or use s3d_gicp_align / s3d_gicp_align_batch on the raw clouds.");
+    else set_error("Unknown registration algorithm specified.");
+  }
+  if (run.empty()) return;
+  const int m = (int)run.size();
   WsLease lease(ctx, slot);
   Workspace& ws = *lease;
   S3D_CUDA(cudaSetDevice(ws.device));
-  const uint32_t ns = 2 * n;
-  ws.n_slots = ns; ws.n_pairs = n; ws.n_tiles = 0;
+  const uint32_t ns = 2 * m;
+  ws.n_slots = ns; ws.n_pairs = m; ws.n_tiles = 0;
   ws.grid_frac = 1.f;  // prepared clouds: the sizes below are the filtered sizes
   ws.h_off.assign(ns, 0); ws.h_n.assign(ns, 0);
-  ws.pair_off.resize(n);
+  ws.pair_off.resize(m);
   ws.slots.reserve(sizeof(SlotInfo) * ns);
   ws.h_slots.reserve(sizeof(SlotInfo) * ns);
   SlotInfo* hs = ws.h_slots.as<SlotInfo>();
   uint64_t total = 0;
   ws.max_na = 0;
-  for (int i = 0; i < n; ++i) {
-    hs[2 * i] = sources[i]->info; hs[2 * i + 1] = targets[i]->info;
-    ws.h_n[2 * i] = sources[i]->info.n_pts; ws.h_n[2 * i + 1] = targets[i]->info.n_pts;
-    ws.pair_off[i] = (uint32_t)total;
+  std::vector<double> g(16 * (size_t)m);
+  std::vector<NdtGrid> grids(ndt ? m : 0);
+  for (int j = 0; j < m; ++j) {
+    const int i = run[j];
+    hs[2 * j] = sources[i]->info; hs[2 * j + 1] = targets[i]->info;
+    ws.h_n[2 * j] = sources[i]->info.n_pts; ws.h_n[2 * j + 1] = targets[i]->info.n_pts;
+    ws.pair_off[j] = (uint32_t)total;
     total += (targets[i]->info.n_pts + 3u) & ~3u;
     ws.max_na = std::max(ws.max_na, targets[i]->info.n_pts);
+    memcpy(&g[16 * (size_t)j], guesses + 16 * (size_t)i, sizeof(double) * 16);
+    if (ndt) grids[j] = sources[i]->grid;
   }
   if (total >= (1ull << 31)) throw CudaError{"batch too large: more than 2^31 points"};
   ws.total = (uint32_t)total;
   S3D_CUDA(cudaMemcpyAsync(ws.slots.p, hs, sizeof(SlotInfo) * ns, cudaMemcpyHostToDevice, ws.stream));
   S3D_CUDA(cudaMemsetAsync(ws.flags.p, 0, 64, ws.stream));
-  if (cfg.registration_algorithm != S3D_ALG_GICP) {  // same order as align(): <100 gate first, then the algorithm switch
-    for (int i = 0; i < n; ++i) {
-      memset(&out[i], 0, sizeof out[i]);
-      for (int j = 0; j < 16; ++j) out[i].T[j] = (j % 5 == 0) ? 1.0 : 0.0;
-      out[i].n_source = ws.h_n[2 * i]; out[i].n_target = ws.h_n[2 * i + 1];
-      out[i].status = (out[i].n_source < 100 || out[i].n_target < 100) ? S3D_TOO_FEW_POINTS : S3D_UNKNOWN_ALGORITHM;
-    }
-    ws.sync();
-    if (cfg.registration_algorithm == S3D_ALG_GICP_OMP || cfg.registration_algorithm == S3D_ALG_NDT_OMP)
-      set_error("OMP is not available, you need to rebuild SLAM3D with OMP or use another matching algorithm.");
-    else if (cfg.registration_algorithm == S3D_ALG_NDT)
-      set_error("NDT voxelises the filtered source scan itself: use s3d_gicp_align / s3d_gicp_align_batch (prepared clouds hold GICP data only).");
-    else set_error("Unknown registration algorithm specified.");
-    return;
-  }
-  std::vector<s3d_registration_parameters> params(n, cfg);
-  run_gicp(ws, params, guesses, out);
+  std::vector<s3d_registration_parameters> params(m, cfg);
+  std::vector<s3d_result> res(m);
+  if (ndt) run_ndt_prepared(ws, params, g.data(), grids.data(), res.data());
+  else run_gicp(ws, params, g.data(), res.data());
+  for (int j = 0; j < m; ++j) out[run[j]] = res[j];
 }
 }  // namespace s3d
 
@@ -735,14 +819,24 @@ int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* co
   if (!ctx || !params || !out || n_pairs < 0 || (n_pairs > 0 && (!sources || !targets || !guesses))) return S3D_INVALID_ARGUMENT;
   if (n_pairs == 0) return S3D_OK;
   const int slot = sources[0] ? sources[0]->device_slot : 0;
+  const int alg = effective_algorithm(params->registration_algorithm);
   for (int i = 0; i < n_pairs; ++i) {
     if (!sources[i] || !targets[i]) return S3D_INVALID_ARGUMENT;
     if (sources[i]->device_slot != slot || targets[i]->device_slot != slot) { set_error("prepared clouds of one call must live on one device"); return S3D_INVALID_ARGUMENT; }
     for (const s3d_prepared_cloud* h : {sources[i], targets[i]})
-      if (h->density != params->point_cloud_density || (effective_algorithm(params->registration_algorithm) == S3D_ALG_GICP && h->k != params->correspondence_randomness)) {
-        set_error("prepared cloud was built with another point_cloud_density / correspondence_randomness");
+      if (h->density != params->point_cloud_density || (alg == S3D_ALG_GICP && (h->k < 1 || h->k != params->correspondence_randomness))) {
+        set_error(h->k < 1 && alg == S3D_ALG_GICP ? "prepared cloud holds NDT data (s3d_prepare_clouds_ndt): GICP needs s3d_prepare_clouds handles"
+                                                  : "prepared cloud was built with another point_cloud_density / correspondence_randomness");
         return S3D_INVALID_ARGUMENT;
       }
+    // NDT reads the source's grid (the PCL target) and the target's points only, so any handle of the right density serves as target
+    float want = params->resolution, have = sources[i]->resolution;
+    if (alg == S3D_ALG_NDT && have > 0.f && memcmp(&have, &want, sizeof(float)) != 0) {
+      char buf[160];
+      snprintf(buf, sizeof buf, "prepared cloud holds an NDT grid of resolution %.9g, the parameters ask for %.9g", (double)have, (double)want);
+      set_error(buf);
+      return S3D_INVALID_ARGUMENT;
+    }
   }
   const int W = std::max(1, ctx->streams_small);
   std::vector<int> st(W, S3D_OK);

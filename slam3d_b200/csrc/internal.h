@@ -117,6 +117,35 @@ struct GicpArgs {
 
 constexpr int kIterTile = 256;   // source points per CTA in the fused correspondence kernel
 
+struct NdtLeaf;  // ndt_math.h
+
+// NDT target grid of one fixed cloud: pcl::VoxelGridCovariance at `resolution` (ndt.cu).  Built in a workspace for the fixed
+// clouds of a raw NDT batch, or for every cloud of s3d_prepare_clouds_ndt, whose handles keep it beside their copies of the leaves
+// and the hash table.  Hash entries are (voxel key, leaf rank) with ranks relative to `leaves`, so a copy of both arrays is valid.
+struct NdtGrid {
+  float resolution, inv_leaf;
+  int32_t min_b[3], div_b[3];
+  uint32_t mul1, mul2;
+  uint32_t n_voxels;         // occupied voxels = entries of `leaves`
+  uint32_t n_leaves;         // voxels with >= 6 points: the centroid cloud
+  uint32_t hash_mask;        // entries of `table` - 1
+  uint32_t escaped;          // some float centroid lies outside its own voxel
+  int32_t searchable;        // grid parameters valid (finite cloud, no int32 overflow)
+  uint32_t reserved;
+  NdtLeaf* leaves;           // n_voxels leaves in ascending key order
+  uint2* table;              // open-addressing hash voxel key -> leaf rank
+};
+
+// Which slots of a workspace batch get an NDT grid, and where it goes: slot s has one iff (s & skip_mask) == 0, grid s >> shift.
+// Raw NDT batches build the grid of every fixed cloud (slot 2p -> grid p); the prepare pass builds one per slot.
+struct NdtGridMap {
+  uint32_t shift, skip_mask;
+  __host__ __device__ bool has(uint32_t slot) const { return (slot & skip_mask) == 0; }
+  __host__ __device__ uint32_t grid(uint32_t slot) const { return slot >> shift; }
+  __host__ __device__ uint32_t slot(uint32_t g) const { return g << shift; }
+};
+constexpr NdtGridMap kNdtFixedSlots{1, 1}, kNdtEverySlot{0, 0};
+
 // All device memory of one in-flight batch on one device.
 struct Workspace {
   int device = 0;
@@ -183,13 +212,14 @@ struct Workspace {
   DevBuf fit_partial;                         // double[iter_tiles*2]
   DevBuf accu, accu2, map_aux;                // map building: accumulated cloud, filtered cloud, poses / keep flags
   DevBuf ndt_pairs, ndt_leaves, ndt_hash, ndt_part;  // NDT: NdtPair[n_pairs], NdtLeaf[], uint2 hash arena, double[tiles * 44]
+  DevBuf ndt_grids;                           // NdtGrid[]: the grids a build writes, or the grids of the pairs of an NDT align
   DevBuf gicp_args, gicp_sched;               // GicpArgs; 16 counter words + PairSched[n_pairs] of the loop kernel
   uint64_t passes = 0, ctrl_steps = 0;        // tiles processed / control steps run by the loop kernel (statistics)
   std::map<uint64_t, cudaGraphExec_t> loop_graphs;  // throughput mode: WHILE (a pair iterates) { per-pass kernels }, by (tiles per pair, pairs)
   std::vector<cudaGraph_t> loop_graph_defs;
   uint64_t loop_graph_sig = 0;                // hash of the pointer values the cached graphs were built with
   DevBuf flags;                               // int32[16]: [0] error bits, [1] active pairs, [2] hash entries used, [3] entries needed, [8] long voxel runs, [9] kept points
-  PinnedBuf h_slots, h_pairs, h_small, h_tiles;  // pinned host mirrors
+  PinnedBuf h_slots, h_pairs, h_small, h_tiles, h_grids;  // pinned host mirrors
   PinnedBuf h_bounce;                            // pinned landing zone for pageable host clouds (setup_batch)
   uint64_t launches = 0, h2d = 0, d2h = 0;
   // optional stage timing (s3d_set_profiling)
@@ -237,6 +267,12 @@ uint32_t run_accumulate(Workspace& ws, const std::vector<const float*>& clouds, 
 uint32_t run_radius_filter(Workspace& ws, const float4* dev_in, uint32_t n, double radius, unsigned min_pts, float4* dev_out);
 void check_arena(Workspace& ws, const int32_t* h_flags);  // throws ArenaOverflow when the grid build flagged it (h_flags: synchronised copy)
 void run_gicp(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);
-void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);  // ndt.cu
+// ndt.cu.  run_ndt: doNDT for every pair of a raw batch (builds the grids of slots 2p).  run_ndt_grids: only the grids of the slots
+// `map` selects, at `resolution`, into ws.ndt_grids (read back by the caller's next synchronise).  run_ndt_prepared: doNDT for
+// pairs whose fixed-cloud grids exist: grids[p] is the grid of pair p (host records whose arrays live on the device).
+void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);
+void run_ndt_grids(Workspace& ws, NdtGridMap map, uint32_t n_grids, const float* resolution);
+void run_ndt_prepared(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, const NdtGrid* grids,
+                      s3d_result* out);
 
 }  // namespace s3d

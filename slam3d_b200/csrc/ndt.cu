@@ -28,6 +28,8 @@
 
 namespace s3d {
 
+// Per-registration state of pair p; its target grid is grids[p] of the launch (built by the raw path, or copied from the
+// prepared handle of its fixed cloud).
 struct NdtPair {
   float guess[16];
   float T_cur[16];           // final_transformation_: matrix of the pending / last evaluation
@@ -36,19 +38,9 @@ struct NdtPair {
   double gauss_d1, gauss_d2;
   double fit_range, fit_sum;
   float r2;                  // float(resolution^2)
-  float resolution, inv_leaf;
-  int32_t min_b[3], div_b[3];
-  uint32_t mul1, mul2;
-  uint32_t n_voxels;         // occupied voxels
-  uint32_t n_leaves;         // voxels with >= 6 points: the centroid cloud
-  uint32_t hash_off, hash_mask;
-  uint32_t leaf_off;
-  uint32_t escaped;          // some float centroid lies outside its own voxel
   uint32_t fit_n;
-  int32_t searchable;        // grid parameters valid (finite cloud, no int32 overflow)
   int32_t enough;            // both clouds hold >= 100 points (align() :134)
   int32_t active, pending;   // pending: an evaluation at T_cur is requested
-  uint32_t reserved;
 };
 
 __device__ __forceinline__ uint32_t ndt_hash_slot(uint32_t key, uint32_t mask) {
@@ -58,47 +50,44 @@ __device__ __forceinline__ uint32_t ndt_hash_slot(uint32_t key, uint32_t mask) {
 }
 
 // VoxelGridCovariance::applyFilter prologue for B: leaf size, int32 overflow guard, min_b / div_b / divb_mul
-__global__ void ndt_params_kernel(const SlotInfo* __restrict__ slots, NdtPair* __restrict__ pairs, uint32_t n_pairs) {
-  const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
-  if (p >= n_pairs) return;
-  NdtPair& np = pairs[p];
-  const SlotInfo& sb = slots[2 * p];
-  const SlotInfo& sa = slots[2 * p + 1];
-  np.enough = (sa.n_pts >= 100 && sb.n_pts >= 100) ? 1 : 0;
-  np.searchable = 0; np.n_voxels = 0; np.n_leaves = 0; np.escaped = 0; np.hash_mask = 0;
-  if (!np.enough) return;
+__global__ void ndt_params_kernel(const SlotInfo* __restrict__ slots, NdtGridMap map, NdtGrid* __restrict__ grids, uint32_t n_grids) {
+  const uint32_t g = blockIdx.x * blockDim.x + threadIdx.x;
+  if (g >= n_grids) return;
+  NdtGrid& G = grids[g];
+  const SlotInfo& sb = slots[map.slot(g)];
+  G.searchable = 0; G.n_voxels = 0; G.n_leaves = 0; G.escaped = 0; G.hash_mask = 0;
+  if (sb.n_pts == 0) return;
   if (!(sb.g_max[0] >= sb.g_min[0]) || !(sb.g_max[1] >= sb.g_min[1]) || !(sb.g_max[2] >= sb.g_min[2])) return;  // no finite point
-  const float inv = __fdiv_rn(1.0f, np.resolution);
-  np.inv_leaf = inv;
+  const float inv = __fdiv_rn(1.0f, G.resolution);
+  G.inv_leaf = inv;
   const long long dx = (long long)__fmul_rn(__fsub_rn(sb.g_max[0], sb.g_min[0]), inv) + 1;
   const long long dy = (long long)__fmul_rn(__fsub_rn(sb.g_max[1], sb.g_min[1]), inv) + 1;
   const long long dz = (long long)__fmul_rn(__fsub_rn(sb.g_max[2], sb.g_min[2]), inv) + 1;
   if (dx * dy * dz > 2147483647ll) return;  // "Leaf size is too small for the input dataset": the grid stays empty
   for (int a = 0; a < 3; ++a) {
-    np.min_b[a] = (int)floorf(__fmul_rn(sb.g_min[a], inv));
-    np.div_b[a] = (int)floorf(__fmul_rn(sb.g_max[a], inv)) - np.min_b[a] + 1;
+    G.min_b[a] = (int)floorf(__fmul_rn(sb.g_min[a], inv));
+    G.div_b[a] = (int)floorf(__fmul_rn(sb.g_max[a], inv)) - G.min_b[a] + 1;
   }
-  np.mul1 = (uint32_t)np.div_b[0];
-  np.mul2 = (uint32_t)np.div_b[0] * (uint32_t)np.div_b[1];
-  np.searchable = 1;
+  G.mul1 = (uint32_t)G.div_b[0];
+  G.mul2 = (uint32_t)G.div_b[0] * (uint32_t)G.div_b[1];
+  G.searchable = 1;
 }
 
-__device__ __forceinline__ uint32_t ndt_voxel_key(const NdtPair& np, float x, float y, float z) {
-  const int i0 = (int)floorf(__fmul_rn(x, np.inv_leaf)) - np.min_b[0];
-  const int i1 = (int)floorf(__fmul_rn(y, np.inv_leaf)) - np.min_b[1];
-  const int i2 = (int)floorf(__fmul_rn(z, np.inv_leaf)) - np.min_b[2];
-  return (uint32_t)i0 + (uint32_t)i1 * np.mul1 + (uint32_t)i2 * np.mul2;
+__device__ __forceinline__ uint32_t ndt_voxel_key(const NdtGrid& G, float x, float y, float z) {
+  const int i0 = (int)floorf(__fmul_rn(x, G.inv_leaf)) - G.min_b[0];
+  const int i1 = (int)floorf(__fmul_rn(y, G.inv_leaf)) - G.min_b[1];
+  const int i2 = (int)floorf(__fmul_rn(z, G.inv_leaf)) - G.min_b[2];
+  return (uint32_t)i0 + (uint32_t)i1 * G.mul1 + (uint32_t)i2 * G.mul2;
 }
 
-// voxel key of every point of B's working cloud (A's slots get key 0: they ride through the segmented sort untouched)
+// voxel key of every point of a grid slot's working cloud (other slots get key 0: they ride through the segmented sort untouched)
 __global__ void __launch_bounds__(kSortThreads) ndt_keys_kernel(const SlotInfo* __restrict__ slots, TileMap tm, const float4* __restrict__ work,
-                                                                 const NdtPair* __restrict__ pairs, uint32_t* __restrict__ keys) {
+                                                                 NdtGridMap map, const NdtGrid* __restrict__ grids, uint32_t* __restrict__ keys) {
   const uint32_t t = blockIdx.x;
   const uint32_t slot = tm.tile_slot[t], first = tm.tile_first[t];
   const SlotInfo& si = slots[slot];
   if (first >= si.n_pts) return;
-  const NdtPair& np = pairs[slot >> 1];
-  const bool fixed = (slot & 1u) == 0 && np.searchable;
+  const bool fixed = map.has(slot) && grids[map.grid(slot)].searchable;
 #pragma unroll
   for (int j = 0; j < kSortTile / kSortThreads; ++j) {
     const uint32_t e = first + j * kSortThreads + threadIdx.x;
@@ -106,22 +95,23 @@ __global__ void __launch_bounds__(kSortThreads) ndt_keys_kernel(const SlotInfo* 
       uint32_t key = 0;
       if (fixed) {
         const float4 v = work[si.off + e];
-        key = finite3(v.x, v.y, v.z) ? ndt_voxel_key(np, v.x, v.y, v.z) : kInvalidKey;
+        key = finite3(v.x, v.y, v.z) ? ndt_voxel_key(grids[map.grid(slot)], v.x, v.y, v.z) : kInvalidKey;
       }
       keys[si.off + e] = key;
     }
   }
 }
 
-// run starts (voxels) per tile of B's sorted keys
-__global__ void __launch_bounds__(kSortThreads) ndt_heads_kernel(const SlotInfo* __restrict__ slots, TileMap tm, const NdtPair* __restrict__ pairs,
-                                                                  const uint32_t* __restrict__ keys, uint32_t* __restrict__ tile_heads) {
+// run starts (voxels) per tile of a grid slot's sorted keys
+__global__ void __launch_bounds__(kSortThreads) ndt_heads_kernel(const SlotInfo* __restrict__ slots, TileMap tm, NdtGridMap map,
+                                                                  const NdtGrid* __restrict__ grids, const uint32_t* __restrict__ keys,
+                                                                  uint32_t* __restrict__ tile_heads) {
   __shared__ uint32_t wsum[8];
   const uint32_t t = blockIdx.x;
   const uint32_t slot = tm.tile_slot[t], first = tm.tile_first[t];
-  if (slot & 1u) return;
+  if (!map.has(slot)) return;
   const SlotInfo& si = slots[slot];
-  if (!pairs[slot >> 1].searchable || first >= si.n_pts) return;
+  if (!grids[map.grid(slot)].searchable || first >= si.n_pts) return;
   const uint32_t n = si.n_pts;
   const uint32_t* k = keys + si.off;
   uint32_t c = 0;
@@ -137,15 +127,16 @@ __global__ void __launch_bounds__(kSortThreads) ndt_heads_kernel(const SlotInfo*
   if (threadIdx.x == 0) { uint32_t s = 0; for (int i = 0; i < 8; ++i) s += wsum[i]; tile_heads[t] = s; }
 }
 
-// one warp per pair: exclusive scan of the tile counts of slot 2p, number of voxels, hash capacity
-__global__ void ndt_scan_kernel(const SlotInfo* __restrict__ slots, NdtPair* __restrict__ pairs, const uint32_t* __restrict__ slot_tile_begin,
-                                uint32_t* __restrict__ tile_heads) {
-  const uint32_t p = blockIdx.x;
-  NdtPair& np = pairs[p];
-  if (!np.searchable) return;
-  const SlotInfo& si = slots[2 * p];
+// one warp per grid: exclusive scan of the tile counts of its slot, number of voxels, hash capacity
+__global__ void ndt_scan_kernel(const SlotInfo* __restrict__ slots, NdtGridMap map, NdtGrid* __restrict__ grids,
+                                const uint32_t* __restrict__ slot_tile_begin, uint32_t* __restrict__ tile_heads) {
+  const uint32_t g = blockIdx.x;
+  NdtGrid& G = grids[g];
+  if (!G.searchable) return;
+  const uint32_t slot = map.slot(g);
+  const SlotInfo& si = slots[slot];
   const uint32_t ntiles = (si.n_pts + kSortTile - 1) / kSortTile;
-  uint32_t* h = tile_heads + slot_tile_begin[2 * p];
+  uint32_t* h = tile_heads + slot_tile_begin[slot];
   const int lane = threadIdx.x;
   uint32_t running = 0;
   for (uint32_t b = 0; b < ntiles; b += 32) {
@@ -158,34 +149,34 @@ __global__ void ndt_scan_kernel(const SlotInfo* __restrict__ slots, NdtPair* __r
     running += __shfl_sync(0xFFFFFFFFu, incl, 31);
   }
   if (lane == 0) {
-    np.n_voxels = running;
+    G.n_voxels = running;
     uint32_t cap = 4;
     while (cap < 2u * running + 2u) cap <<= 1;
-    np.hash_mask = cap - 1u;
+    G.hash_mask = cap - 1u;
   }
 }
 
-__global__ void ndt_hash_clear_kernel(const NdtPair* __restrict__ pairs, uint2* __restrict__ table) {
-  const NdtPair& np = pairs[blockIdx.y];
-  if (!np.searchable) return;
-  uint2* tab = table + np.hash_off;
-  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i <= np.hash_mask; i += gridDim.x * blockDim.x) tab[i] = make_uint2(0xFFFFFFFFu, 0u);
+__global__ void ndt_hash_clear_kernel(const NdtGrid* __restrict__ grids) {
+  const NdtGrid& G = grids[blockIdx.y];
+  if (!G.searchable) return;
+  uint2* tab = G.table;
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i <= G.hash_mask; i += gridDim.x * blockDim.x) tab[i] = make_uint2(0xFFFFFFFFu, 0u);
 }
 
 // One thread per voxel (run of equal sorted keys): sums in ascending input order (the sort is stable), Gaussian, leaf record,
 // hash insertion.  Leaves with fewer than 6 points are recorded with key = kInvalidKey and stay out of the hash.
-__global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* __restrict__ slots, TileMap tm, NdtPair* __restrict__ pairs,
-                                                                 const uint32_t* __restrict__ keys, const uint32_t* __restrict__ vals,
-                                                                 const float4* __restrict__ work, const uint32_t* __restrict__ tile_heads,
-                                                                 NdtLeaf* __restrict__ leaves, uint2* __restrict__ table) {
+__global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* __restrict__ slots, TileMap tm, NdtGridMap map,
+                                                                 NdtGrid* __restrict__ grids, const uint32_t* __restrict__ keys,
+                                                                 const uint32_t* __restrict__ vals, const float4* __restrict__ work,
+                                                                 const uint32_t* __restrict__ tile_heads) {
   __shared__ uint32_t wsum[8];
   const uint32_t t = blockIdx.x;
   const uint32_t slot = tm.tile_slot[t], first = tm.tile_first[t];
-  if (slot & 1u) return;
+  if (!map.has(slot)) return;
   const SlotInfo& si = slots[slot];
-  NdtPair& np = pairs[slot >> 1];
+  NdtGrid& G = grids[map.grid(slot)];
   const uint32_t n = si.n_pts;
-  if (!np.searchable || first >= n) return;
+  if (!G.searchable || first >= n) return;
   const uint32_t* k = keys + si.off;
   const uint32_t* v = vals + si.off;
   const float4* pts = work + si.off;
@@ -210,8 +201,8 @@ __global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* 
   __syncthreads();
   uint32_t rank = tile_heads[t] + incl - cnt;
   for (int i = 0; i < w; ++i) rank += wsum[i];
-  uint2* tab = table + np.hash_off;
-  NdtLeaf* out = leaves + np.leaf_off;
+  uint2* tab = G.table;
+  NdtLeaf* out = G.leaves;
 #pragma unroll 1
   for (int j = 0; j < kPer; ++j) {
     if (!(head_mask & (1u << j))) continue;
@@ -242,12 +233,12 @@ __global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* 
       L.cx = __fdiv_rn(cs0, fn); L.cy = __fdiv_rn(cs1, fn); L.cz = __fdiv_rn(cs2, fn);
       L.key = kk;
       ndt_finalize_leaf(nr, ms, cv, L.mean, L.icov);
-      if (ndt_voxel_key(np, L.cx, L.cy, L.cz) != kk) atomicOr(&np.escaped, 1u);
-      atomicAdd(&np.n_leaves, 1u);
-      uint32_t s = ndt_hash_slot(kk, np.hash_mask);
+      if (ndt_voxel_key(G, L.cx, L.cy, L.cz) != kk) atomicOr(&G.escaped, 1u);
+      atomicAdd(&G.n_leaves, 1u);
+      uint32_t s = ndt_hash_slot(kk, G.hash_mask);
       for (;;) {
         if (atomicCAS(&tab[s].x, 0xFFFFFFFFu, kk) == 0xFFFFFFFFu) { tab[s].y = rank; break; }
-        s = (s + 1) & np.hash_mask;
+        s = (s + 1) & G.hash_mask;
       }
     }
     out[rank] = L;
@@ -255,12 +246,14 @@ __global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* 
   }
 }
 
-// Registration::align set-up after the grid is known: "Voxel grid is not searchable" ends the registration at once
-__global__ void ndt_prepare_kernel(NdtPair* __restrict__ pairs, uint32_t n_pairs, int32_t* __restrict__ flags) {
+// Registration::align set-up after the grid is known: the <100 gate, and "Voxel grid is not searchable" ends the registration at once
+__global__ void ndt_prepare_kernel(const SlotInfo* __restrict__ slots, NdtPair* __restrict__ pairs, const NdtGrid* __restrict__ grids,
+                                   uint32_t n_pairs, int32_t* __restrict__ flags) {
   const uint32_t p = blockIdx.x * blockDim.x + threadIdx.x;
   if (p >= n_pairs) return;
   NdtPair& np = pairs[p];
-  if (np.enough && np.searchable && np.n_leaves > 0) {
+  np.enough = (slots[2 * p + 1].n_pts >= 100 && slots[2 * p].n_pts >= 100) ? 1 : 0;
+  if (np.enough && grids[p].searchable && grids[p].n_leaves > 0) {
     np.active = 1; np.pending = 1;  // first computeDerivatives at `transform` with output = guess * input (T_cur = guess)
     ndt_angle_derivatives(np.opt.x_t, np.ang);
     atomicAdd(&flags[1], 1);
@@ -275,13 +268,13 @@ constexpr int kNdtMaxCand = 32;
 
 // computeDerivatives: one thread per moving point
 __global__ void __launch_bounds__(kIterTile) ndt_eval_kernel(const SlotInfo* __restrict__ slots, const NdtPair* __restrict__ pairs,
-                                                             const NdtLeaf* __restrict__ leaves, const uint2* __restrict__ table,
-                                                             double* __restrict__ part) {
+                                                             const NdtGrid* __restrict__ grids, double* __restrict__ part) {
   __shared__ NdtAngular ang;
   __shared__ double wpart[kIterTile / 32][kNdtSums];
   const uint32_t p = blockIdx.y;
   const NdtPair& np = pairs[p];
   if (!np.pending) return;
+  const NdtGrid& G = grids[p];
   const SlotInfo& sa = slots[2 * p + 1];
   const uint32_t first = blockIdx.x * kIterTile;
   if (first >= sa.n_pts) return;
@@ -296,34 +289,34 @@ __global__ void __launch_bounds__(kIterTile) ndt_eval_kernel(const SlotInfo* __r
     const float4 pt = sa.gpts[r];
     const float3 q = transform_se3(np.T_cur, pt.x, pt.y, pt.z);
     if (finite3(q.x, q.y, q.z)) {
-      const float inv = np.inv_leaf;
+      const float inv = G.inv_leaf;
       const float ux = __fmul_rn(q.x, inv), uy = __fmul_rn(q.y, inv), uz = __fmul_rn(q.z, inv);
       const float fx = floorf(ux), fy = floorf(uy), fz = floorf(uz);
       if (fabsf(fx) < 1.0e9f && fabsf(fy) < 1.0e9f && fabsf(fz) < 1.0e9f) {
-        const int cx = (int)fx - np.min_b[0], cy = (int)fy - np.min_b[1], cz = (int)fz - np.min_b[2];
+        const int cx = (int)fx - G.min_b[0], cy = (int)fy - G.min_b[1], cz = (int)fz - G.min_b[2];
         // a centroid within `resolution` of q lies in the 3x3x3 block around q's voxel unless q sits on a face or the
         // float centroid was rounded out of its voxel: then the block widens on that side
-        const bool esc = np.escaped != 0;
+        const bool esc = G.escaped != 0;
         const float ax = ux - fx, ay = uy - fy, az = uz - fz;
         const int lox = (esc || ax < 1e-3f) ? -2 : -1, hix = (esc || ax > 0.999f) ? 2 : 1;
         const int loy = (esc || ay < 1e-3f) ? -2 : -1, hiy = (esc || ay > 0.999f) ? 2 : 1;
         const int loz = (esc || az < 1e-3f) ? -2 : -1, hiz = (esc || az > 0.999f) ? 2 : 1;
-        const uint2* tab = table + np.hash_off;
-        const NdtLeaf* lv = leaves + np.leaf_off;
-        const uint32_t mask = np.hash_mask;
+        const uint2* tab = G.table;
+        const NdtLeaf* lv = G.leaves;
+        const uint32_t mask = G.hash_mask;
         float cd[kNdtMaxCand];
         uint32_t ck[kNdtMaxCand], cr[kNdtMaxCand];
         int nc = 0;
         for (int dz = loz; dz <= hiz; ++dz) {
           const int iz = cz + dz;
-          if ((unsigned)iz >= (unsigned)np.div_b[2]) continue;
+          if ((unsigned)iz >= (unsigned)G.div_b[2]) continue;
           for (int dy = loy; dy <= hiy; ++dy) {
             const int iy = cy + dy;
-            if ((unsigned)iy >= (unsigned)np.div_b[1]) continue;
+            if ((unsigned)iy >= (unsigned)G.div_b[1]) continue;
             for (int dx = lox; dx <= hix; ++dx) {
               const int ix = cx + dx;
-              if ((unsigned)ix >= (unsigned)np.div_b[0]) continue;
-              const uint32_t key = (uint32_t)ix + (uint32_t)iy * np.mul1 + (uint32_t)iz * np.mul2;
+              if ((unsigned)ix >= (unsigned)G.div_b[0]) continue;
+              const uint32_t key = (uint32_t)ix + (uint32_t)iy * G.mul1 + (uint32_t)iz * G.mul2;
               uint32_t s = ndt_hash_slot(key, mask), rank = kNoIndex;
               for (;;) {
                 const uint2 en = __ldg(tab + s);
@@ -475,16 +468,61 @@ static void m4d_mul_d(const double A[16], const double B[16], double C[16]) {
 }
 double rotation_angle_of(const double T[16]);  // gicp.cu: Eigen::AngleAxisd(R).angle()
 
-// Runs doNDT for every pair of the batch (voxel filter and NN grid must be ready) and fills `out` with the decisions of
-// doNDT (:107-110) and align() (:134-135, :167-172).
-void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out) {
+// VoxelGridCovariance of the slots `map` selects (voxel filter and NN grid must be ready): grid g at resolution[g] lands in
+// ws.ndt_grids[g], its leaves and hash table in the workspace's NDT arenas.  Nothing is synchronised.
+void run_ndt_grids(Workspace& ws, NdtGridMap map, uint32_t n_grids, const float* resolution) {
+  cudaStream_t st = ws.stream;
+  ws.ndt_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(n_grids, 1));
+  ws.h_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(n_grids, 1));
+  NdtGrid* hg = ws.h_grids.as<NdtGrid>();
+  std::vector<size_t> leaf_off(n_grids), hash_off(n_grids);
+  size_t leaf_total = 0, hash_total = 0;
+  for (uint32_t g = 0; g < n_grids; ++g) {
+    const size_t nb = ws.h_n[map.slot(g)];  // raw size of the cloud bounds its voxel count
+    leaf_off[g] = leaf_total;
+    hash_off[g] = hash_total;
+    leaf_total += nb;
+    size_t cap = 4;
+    while (cap < 2 * nb + 2) cap <<= 1;
+    hash_total += cap;
+  }
+  ws.ndt_leaves.reserve(sizeof(NdtLeaf) * std::max<size_t>(leaf_total, 1));
+  ws.ndt_hash.reserve(sizeof(uint2) * std::max<size_t>(hash_total, 4));
+  for (uint32_t g = 0; g < n_grids; ++g) {
+    memset(&hg[g], 0, sizeof(NdtGrid));
+    hg[g].resolution = resolution[g];
+    hg[g].leaves = ws.ndt_leaves.as<NdtLeaf>() + leaf_off[g];
+    hg[g].table = ws.ndt_hash.as<uint2>() + hash_off[g];
+  }
+  S3D_CUDA(cudaMemcpyAsync(ws.ndt_grids.p, hg, sizeof(NdtGrid) * n_grids, cudaMemcpyHostToDevice, st));
+  const SlotInfo* slots = ws.slots.as<SlotInfo>();
+  NdtGrid* grids = ws.ndt_grids.as<NdtGrid>();
+  TileMap tm{ws.tile_slot.as<uint32_t>(), ws.tile_first.as<uint32_t>(), ws.n_tiles};
+  StageTimer timer(ws, kStageKnn);  // the target's Gaussian voxel grid takes the place of GICP's covariance stage
+  uint32_t* keys[2] = {ws.keys0.as<uint32_t>(), ws.keys1.as<uint32_t>()};
+  uint32_t* vals[2] = {ws.vals0.as<uint32_t>(), ws.vals1.as<uint32_t>()};
+  ndt_params_kernel<<<(n_grids + 63) / 64, 64, 0, st>>>(slots, map, grids, n_grids);
+  ndt_keys_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, ws.work.as<float4>(), map, grids, keys[0]);
+  ws.launches += 2;
+  radix_sort_segmented(st, slots, ws.n_slots, tm, ws.slot_tile_begin.as<uint32_t>(), keys, vals, ws.sort_state(), kCountPts, /*digits_done=*/false,
+                       &ws.launches);
+  ndt_heads_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, map, grids, keys[0], ws.tile_heads.as<uint32_t>());
+  ndt_scan_kernel<<<n_grids, 32, 0, st>>>(slots, map, grids, ws.slot_tile_begin.as<uint32_t>(), ws.tile_heads.as<uint32_t>());
+  ndt_hash_clear_kernel<<<dim3(32, n_grids), 256, 0, st>>>(grids);
+  ndt_leaf_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, map, grids, keys[0], vals[0], ws.work.as<float4>(), ws.tile_heads.as<uint32_t>());
+  ws.launches += 4;
+}
+
+// The optimiser of doNDT for every pair of ws's batch; ws.ndt_grids[p] holds the grid of pair p on the device (built by
+// run_ndt_grids on this stream, or uploaded from prepared handles).  Fills `out` with the decisions of doNDT (:107-110) and
+// align() (:134-135, :167-172).
+static void ndt_optimise(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out) {
   const uint32_t np = ws.n_pairs;
   cudaStream_t st = ws.stream;
   const uint32_t tiles_per_pair = std::max<uint32_t>(1, (ws.max_na + kIterTile - 1) / kIterTile);
   ws.ndt_pairs.reserve(sizeof(NdtPair) * np);
   ws.h_pairs.reserve(sizeof(NdtPair) * np);
   NdtPair* hp = ws.h_pairs.as<NdtPair>();
-  size_t leaf_total = 0, hash_total = 0;
   int max_iter = 0;
   for (uint32_t p = 0; p < np; ++p) {
     const s3d_registration_parameters& cfg = params[p];
@@ -499,45 +537,21 @@ void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& para
     ndt_opt_begin(q.opt, x0, cfg.step_size, cfg.transformation_epsilon, cfg.maximum_iterations);
     ndt_gauss_constants((double)cfg.resolution, cfg.outlier_ratio, q.gauss_d1, q.gauss_d2);
     q.fit_range = cfg.max_correspondence_distance;
-    q.resolution = cfg.resolution;
     q.r2 = (float)((double)cfg.resolution * (double)cfg.resolution);
-    const size_t nb = ws.h_n[2 * p];  // raw size of B bounds its voxel count
-    q.leaf_off = (uint32_t)leaf_total;
-    q.hash_off = (uint32_t)hash_total;
-    leaf_total += nb;
-    size_t cap = 4;
-    while (cap < 2 * nb + 2) cap <<= 1;
-    hash_total += cap;
     max_iter = std::max(max_iter, cfg.maximum_iterations);
   }
-  if (leaf_total >= (1ull << 32) || hash_total >= (1ull << 32)) throw CudaError{"NDT batch too large"};
-  ws.ndt_leaves.reserve(sizeof(NdtLeaf) * std::max<size_t>(leaf_total, 1));
-  ws.ndt_hash.reserve(sizeof(uint2) * std::max<size_t>(hash_total, 4));
   ws.ndt_part.reserve(sizeof(double) * kNdtSums * size_t(tiles_per_pair) * np);
   ws.fit_partial.reserve(sizeof(double) * 2 * size_t(tiles_per_pair) * np);
   S3D_CUDA(cudaMemcpyAsync(ws.ndt_pairs.p, hp, sizeof(NdtPair) * np, cudaMemcpyHostToDevice, st));
   const SlotInfo* slots = ws.slots.as<SlotInfo>();
   NdtPair* pairs = ws.ndt_pairs.as<NdtPair>();
-  NdtLeaf* leaves = ws.ndt_leaves.as<NdtLeaf>();
-  uint2* table = ws.ndt_hash.as<uint2>();
+  const NdtGrid* grids = ws.ndt_grids.as<NdtGrid>();
   int32_t* flags = ws.flags.as<int32_t>();
   int32_t* h_flags = ws.h_small.as<int32_t>();
-  TileMap tm{ws.tile_slot.as<uint32_t>(), ws.tile_first.as<uint32_t>(), ws.n_tiles};
   {
-    StageTimer timer(ws, kStageKnn);  // the target's Gaussian voxel grid takes the place of GICP's covariance stage
-    uint32_t* keys[2] = {ws.keys0.as<uint32_t>(), ws.keys1.as<uint32_t>()};
-    uint32_t* vals[2] = {ws.vals0.as<uint32_t>(), ws.vals1.as<uint32_t>()};
-    ndt_params_kernel<<<(np + 63) / 64, 64, 0, st>>>(slots, pairs, np);
-    ndt_keys_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, ws.work.as<float4>(), pairs, keys[0]);
-    ws.launches += 2;
-    radix_sort_segmented(st, slots, ws.n_slots, tm, ws.slot_tile_begin.as<uint32_t>(), keys, vals, ws.sort_state(), kCountPts, /*digits_done=*/false,
-                         &ws.launches);
-    ndt_heads_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, pairs, keys[0], ws.tile_heads.as<uint32_t>());
-    ndt_scan_kernel<<<np, 32, 0, st>>>(slots, pairs, ws.slot_tile_begin.as<uint32_t>(), ws.tile_heads.as<uint32_t>());
-    ndt_hash_clear_kernel<<<dim3(32, np), 256, 0, st>>>(pairs, table);
-    ndt_leaf_kernel<<<ws.n_tiles, kSortThreads, 0, st>>>(slots, tm, pairs, keys[0], vals[0], ws.work.as<float4>(), ws.tile_heads.as<uint32_t>(), leaves, table);
-    ndt_prepare_kernel<<<(np + 63) / 64, 64, 0, st>>>(pairs, np, flags);
-    ws.launches += 5;
+    StageTimer timer(ws, kStageSolve);
+    ndt_prepare_kernel<<<(np + 63) / 64, 64, 0, st>>>(slots, pairs, grids, np, flags);
+    ++ws.launches;
   }
   const bool trace = getenv("S3D_TRACE") != nullptr;
   dim3 grid(tiles_per_pair, np);
@@ -547,7 +561,7 @@ void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& para
     for (int e = 0; e < 4; ++e) {
       {
         StageTimer timer(ws, kStageIter);
-        ndt_eval_kernel<<<grid, kIterTile, 0, st>>>(slots, pairs, leaves, table, ws.ndt_part.as<double>());
+        ndt_eval_kernel<<<grid, kIterTile, 0, st>>>(slots, pairs, grids, ws.ndt_part.as<double>());
         ++ws.launches;
       }
       {
@@ -560,11 +574,14 @@ void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& para
     ws.sync();
     ws.d2h += 16;
     if (trace && np <= 4) {
+      ws.h_grids.reserve(sizeof(NdtGrid) * np);
+      NdtGrid* hg = ws.h_grids.as<NdtGrid>();
       S3D_CUDA(cudaMemcpy(hp, pairs, sizeof(NdtPair) * np, cudaMemcpyDeviceToHost));
+      S3D_CUDA(cudaMemcpy(hg, grids, sizeof(NdtGrid) * np, cudaMemcpyDeviceToHost));
       for (uint32_t p = 0; p < np; ++p)
         fprintf(stderr, "[s3d ndt] round=%ld pair=%u phase=%d outer=%d line=%d score=%.12g x=(%.9g %.9g %.9g %.9g %.9g %.9g) pairs=%u leaves=%u/%u esc=%u\n", round, p,
                 hp[p].opt.phase, hp[p].opt.nr_iterations, hp[p].opt.line_iterations, hp[p].opt.score, hp[p].opt.x[0], hp[p].opt.x[1], hp[p].opt.x[2],
-                hp[p].opt.x[3], hp[p].opt.x[4], hp[p].opt.x[5], hp[p].opt.n_pairs_last, hp[p].n_leaves, hp[p].n_voxels, hp[p].escaped);
+                hp[p].opt.x[3], hp[p].opt.x[4], hp[p].opt.x[5], hp[p].opt.n_pairs_last, hg[p].n_leaves, hg[p].n_voxels, hg[p].escaped);
     }
     if (h_flags[1] <= 0) break;
   }
@@ -602,6 +619,23 @@ void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& para
     const double tn = sqrt(delta[12] * delta[12] + delta[13] * delta[13] + delta[14] * delta[14]);
     r.status = (tn > cfg.max_translation || rotation_angle_of(delta) > cfg.max_rotation) ? S3D_TOO_FAR_FROM_GUESS : S3D_OK;  // :167-172
   }
+}
+
+void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out) {
+  std::vector<float> resolution(ws.n_pairs);
+  for (uint32_t p = 0; p < ws.n_pairs; ++p) resolution[p] = params[p].resolution;
+  run_ndt_grids(ws, kNdtFixedSlots, ws.n_pairs, resolution.data());
+  ndt_optimise(ws, params, guesses, out);
+}
+
+void run_ndt_prepared(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, const NdtGrid* grids,
+                      s3d_result* out) {
+  const uint32_t np = ws.n_pairs;
+  ws.ndt_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(np, 1));
+  ws.h_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(np, 1));
+  memcpy(ws.h_grids.p, grids, sizeof(NdtGrid) * np);
+  S3D_CUDA(cudaMemcpyAsync(ws.ndt_grids.p, ws.h_grids.p, sizeof(NdtGrid) * np, cudaMemcpyHostToDevice, ws.stream));
+  ndt_optimise(ws, params, guesses, out);
 }
 
 }  // namespace s3d

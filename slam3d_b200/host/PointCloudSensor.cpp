@@ -2,6 +2,7 @@
 // Reference behaviour cited per function (slam3d/sensor/pcl/PointCloudSensor.cpp).
 #include "PointCloudSensor.hpp"
 
+#include <cmath>
 #include <list>
 #include <stdexcept>
 
@@ -28,7 +29,8 @@ struct Prepared {
   s3d_prepared_cloud* h = nullptr;
   ~Prepared() { if (h) s3d_release_cloud(defaultContext(), h); }
 };
-struct CacheEntry { const PointCloud* key; std::weak_ptr<PointCloud> alive; double density; int k; std::shared_ptr<Prepared> prepared; };
+// key: (cloud, density, kind, k | resolution); GICP entries have resolution 0, NDT entries k 0
+struct CacheEntry { const PointCloud* key; std::weak_ptr<PointCloud> alive; double density; int k; float resolution; std::shared_ptr<Prepared> prepared; };
 std::mutex g_cache_mutex;
 std::list<CacheEntry> g_cache;  // front = most recently used
 size_t g_cache_capacity = 32;
@@ -44,13 +46,14 @@ size_t preparedCacheHits() { std::lock_guard<std::mutex> g(g_cache_mutex); retur
 
 static s3d_cloud asCloud(const PointCloud::Ptr& c);
 
-// the prepared form of `cloud` for (density, k): from the cache, or built now and remembered
-static std::shared_ptr<Prepared> prepared(const PointCloud::Ptr& cloud, double density, int k) {
+// the prepared form of `cloud` for (density, k) — or, with resolution > 0, its NDT form for (density, resolution): from the
+// cache, or built now and remembered
+static std::shared_ptr<Prepared> prepared(const PointCloud::Ptr& cloud, double density, int k, float resolution = 0.f) {
   {
     std::lock_guard<std::mutex> g(g_cache_mutex);
     for (auto it = g_cache.begin(); it != g_cache.end();) {
       if (it->alive.expired()) { it = g_cache.erase(it); continue; }  // the measurement is gone; its address may be reused
-      if (it->key == cloud.get() && it->density == density && it->k == k) {
+      if (it->key == cloud.get() && it->density == density && it->k == k && it->resolution == resolution) {
         ++g_cache_hits;
         g_cache.splice(g_cache.begin(), g_cache, it);
         return g_cache.front().prepared;
@@ -59,9 +62,11 @@ static std::shared_ptr<Prepared> prepared(const PointCloud::Ptr& cloud, double d
     }
   }
   std::shared_ptr<Prepared> p(new Prepared());
-  if (s3d_prepare_cloud(defaultContext(), 0, asCloud(cloud), density, k, &p->h) != S3D_OK) throw std::runtime_error(s3d_last_error());
+  const int st = resolution > 0.f ? s3d_prepare_cloud_ndt(defaultContext(), 0, asCloud(cloud), density, resolution, &p->h)
+                                  : s3d_prepare_cloud(defaultContext(), 0, asCloud(cloud), density, k, &p->h);
+  if (st != S3D_OK) throw std::runtime_error(s3d_last_error());
   std::lock_guard<std::mutex> g(g_cache_mutex);
-  g_cache.push_front({cloud.get(), cloud, density, k, p});
+  g_cache.push_front({cloud.get(), cloud, density, k, resolution, p});
   while (g_cache.size() > g_cache_capacity) g_cache.pop_back();
   return p;
 }
@@ -81,9 +86,14 @@ Transform align(PointCloudMeasurement::Ptr source, PointCloudMeasurement::Ptr ta
   int st;
   bool use_cache;
   { std::lock_guard<std::mutex> g(g_cache_mutex); use_cache = g_cache_capacity > 0; }
+  const bool ndt = config.registration_algorithm == NDT || config.registration_algorithm == NDT_OMP;
   if (use_cache && (config.registration_algorithm == GICP || config.registration_algorithm == GICP_OMP) && config.correspondence_randomness >= 1 && config.correspondence_randomness <= 4096) {
     std::shared_ptr<Prepared> ps = prepared(source->getPointCloud(), config.point_cloud_density, config.correspondence_randomness);
     std::shared_ptr<Prepared> pt = prepared(target->getPointCloud(), config.point_cloud_density, config.correspondence_randomness);
+    st = s3d_gicp_align_prepared(defaultContext(), ps->h, pt->h, guess.data(), &c, &res);
+  } else if (use_cache && ndt && config.resolution > 0.f && std::isfinite(config.resolution) && !std::isnan(config.point_cloud_density)) {
+    std::shared_ptr<Prepared> ps = prepared(source->getPointCloud(), config.point_cloud_density, 0, config.resolution);
+    std::shared_ptr<Prepared> pt = prepared(target->getPointCloud(), config.point_cloud_density, 0, config.resolution);
     st = s3d_gicp_align_prepared(defaultContext(), ps->h, pt->h, guess.data(), &c, &res);
   } else {
     st = s3d_gicp_align(defaultContext(), asCloud(source->getPointCloud()), asCloud(target->getPointCloud()), guess.data(), &c, &res);
