@@ -254,6 +254,23 @@ int s3d_build_map(s3d_context* ctx, const s3d_cloud* clouds, const double* poses
 int s3d_create_combined_measurement(s3d_context* ctx, const s3d_cloud* clouds, const double* poses, int n, const double patch_pose[16],
                                     float* out_xyzw, uint64_t* n_out);
 
+/* ---- ground plane (PointCloudSensor::fillGroundPlane, PointCloudSensor.cpp:362-388) ---------------------------------------
+ * pcl::RandomSampleConsensus + SampleConsensusModelPlane (DESIGN.md 6f): coefficients[4] = (a, b, c, d), unit normal.
+ * iterations = PCL's iterations_, n_inliers = points with |a x + b y + c z + d| < threshold; inliers (may be NULL; host or device,
+ * cloud.n entries) receives their indices in ascending order.  N < 3, no non-degenerate sample in 1000 draws, or no plane with
+ * an inlier: S3D_INVALID_ARGUMENT.  threshold must be positive and finite, probability in (0, 1), max_iterations >= 1.
+ * S3D_RANSAC_BLOCK (environment, read once; measurement aid) sets how many planes are sampled and scored per round (default
+ * 256, at most 2048); results never depend on it. */
+int s3d_fit_plane_ransac(s3d_context* ctx, s3d_cloud cloud, double threshold, int max_iterations, double probability,
+                         float coefficients[4], int32_t* iterations, uint64_t* n_inliers, uint32_t* inliers);
+/* Number of points that fillGroundPlane appends for (map_resolution, radius): it depends on these two values only.  Both must be
+ * positive and finite; more than 2^31 - 1 points is S3D_INVALID_ARGUMENT. */
+int s3d_ground_fill_size(double map_resolution, double radius, uint64_t* n);
+/* PointCloudSensor::fillGroundPlane (:362-388): RANSAC plane (threshold 0.01, PCL defaults), then rings of points.  out_xyzw
+ * (host or device) receives the s3d_ground_fill_size() new points; the caller appends them.  coefficients may be NULL. */
+int s3d_fill_ground_plane(s3d_context* ctx, s3d_cloud cloud, double map_resolution, double radius, float* out_xyzw,
+                          float coefficients[4]);
+
 /* Optional per-stage device timing (CUDA events on the launching stream, read back at the call's final
  * synchronisation).  Stage ids: 0 voxel filter, 1 NN grid build, 2 kNN+covariances (NDT: the target's Gaussian voxel
  * grid), 3 the GICP loop kernel — search, trial and fitness passes and the control steps of all outer iterations (NDT:

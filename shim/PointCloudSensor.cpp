@@ -5,9 +5,9 @@
 // serializers at the end of PointCloudSensor.hpp, ScanSensor, the graph and the g2o back end are untouched and the library keeps
 // its name (libslam3d_sensor_pcl, sensor/pcl/CMakeLists.txt:57-59).  Every method of the class is defined here:
 //   * the arithmetic ones go to libs3d_b200.so (include/s3d_b200.h): downsample, transform, removeOutliers, getAccumulatedCloud,
-//     createCombinedMeasurement, buildMap and the free function align() behind createConstraint;
-//   * fillGroundPlane and loadPLY are not on the hot path (SURVEY 2.1): they keep using PCL's sample-consensus / PLY reader, so
-//     the target still links pcl_sample_consensus and pcl_io — but no longer pcl_registration or pcl_filters.
+//     createCombinedMeasurement, buildMap, fillGroundPlane and the free function align() behind createConstraint;
+//   * loadPLY keeps PCL's PLY reader, so the target still links pcl_io — but no longer pcl_registration, pcl_filters or
+//     pcl_sample_consensus.
 // This file cannot be compiled in this repository's environment (no PCL / Boost / Eigen, SURVEY 8c); the same bodies with
 // stand-in types are compiled and tested as slam3d_b200/host/PointCloudSensor.cpp (tests/test_gpu_host.py).
 #include <slam3d/sensor/pcl/PointCloudSensor.hpp>
@@ -15,8 +15,6 @@
 #include <slam3d/core/Mapper.hpp>
 
 #include <pcl/io/ply_io.h>
-#include <pcl/sample_consensus/ransac.h>
-#include <pcl/sample_consensus/sac_model_plane.h>
 
 #include <boost/format.hpp>
 
@@ -252,26 +250,15 @@ void PointCloudSensor::setMapOutlierRemoval(double r, unsigned n) {
   mMapOutlierNeighbors = n;
 }
 
-// Not on the hot path: PCL's RANSAC plane fit stays, then rings of points at map resolution are laid into the plane around the origin.
+// :362-388 on the GPU: PCL's RANSAC plane fit (same seed, same samples, same plane) and the rings of points at map resolution laid
+// into the plane around the origin (s3d_fill_ground_plane, DESIGN.md 6f).
 void PointCloudSensor::fillGroundPlane(PointCloud::Ptr cloud, ScalarType radius) {
-  pcl::SampleConsensusModelPlane<PointType>::Ptr model(new pcl::SampleConsensusModelPlane<PointType>(cloud));
-  pcl::RandomSampleConsensus<PointType> ransac(model);
-  ransac.setDistanceThreshold(0.01);
-  ransac.computeModel();
-  Eigen::VectorXf coeff;
-  ransac.getModelCoefficients(coeff);
-  const Direction normal(coeff[0], coeff[1], coeff[2]);
-  const Eigen::Hyperplane<ScalarType, 3> plane(normal, coeff[3]);
-  const double two_pi = 2 * 3.141592654, step = mMapResolution / radius;
-  for (ScalarType ring = mMapResolution; ring <= radius; ring += mMapResolution) {
-    const Position on_plane = plane.projection(Position(ring, 0, 0));
-    for (ScalarType angle = 0; angle < two_pi; angle += step) {
-      const Position q = Eigen::AngleAxis<ScalarType>(angle, normal).toRotationMatrix() * on_plane;
-      PointType p;
-      p.x = q[0]; p.y = q[1]; p.z = q[2];
-      cloud->push_back(p);
-    }
-  }
+  uint64_t m = 0;
+  if (s3d_ground_fill_size(mMapResolution, radius, &m) != S3D_OK) throw std::runtime_error(s3d_last_error());
+  std::vector<PointType, Eigen::aligned_allocator<PointType> > fill(m);
+  if (s3d_fill_ground_plane(gpu(), view(*cloud), mMapResolution, radius, m ? &fill[0].x : nullptr, nullptr) != S3D_OK)
+    throw std::runtime_error(s3d_last_error());
+  for (const PointType& p : fill) cloud->push_back(p);
 }
 
 // Not on the hot path: the PLY reader stays with PCL; the cloud becomes vertex + pose prior exactly as before.

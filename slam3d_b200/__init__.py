@@ -53,6 +53,10 @@ def lib():
         L.s3d_build_map.argtypes = [C.c_void_p, C.POINTER(Cloud), C.c_void_p, C.c_int, C.c_double, C.c_uint, C.c_double, C.c_void_p,
                                     C.POINTER(C.c_uint64)]
         L.s3d_create_combined_measurement.argtypes = [C.c_void_p, C.POINTER(Cloud), C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]
+        L.s3d_fit_plane_ransac.argtypes = [C.c_void_p, Cloud, C.c_double, C.c_int, C.c_double, C.c_void_p, C.POINTER(C.c_int32),
+                                           C.POINTER(C.c_uint64), C.c_void_p]
+        L.s3d_ground_fill_size.argtypes = [C.c_double, C.c_double, C.POINTER(C.c_uint64)]
+        L.s3d_fill_ground_plane.argtypes = [C.c_void_p, Cloud, C.c_double, C.c_double, C.c_void_p, C.c_void_p]
         L.s3d_prepare_cloud.argtypes = [C.c_void_p, C.c_int, Cloud, C.c_double, C.c_int, C.POINTER(C.c_void_p)]
         L.s3d_prepare_clouds.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.c_double, C.c_int, C.POINTER(C.c_void_p)]
         L.s3d_prepare_cloud_ndt.argtypes = [C.c_void_p, C.c_int, Cloud, C.c_double, C.c_float, C.POINTER(C.c_void_p)]
@@ -384,6 +388,42 @@ def _combined_measurement(self, clouds, poses, patch_pose):
     return out[: m.value].copy()
 
 
+def _fit_plane_ransac(self, cloud, threshold, max_iterations=10000, probability=0.99, want_inliers=False):
+    """pcl::RandomSampleConsensus + SampleConsensusModelPlane (seeded as PCL seeds it, so the result is PCL's).  Returns
+    (coefficients float32[4] = (a, b, c, d) with a unit normal, iterations, n_inliers, inliers): inliers are the ascending indices
+    of the points with |a x + b y + c z + d| < threshold when want_inliers, else None."""
+    a, c = _cloud(self, cloud)
+    coeff = np.zeros(4, np.float32)
+    it = C.c_int32(0)
+    m = C.c_uint64(0)
+    inl = np.empty(max(a.shape[0], 1), np.uint32) if want_inliers else None
+    st = lib().s3d_fit_plane_ransac(self._h, c, float(threshold), int(max_iterations), float(probability), coeff.ctypes.data, C.byref(it),
+                                    C.byref(m), inl.ctypes.data if want_inliers else None)
+    self._check(st, "s3d_fit_plane_ransac")
+    return coeff, it.value, m.value, (inl[: m.value].copy() if want_inliers else None)
+
+
+def ground_fill_size(map_resolution, radius):
+    """Number of points fill_ground_plane returns for (map_resolution, radius)."""
+    n = C.c_uint64(0)
+    st = lib().s3d_ground_fill_size(float(map_resolution), float(radius), C.byref(n))
+    if st != _abi.S3D_OK:
+        raise S3DError(f"s3d_ground_fill_size failed ({st}): {last_error()}")
+    return n.value
+
+
+def _fill_ground_plane(self, cloud, radius, map_resolution=0.1):
+    """PointCloudSensor::fillGroundPlane: RANSAC plane of `cloud` (threshold 0.01), then rings of points every map_resolution up to
+    `radius` laid into it.  Returns the new points (n,4) float32; the reference appends them to `cloud`."""
+    a, c = _cloud(self, cloud)
+    n = ground_fill_size(map_resolution, radius)
+    out = np.empty((max(n, 1), 4), np.float32)
+    self._check(lib().s3d_fill_ground_plane(self._h, c, float(map_resolution), float(radius), out.ctypes.data, None), "s3d_fill_ground_plane")
+    return out[:n].copy()
+
+
+Context.fit_plane_ransac = _fit_plane_ransac
+Context.fill_ground_plane = _fill_ground_plane
 Context.combined_measurement = _combined_measurement
 Context.transform_cloud = _transform_cloud
 Context.remove_outliers = _remove_outliers

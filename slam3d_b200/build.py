@@ -8,7 +8,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libs3d_b200.so")
-SOURCES = ["voxel.cu", "grid.cu", "knn.cu", "gicp.cu", "ndt.cu", "map.cu", "api.cu"]
+SOURCES = ["voxel.cu", "grid.cu", "knn.cu", "gicp.cu", "ndt.cu", "map.cu", "ransac.cu", "api.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 # -fmad=false: every float/double expression keeps its written operation order (PCL parity; see DESIGN.md)
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-fmad=false", "-Xcompiler", "-fPIC,-O2"]

@@ -19,6 +19,7 @@
 
 #include "internal.h"
 #include "ndt_math.h"
+#include "ransac_math.h"
 
 namespace s3d {
 
@@ -977,6 +978,91 @@ int s3d_build_map(s3d_context* ctx, const s3d_cloud* clouds, const double* poses
     *n_out = hs[0].n_pts;
     copy_out(ws, out_xyzw, ws.work.p, 16 * (size_t)hs[0].n_pts);
     ws.sync();
+    return S3D_OK;
+  });
+}
+
+// ---- ground plane ------------------------------------------------------------------------------------------------------
+namespace {
+constexpr uint64_t kMaxGroundFill = (1ull << 31) - 1;
+
+// the cloud in ws.accu (device): the sampler and the counting kernel read it many times, whatever memory it came from
+const float4* stage_cloud(Workspace& ws, s3d_cloud cloud) {
+  S3D_CUDA(cudaSetDevice(ws.device));
+  ws.order_after_input();
+  ws.accu.reserve(16 * cloud.n);
+  S3D_CUDA(cudaMemcpyAsync(ws.accu.p, cloud.xyzw, 16 * cloud.n, cudaMemcpyDefault, ws.stream));
+  return ws.accu.as<float4>();
+}
+
+int ransac_failed(const RansacFit& fit, uint64_t n) {
+  if (n < 3) set_error("RANSAC plane fit: fewer than 3 points");
+  else if (fit.iterations == 0) set_error("RANSAC plane fit: no non-degenerate sample of 3 points in 1000 draws");
+  else set_error("RANSAC plane fit: no plane has an inlier");
+  return S3D_INVALID_ARGUMENT;
+}
+}  // namespace
+
+int s3d_fit_plane_ransac(s3d_context* ctx, s3d_cloud cloud, double threshold, int max_iterations, double probability,
+                         float coefficients[4], int32_t* iterations, uint64_t* n_inliers, uint32_t* inliers) {
+  if (!ctx || !coefficients || !iterations || !n_inliers || (cloud.n && !cloud.xyzw)) return S3D_INVALID_ARGUMENT;
+  if (!(threshold > 0) || !std::isfinite(threshold) || !(probability > 0 && probability < 1) || max_iterations < 1) {
+    set_error("RANSAC plane fit: threshold must be positive and finite, probability in (0, 1), max_iterations >= 1");
+    return S3D_INVALID_ARGUMENT;
+  }
+  if (cloud.n >= (1ull << 31)) { set_error("RANSAC plane fit: more than 2^31 - 1 points"); return S3D_INVALID_ARGUMENT; }
+  *iterations = 0; *n_inliers = 0;
+  if (cloud.n < 3) return ransac_failed(RansacFit{}, cloud.n);
+  return guarded([&]() -> int {
+    WsLease lease(ctx, 0);
+    Workspace& ws = *lease;
+    const float4* pts = stage_cloud(ws, cloud);
+    const RansacFit fit = run_ransac_plane(ws, pts, (uint32_t)cloud.n, threshold, max_iterations, probability, inliers != nullptr);
+    *iterations = fit.iterations;
+    if (!fit.ok) return ransac_failed(fit, cloud.n);
+    for (int i = 0; i < 4; ++i) coefficients[i] = fit.coeff[i];
+    *n_inliers = fit.n_inliers;
+    if (inliers) { copy_out(ws, inliers, fit.inliers_dev, 4 * (size_t)fit.n_inliers); ws.sync(); }
+    return S3D_OK;
+  });
+}
+
+int s3d_ground_fill_size(double map_resolution, double radius, uint64_t* n) {
+  if (!n) return S3D_INVALID_ARGUMENT;
+  *n = 0;
+  if (!(map_resolution > 0) || !(radius > 0) || !std::isfinite(map_resolution) || !std::isfinite(radius)) {
+    set_error("ground fill: map resolution and radius must be positive and finite");
+    return S3D_INVALID_ARGUMENT;
+  }
+  if (!ground_fill_lists(map_resolution, radius, kMaxGroundFill, nullptr, nullptr, nullptr, n)) {
+    set_error("ground fill: more than 2^31 - 1 points");
+    return S3D_INVALID_ARGUMENT;
+  }
+  return S3D_OK;
+}
+
+int s3d_fill_ground_plane(s3d_context* ctx, s3d_cloud cloud, double map_resolution, double radius, float* out_xyzw, float coefficients[4]) {
+  uint64_t m = 0;
+  if (!ctx || (cloud.n && !cloud.xyzw)) return S3D_INVALID_ARGUMENT;
+  if (const int st = s3d_ground_fill_size(map_resolution, radius, &m)) return st;
+  if (m && !out_xyzw) return S3D_INVALID_ARGUMENT;
+  if (cloud.n >= (1ull << 31)) { set_error("ground fill: more than 2^31 - 1 points"); return S3D_INVALID_ARGUMENT; }
+  if (cloud.n < 3) return ransac_failed(RansacFit{}, cloud.n);
+  return guarded([&]() -> int {
+    WsLease lease(ctx, 0);
+    Workspace& ws = *lease;
+    const float4* pts = stage_cloud(ws, cloud);
+    const RansacFit fit = run_ransac_plane(ws, pts, (uint32_t)cloud.n, 0.01, 10000, 0.99, false);  // PointCloudSensor.cpp:364-366
+    if (!fit.ok) return ransac_failed(fit, cloud.n);
+    if (coefficients) for (int i = 0; i < 4; ++i) coefficients[i] = fit.coeff[i];
+    std::vector<double> rings, sin_a, cos_a;
+    uint64_t total = 0;
+    ground_fill_lists(map_resolution, radius, kMaxGroundFill, &rings, &sin_a, &cos_a, &total);
+    if (total == 0) return S3D_OK;
+    ws.accu2.reserve(16 * total);
+    run_ground_fill(ws, fit.coeff, rings, sin_a, cos_a, ws.accu2.as<float4>());
+    copy_out(ws, out_xyzw, ws.accu2.p, 16 * total);
+    ws.sync();  // the host vectors must outlive the copies
     return S3D_OK;
   });
 }

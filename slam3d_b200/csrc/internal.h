@@ -213,6 +213,7 @@ struct Workspace {
   DevBuf accu, accu2, map_aux;                // map building: accumulated cloud, filtered cloud, poses / keep flags
   DevBuf ndt_pairs, ndt_leaves, ndt_hash, ndt_part;  // NDT: NdtPair[n_pairs], NdtLeaf[], uint2 hash arena, double[tiles * 44]
   DevBuf ndt_grids;                           // NdtGrid[]: the grids a build writes, or the grids of the pairs of an NDT align
+  DevBuf ransac, ransac_idx;                  // RANSAC plane fit (ransac.cu): sampler state + one block of planes / flags / counts; uint32[n] shuffled indices
   DevBuf gicp_args, gicp_sched;               // GicpArgs; 16 counter words + PairSched[n_pairs] of the loop kernel
   uint64_t passes = 0, ctrl_steps = 0;        // tiles processed / control steps run by the loop kernel (statistics)
   std::map<uint64_t, cudaGraphExec_t> loop_graphs;  // throughput mode: WHILE (a pair iterates) { per-pass kernels }, by (tiles per pair, pairs)
@@ -221,6 +222,7 @@ struct Workspace {
   DevBuf flags;                               // int32[16]: [0] error bits, [1] active pairs, [2] hash entries used, [3] entries needed, [8] long voxel runs, [9] kept points
   PinnedBuf h_slots, h_pairs, h_small, h_tiles, h_grids;  // pinned host mirrors
   PinnedBuf h_bounce;                            // pinned landing zone for pageable host clouds (setup_batch)
+  PinnedBuf h_ransac;                            // one block of RANSAC planes / flags / counts read back for the replay
   uint64_t launches = 0, h2d = 0, d2h = 0;
   // optional stage timing (s3d_set_profiling)
   bool profiling = false;
@@ -265,6 +267,22 @@ void run_nn_stage(Workspace& ws, uint32_t ref_slot, uint32_t qry_slot, const flo
 uint32_t run_accumulate(Workspace& ws, const std::vector<const float*>& clouds, const std::vector<uint64_t>& sizes, const double* poses,
                         const double* second = nullptr);  // -> ws.accu; second: one more 4x4 applied to every (float-rounded) point
 uint32_t run_radius_filter(Workspace& ws, const float4* dev_in, uint32_t n, double radius, unsigned min_pts, float4* dev_out);
+// map.cu: exclusive scan of n_tiles per-tile counts in place (one warp); *total = their sum
+__global__ void keep_scan_kernel(uint32_t n_tiles, uint32_t* __restrict__ tile_counts, uint32_t* __restrict__ total);
+// ransac.cu.  run_ransac_plane: RandomSampleConsensus + SampleConsensusModelPlane on the n device points (ransac_math.h); with
+// want_inliers the ascending inlier indices are left at inliers_dev (workspace memory, valid until the next call on ws).
+// run_ground_fill: the fill points of fillGroundPlane for the plane `coeff` and the loop values of ground_fill_lists().
+struct RansacFit {
+  bool ok = false;
+  float coeff[4] = {0, 0, 0, 0};
+  int32_t iterations = 0;
+  uint64_t n_inliers = 0;
+  uint32_t* inliers_dev = nullptr;
+};
+RansacFit run_ransac_plane(Workspace& ws, const float4* pts, uint32_t n, double threshold, int max_iterations, double probability,
+                           bool want_inliers);
+void run_ground_fill(Workspace& ws, const float coeff[4], const std::vector<double>& rings, const std::vector<double>& sin_a,
+                     const std::vector<double>& cos_a, float4* dev_out);
 void check_arena(Workspace& ws, const int32_t* h_flags);  // throws ArenaOverflow when the grid build flagged it (h_flags: synchronised copy)
 void run_gicp(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);
 // ndt.cu.  run_ndt: doNDT for every pair of a raw batch (builds the grids of slots 2p).  run_ndt_grids: only the grids of the slots

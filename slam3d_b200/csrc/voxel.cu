@@ -83,9 +83,9 @@ void Workspace::destroy() {
 
   DevBuf* bufs[] = {&slots, &pairs, &raw_stage, &work, &gpts, &keys0, &keys1, &vals0, &vals1, &hist, &sort_totals, &long_runs, &tile_slot, &tile_first,
                     &slot_tile_begin, &tile_heads, &hash, &normals, &moved, &prev_nn, &sec_lb, &moments, &eval_part, &corr, &mahal, &iter_tile_pair, &iter_tile_first,
-                    &fit_partial, &flags, &accu, &accu2, &map_aux, &ndt_pairs, &ndt_leaves, &ndt_hash, &ndt_part, &ndt_grids, &gicp_args, &gicp_sched, &knn_arena};
+                    &fit_partial, &flags, &accu, &accu2, &map_aux, &ndt_pairs, &ndt_leaves, &ndt_hash, &ndt_part, &ndt_grids, &gicp_args, &gicp_sched, &knn_arena, &ransac, &ransac_idx};
   for (DevBuf* b : bufs) b->release();
-  h_slots.release(); h_pairs.release(); h_small.release(); h_tiles.release(); h_grids.release(); h_bounce.release();
+  h_slots.release(); h_pairs.release(); h_small.release(); h_tiles.release(); h_grids.release(); h_bounce.release(); h_ransac.release();
   if (stream) cudaStreamDestroy(stream);
   stream = nullptr;
 }

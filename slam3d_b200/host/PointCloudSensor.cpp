@@ -166,6 +166,16 @@ PointCloud::Ptr PointCloudSensor::removeOutliers(PointCloud::Ptr in, double radi
   return in;
 }
 
+// :362-388  RANSAC ground plane of the cloud, then rings of points every mMapResolution up to `radius` appended to it
+void PointCloudSensor::fillGroundPlane(PointCloud::Ptr cloud, ScalarType radius) {
+  uint64_t m = 0;
+  if (s3d_ground_fill_size(mMapResolution, radius, &m) != S3D_OK) throw std::runtime_error(s3d_last_error());
+  std::vector<PointType> fill(m);
+  if (s3d_fill_ground_plane(defaultContext(), asCloud(cloud), mMapResolution, radius, m ? &fill[0].x : nullptr, nullptr) != S3D_OK)
+    throw std::runtime_error(s3d_last_error());
+  cloud->points.insert(cloud->points.end(), fill.begin(), fill.end());
+}
+
 // :235-256  (pose = vertex.correctedPose * measurement.sensorPose, accumulated in list order)
 PointCloud::Ptr PointCloudSensor::getAccumulatedCloud(const PosedMeasurements& vertices) const {
   PointCloud::Ptr accu(new PointCloud);

@@ -205,4 +205,19 @@ int64_t s3dhost_combined_measurement(void* s, const float* const* scans, const u
   return m;
 }
 
+// fillGroundPlane on a copy of the n input points with map resolution `resolution`: out receives the whole resulting cloud
+// (input then fill points) and must hold n + s3d_ground_fill_size(resolution, radius) points.  Returns its size or -1.
+int64_t s3dhost_fill_ground_plane(void* s, const float* in, uint64_t n, double resolution, double radius, float* out) {
+  int64_t m = -1;
+  wrap([&] {
+    PointCloudSensor* sensor = static_cast<PointCloudSensor*>(s);
+    sensor->setMapResolution(resolution);
+    PointCloud::Ptr cloud = makeCloud(in, n);
+    sensor->fillGroundPlane(cloud, radius);
+    m = (int64_t)cloud->size();
+    if (m) std::memcpy(out, &cloud->points[0].x, 16 * m);
+  });
+  return m;
+}
+
 }  // extern "C"
