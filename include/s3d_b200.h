@@ -123,8 +123,10 @@ int s3d_voxel_downsample(s3d_context* ctx, s3d_cloud in, float leaf, float* out_
  *   NDT   doNDT<pcl::NormalDistributionsTransform>      (:84-117): resolution, step_size, outlier_ratio, maximum_iterations,
  *         transformation_epsilon are read; out->outer_iterations = nr_iterations_, out->inner_iterations = More-Thuente
  *         line-search iterations, out->n_correspondences = (point, voxel) pairs of the last evaluation
- *   GICP_OMP / NDT_OMP  (:149-157, pclomp's multi-threaded builds of the same two algorithms) run the GICP / NDT branch of this
- *         library; a build with -DS3D_OMP_UNAVAILABLE keeps the error of a reference build without pclomp (:158-161)
+ *   GICP_OMP / NDT_OMP  (:149-157, pclomp's multi-threaded builds of GICP and NDT) run the GICP / NDT branch of this library.
+ *         pclomp's GICP is PCL's; pclomp's NDT has PCL's optimiser but by default another neighbour search (DIRECT7: the
+ *         query's voxel and its 6 face neighbours, not PCL's kd-tree radius search), which s3d_set_ndt_omp_search selects.
+ *         A build with -DS3D_OMP_UNAVAILABLE keeps the error of a reference build without pclomp (:158-161)
  *   anything else -> S3D_UNKNOWN_ALGORITHM with the reference's message (:162-164). */
 int s3d_gicp_align(s3d_context* ctx, s3d_cloud source, s3d_cloud target, const double guess[16],
                    const s3d_registration_parameters* params, s3d_result* out);
@@ -156,6 +158,19 @@ int s3d_gicp_align_loop_batch(s3d_context* ctx, const s3d_cloud* sources, const 
  * setting it replaces.  Any other value returns S3D_INVALID_ARGUMENT and changes nothing. */
 enum { S3D_GICP_NEWTON = 0, S3D_GICP_BFGS = 1 };
 int s3d_set_gicp_optimizer(s3d_context* ctx, int optimizer, int* previous);
+
+/* Neighbour search of registration_algorithm = NDT_OMP, the one step in which pclomp's NDT differs from PCL's:
+ *   S3D_NDT_OMP_KDTREE   PCL's kd-tree radius search (every centroid within `resolution`): NDT_OMP returns what NDT returns
+ *                        (the default here; pclomp's KDTREE mode)
+ *   S3D_NDT_OMP_DIRECT7  pclomp's default, DIRECT7 (VoxelGridCovariance::getNeighborhoodAtPoint7, never changed by slam3d's
+ *                        doNDT): the query's own voxel and its 6 face neighbours, in the order (0,0,0) (+-1,0,0) (0,+-1,0)
+ *                        (0,0,+-1), cell = floor(p / leaf size), leaves with >= 6 points that PCL did not mark invalid.
+ * Like s3d_set_gicp_optimizer it belongs to the context: it applies to NDT_OMP in every align entry point — s3d_gicp_align,
+ * _batch, _loop_batch (coarse and fine each by their own algorithm), _prepared, _prepared_batch — and NDT, GICP and GICP_OMP
+ * ignore it.  Calls that start after it returns use the new setting: change it while no call is running on the context.
+ * `previous` (may be NULL) receives the setting it replaces.  Any other value returns S3D_INVALID_ARGUMENT and changes nothing. */
+enum { S3D_NDT_OMP_KDTREE = 0, S3D_NDT_OMP_DIRECT7 = 1 };
+int s3d_set_ndt_omp_search(s3d_context* ctx, int method, int* previous);
 
 /* ---- stage-level entry points (used by the parity tests and the bench; same kernels as align) ---------- */
 

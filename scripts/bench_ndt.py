@@ -3,7 +3,13 @@ through s3d_gicp_align_batch with host scans (e2e) and per-stage device times; o
 
 --prepared adds the device cache for NDT (s3d_prepare_clouds_ndt + s3d_gicp_align_prepared_batch) on the same workload, in the
 same process: prepare time per cloud, prepared and raw batch rates measured alternately, one pair's latency both ways, stage
-times of both, the card's name and power limit, and a check that the prepared results equal the raw ones field for field."""
+times of both, the card's name and power limit, and a check that the prepared results equal the raw ones field for field.
+
+--omp-search [kdtree] [direct7] times NDT_OMP with the listed neighbour searches (both when none is named) on the same workload,
+one context per search, calls alternated in one process: registrations/s end to end, then the derivative-evaluation stage
+(ndt_eval_kernel, stage gicp_iter) and the others of one profiled call each, with the card's name and power limit.  DIRECT7's
+GPU results on the first --check-pairs distinct pairs are checked against the oracle's DIRECT7 restatement (same status,
+converged flag and counts, pose within 1e-4 m / 1e-4 rad, fitness within 1e-4)."""
 import argparse
 import json
 import os
@@ -25,8 +31,12 @@ ap.add_argument("--steps", type=int, default=3)
 ap.add_argument("--oracle", action="store_true")
 ap.add_argument("--prepared", action="store_true", help="also time NDT on prepared clouds, alternating with the raw path")
 ap.add_argument("--latency-reps", type=int, default=10, help="--prepared: single-pair calls per path")
+ap.add_argument("--omp-search", nargs="*", choices=["kdtree", "direct7"], help="time NDT_OMP with these neighbour searches, alternated")
+ap.add_argument("--check-pairs", type=int, default=2, help="--omp-search: distinct pairs checked against the oracle (DIRECT7)")
 ap.add_argument("--out", help="also write the JSON to this file (--prepared: default profiles/r03_ndt_prepared.json)")
 a = ap.parse_args()
+if a.omp_search is not None and a.prepared:
+    sys.exit("--omp-search and --prepared are separate measurements")
 if a.prepared and not a.out:
     a.out = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "profiles", "r03_ndt_prepared.json")
 P = RegistrationParameters.defaults(point_cloud_density=0.1, registration_algorithm=_abi.ALG_NDT)
@@ -39,6 +49,12 @@ ctx = slam3d_b200.Context()
 def fields(r):
     return (r.status, r.converged, r.outer_iterations, r.inner_iterations, r.n_correspondences, r.n_source, r.n_target,
             r.fitness, tuple(r.T))
+
+
+def pose_delta(A, B):
+    """(translation [m], rotation angle [rad]) of inv(A) B."""
+    D = np.linalg.inv(np.asarray(A, np.float64)) @ np.asarray(B, np.float64)
+    return float(np.linalg.norm(D[:3, 3])), float(np.arccos(np.clip((np.trace(D[:3, :3]) - 1.0) / 2.0, -1.0, 1.0)))
 
 
 def card():
@@ -54,7 +70,58 @@ def card():
 
 
 res = ctx.gicp_align_batch(srcs, tgts, None, P)  # warm-up
-if not a.prepared:
+omp_ok = True
+if a.omp_search is not None:
+    methods = list(dict.fromkeys(a.omp_search)) or ["kdtree", "direct7"]
+    Pomp = RegistrationParameters.defaults(point_cloud_density=P.point_cloud_density, registration_algorithm=_abi.ALG_NDT_OMP)
+    ctxs = {}
+    for m in methods:
+        ctxs[m] = slam3d_b200.Context()
+        ctxs[m].set_ndt_omp_search(m)
+        ctxs[m].gicp_align_batch(srcs, tgts, None, Pomp)  # warm-up
+    t_step = {m: [] for m in methods}
+    last = {}
+    for _ in range(a.steps):  # alternate the searches, so that both see the same host and GPU conditions
+        for m in methods:
+            t0 = time.perf_counter()
+            last[m] = ctxs[m].gicp_align_batch(srcs, tgts, None, Pomp)
+            t_step[m].append(time.perf_counter() - t0)
+    stages = {}
+    for m in methods:  # profiled in calls of their own: the stage events are not part of the timed calls
+        ctxs[m].set_profiling(True)
+        ctxs[m].stage_times(reset=True)
+        ctxs[m].gicp_align_batch(srcs, tgts, None, Pomp)
+        stages[m] = {k: round(v["ms"], 3) for k, v in ctxs[m].stage_times(reset=True).items()}  # summed over the streams
+        ctxs[m].set_profiling(False)
+    out = {"workload": f"{a.pairs} pairs of synthetic {srcs[0].shape[0]}-point scans ({a.distinct} distinct), density {Pomp.point_cloud_density} m, "
+                       f"NDT_OMP resolution {Pomp.resolution} m, step {Pomp.step_size}, outlier ratio {Pomp.outlier_ratio}",
+           "card": card(), "steps": a.steps}
+    for m in methods:
+        med = float(np.median(t_step[m]))
+        out[m] = {"ms_per_step": [t * 1e3 for t in t_step[m]], "registrations_per_s_e2e": a.pairs / med,
+                  "derivative_eval_ms_one_call": stages[m]["gicp_iter"], "stage_ms_one_call": stages[m],
+                  "ok": sum(r.status == 0 for r in last[m]),
+                  "outer_iterations": [r.outer_iterations for r in last[m][: a.distinct]],
+                  "line_iterations": [r.inner_iterations for r in last[m][: a.distinct]],
+                  "pairs_last_evaluation": [r.n_correspondences for r in last[m][: a.distinct]]}
+    if "direct7" in methods:
+        from oracle import ndt_omp
+        ndt_omp.set_ndt_omp_search("direct7")
+        checked = []
+        for i in range(min(a.check_pairs, a.distinct)):
+            got, want = last["direct7"][i], ndt_omp.gicp_align(srcs[i], tgts[i], None, Pomp)
+            dt, dr = pose_delta(want.pose(), got.pose())
+            ok = ((got.status, got.converged, got.outer_iterations, got.inner_iterations, got.n_correspondences) ==
+                  (want.status, want.converged, want.outer_iterations, want.inner_iterations, want.n_correspondences)
+                  and dt < 1e-4 and dr < 1e-4 and abs(got.fitness - want.fitness) <= 1e-4 * abs(want.fitness))
+            checked.append({"pair": i, "ok": bool(ok), "dt_m": dt, "dr_rad": dr})
+            omp_ok = omp_ok and ok
+        out["direct7_vs_oracle"] = checked
+    if len(methods) == 2:
+        out["direct7_over_kdtree_rate"] = out["direct7"]["registrations_per_s_e2e"] / out["kdtree"]["registrations_per_s_e2e"]
+    for c in ctxs.values():
+        c.close()
+elif not a.prepared:
     ctx.set_profiling(True)
     ctx.stage_times(reset=True)
     t0 = time.perf_counter()
@@ -125,5 +192,7 @@ if a.out:
     os.makedirs(os.path.dirname(os.path.abspath(a.out)), exist_ok=True)
     with open(a.out, "w") as f:
         f.write(json.dumps(out, indent=1) + "\n")
+if not omp_ok:
+    sys.exit("DIRECT7 GPU results differ from the oracle")
 if a.prepared and not out["prepared_equals_raw"]:
     sys.exit("prepared NDT results differ from the raw ones")

@@ -36,6 +36,9 @@ s3d_context* gpu() {
 #ifdef S3D_GICP_USE_BFGS  // built against PCL < 1.14 (shim/CMakeLists.txt): GICP runs that PCL's BFGS inner optimiser
     if (s3d_set_gicp_optimizer(c, S3D_GICP_BFGS, nullptr) != S3D_OK) throw std::runtime_error(s3d_last_error());
 #endif
+#ifdef S3D_NDT_OMP_USE_DIRECT7  // shim/CMakeLists.txt: NDT_OMP runs pclomp's default DIRECT7 neighbour search
+    if (s3d_set_ndt_omp_search(c, S3D_NDT_OMP_DIRECT7, nullptr) != S3D_OK) throw std::runtime_error(s3d_last_error());
+#endif
     return c;
   }();
   return ctx;

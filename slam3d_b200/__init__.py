@@ -39,6 +39,7 @@ def lib():
         L.s3d_get_loop_stats.argtypes = [C.c_void_p, C.POINTER(C.c_uint64), C.POINTER(C.c_uint64), C.c_int]
         L.s3d_set_profiling.argtypes = [C.c_void_p, C.c_int]
         L.s3d_set_gicp_optimizer.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int)]
+        L.s3d_set_ndt_omp_search.argtypes = [C.c_void_p, C.c_int, C.POINTER(C.c_int)]
         L.s3d_get_stage_times.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int]
         L.s3d_voxel_downsample.argtypes = [C.c_void_p, Cloud, C.c_float, C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p, C.POINTER(C.c_int32)]
         L.s3d_knn_covariances.argtypes = [C.c_void_p, Cloud, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
@@ -158,6 +159,16 @@ class Context:
         prev = C.c_int(0)
         self._check(lib().s3d_set_gicp_optimizer(self._h, _abi.GICP_OPTIMIZERS[which], C.byref(prev)), "s3d_set_gicp_optimizer")
         return "bfgs" if prev.value == _abi.GICP_BFGS else "newton"
+
+    def set_ndt_omp_search(self, which):
+        """Neighbour search of every NDT_OMP registration on this context: "kdtree" (PCL's radius search, so NDT_OMP returns what NDT
+        returns; the default here) or "direct7" (pclomp's default: the query's voxel and its 6 face neighbours).  NDT, GICP and
+        GICP_OMP ignore it.  Change it while no call is running on the context.  Returns the previous setting."""
+        if which not in _abi.NDT_OMP_SEARCHES:
+            raise ValueError(f"NDT_OMP search must be one of {sorted(_abi.NDT_OMP_SEARCHES)}, not {which!r}")
+        prev = C.c_int(0)
+        self._check(lib().s3d_set_ndt_omp_search(self._h, _abi.NDT_OMP_SEARCHES[which], C.byref(prev)), "s3d_set_ndt_omp_search")
+        return "direct7" if prev.value == _abi.NDT_OMP_DIRECT7 else "kdtree"
 
     def loop_stats(self, reset=False):
         t, c = C.c_uint64(0), C.c_uint64(0)

@@ -15,6 +15,10 @@ ALG_ICP, ALG_GICP, ALG_GICP_OMP, ALG_NDT, ALG_NDT_OMP = range(5)
 GICP_NEWTON, GICP_BFGS = 0, 1
 GICP_OPTIMIZERS = {"newton": GICP_NEWTON, "bfgs": GICP_BFGS}
 
+# s3d_set_ndt_omp_search: the neighbour search of NDT_OMP (PCL's kd-tree radius search / pclomp's default DIRECT7)
+NDT_OMP_KDTREE, NDT_OMP_DIRECT7 = 0, 1
+NDT_OMP_SEARCHES = {"kdtree": NDT_OMP_KDTREE, "direct7": NDT_OMP_DIRECT7}
+
 
 class RegistrationParameters(C.Structure):
     """slam3d::RegistrationParameters (RegistrationParameters.hpp:36-97), field for field."""

@@ -176,6 +176,7 @@ struct Workspace {
   float batch_leaf = 0.f;                     // leaf size of the current batch (set by run_voxel)
   float grid_frac = 1.f;                      // what the current batch uses (1 for prepared clouds: their sizes are exact)
   int gicp_optimizer = S3D_GICP_NEWTON;       // inner optimiser of the GICP loop: the context's setting at the time the workspace was leased
+  int ndt_omp_search = S3D_NDT_OMP_KDTREE;    // neighbour search of NDT_OMP: the context's setting at the time the workspace was leased
   // after a batch: `hs` = the slot table read back from the device
   void learn_grid_frac(const SlotInfo* hs, uint32_t ns) {
     if (!(batch_leaf > 0.f)) return;
@@ -287,10 +288,11 @@ void check_arena(Workspace& ws, const int32_t* h_flags);  // throws ArenaOverflo
 void run_gicp(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);
 // ndt.cu.  run_ndt: doNDT for every pair of a raw batch (builds the grids of slots 2p).  run_ndt_grids: only the grids of the slots
 // `map` selects, at `resolution`, into ws.ndt_grids (read back by the caller's next synchronise).  run_ndt_prepared: doNDT for
-// pairs whose fixed-cloud grids exist: grids[p] is the grid of pair p (host records whose arrays live on the device).
-void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out);
+// pairs whose fixed-cloud grids exist: grids[p] is the grid of pair p (host records whose arrays live on the device).  direct7: the
+// neighbourhood of pclomp's DIRECT7 search (NDT_OMP with S3D_NDT_OMP_DIRECT7) instead of PCL's radius search.
+void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, bool direct7, s3d_result* out);
 void run_ndt_grids(Workspace& ws, NdtGridMap map, uint32_t n_grids, const float* resolution);
 void run_ndt_prepared(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, const NdtGrid* grids,
-                      s3d_result* out);
+                      bool direct7, s3d_result* out);
 
 }  // namespace s3d

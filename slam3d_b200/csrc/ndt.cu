@@ -11,7 +11,8 @@
 //                 probe of the 3x3x3 voxels around q's own voxel (a centroid lies in its voxel; the block widens to
 //                 5x5x5 when q sits within 1e-3 of a voxel face or some centroid was rounded out of its voxel, so the
 //                 result is exact), then score, gradient (6) and Hessian (36) of eq. 6.9/6.12/6.13 in FP64, reduced by
-//                 a fixed shuffle tree to one partial per 256-point tile.
+//                 a fixed shuffle tree to one partial per 256-point tile.  NDT_OMP with S3D_NDT_OMP_DIRECT7 launches the
+//                 DIRECT7 instantiation instead: pclomp's 7 fixed cells (own voxel + 6 face neighbours) in offset order.
 //   control       ndt_ctrl_kernel, one CTA per pair: fixed-order sum of the tile partials, then ONE thread advances
 //                 computeTransformation / computeStepLengthMT (resumable state machine, ndt_math.h) to the next
 //                 evaluation or to the end.  Pairs of a batch advance independently; the host polls one counter.
@@ -164,7 +165,8 @@ __global__ void ndt_hash_clear_kernel(const NdtGrid* __restrict__ grids) {
 }
 
 // One thread per voxel (run of equal sorted keys): sums in ascending input order (the sort is stable), Gaussian, leaf record,
-// hash insertion.  Leaves with fewer than 6 points are recorded with key = kInvalidKey and stay out of the hash.
+// hash insertion.  Leaves with fewer than 6 points are recorded with key = kInvalidKey and stay out of the hash; leaves PCL marks
+// invalid go into the hash with kNdtLeafInvalid in their key.
 __global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* __restrict__ slots, TileMap tm, NdtGridMap map,
                                                                  NdtGrid* __restrict__ grids, const uint32_t* __restrict__ keys,
                                                                  const uint32_t* __restrict__ vals, const float4* __restrict__ work,
@@ -231,8 +233,8 @@ __global__ void __launch_bounds__(kSortThreads) ndt_leaf_kernel(const SlotInfo* 
     if (nr >= 6) {  // min_points_per_voxel_
       const float fn = (float)nr;
       L.cx = __fdiv_rn(cs0, fn); L.cy = __fdiv_rn(cs1, fn); L.cz = __fdiv_rn(cs2, fn);
-      L.key = kk;
-      ndt_finalize_leaf(nr, ms, cv, L.mean, L.icov);
+      const bool valid = ndt_finalize_leaf(nr, ms, cv, L.mean, L.icov) && ndt_icov_usable(L.icov);
+      L.key = valid ? kk : (kk | kNdtLeafInvalid);
       if (ndt_voxel_key(G, L.cx, L.cy, L.cz) != kk) atomicOr(&G.escaped, 1u);
       atomicAdd(&G.n_leaves, 1u);
       uint32_t s = ndt_hash_slot(kk, G.hash_mask);
@@ -266,7 +268,21 @@ __global__ void ndt_prepare_kernel(const SlotInfo* __restrict__ slots, NdtPair* 
 
 constexpr int kNdtMaxCand = 32;
 
-// computeDerivatives: one thread per moving point
+// rank of the leaf under `key`, or kNoIndex (DIRECT7 lookups)
+__device__ __forceinline__ uint32_t ndt_hash_find(const uint2* __restrict__ tab, uint32_t mask, uint32_t key) {
+  uint32_t s = ndt_hash_slot(key, mask);
+  for (;;) {
+    const uint2 en = __ldg(tab + s);
+    if (en.x == key) return en.y;
+    if (en.x == 0xFFFFFFFFu) return kNoIndex;
+    s = (s + 1) & mask;
+  }
+}
+
+// computeDerivatives: one thread per moving point.  kDirect7 = false: PCL's kd-tree radius search (NDT, and NDT_OMP with
+// S3D_NDT_OMP_KDTREE).  kDirect7 = true: pclomp's DIRECT7 neighbourhood (NDT_OMP with S3D_NDT_OMP_DIRECT7): the query's own voxel
+// and its 6 face neighbours in pclomp's order, cell by float division, leaves with >= 6 points that PCL did not mark invalid.
+template <bool kDirect7>
 __global__ void __launch_bounds__(kIterTile) ndt_eval_kernel(const SlotInfo* __restrict__ slots, const NdtPair* __restrict__ pairs,
                                                              const NdtGrid* __restrict__ grids, double* __restrict__ part) {
   __shared__ NdtAngular ang;
@@ -285,7 +301,42 @@ __global__ void __launch_bounds__(kIterTile) ndt_eval_kernel(const SlotInfo* __r
 #pragma unroll
   for (int i = 0; i < kNdtSums; ++i) acc[i] = 0.0;
   const uint32_t r = first + threadIdx.x;
-  if (r < sa.n_pts) {
+  if constexpr (kDirect7) {
+    if (r < sa.n_pts) {
+      const float4 pt = sa.gpts[r];
+      const float3 q = transform_se3(np.T_cur, pt.x, pt.y, pt.z);
+      long long ijk[3];
+      if (ndt_direct7_cell(q.x, q.y, q.z, G.resolution, ijk)) {
+        const uint2* tab = G.table;
+        const NdtLeaf* lv = G.leaves;
+        uint32_t cr[7];
+        int nc = 0;
+#pragma unroll
+        for (int i = 0; i < 7; ++i) {
+          uint32_t key;
+          if (!ndt_direct7_key(ijk, i, G.min_b, G.div_b, G.mul1, G.mul2, key)) continue;
+          const uint32_t rank = ndt_hash_find(tab, G.hash_mask, key);
+          if (rank == kNoIndex) continue;  // no leaf, or fewer than 6 points (those stay out of the hash)
+          if (__ldg(&lv[rank].key) & kNdtLeafInvalid) continue;
+          cr[nc++] = rank;
+        }
+        if (nc) {
+          const double xo[3] = {(double)pt.x, (double)pt.y, (double)pt.z};
+          NdtPointDerivs P;
+          ndt_point_derivatives(ang, xo, P);
+          for (int i = 0; i < nc; ++i) {
+            const double* lp = reinterpret_cast<const double*>(lv + cr[i]);  // [2..4] mean, [5..13] icov
+            double ci[9];
+            const double xt[3] = {(double)q.x - __ldg(lp + 2), (double)q.y - __ldg(lp + 3), (double)q.z - __ldg(lp + 4)};
+#pragma unroll
+            for (int a = 0; a < 9; ++a) ci[a] = __ldg(lp + 5 + a);
+            ndt_accumulate(P, np.gauss_d1, np.gauss_d2, xt, ci, acc);
+            acc[43] += 1.0;
+          }
+        }
+      }
+    }
+  } else if (r < sa.n_pts) {
     const float4 pt = sa.gpts[r];
     const float3 q = transform_se3(np.T_cur, pt.x, pt.y, pt.z);
     if (finite3(q.x, q.y, q.z)) {
@@ -515,8 +566,9 @@ void run_ndt_grids(Workspace& ws, NdtGridMap map, uint32_t n_grids, const float*
 
 // The optimiser of doNDT for every pair of ws's batch; ws.ndt_grids[p] holds the grid of pair p on the device (built by
 // run_ndt_grids on this stream, or uploaded from prepared handles).  Fills `out` with the decisions of doNDT (:107-110) and
-// align() (:134-135, :167-172).
-static void ndt_optimise(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out) {
+// align() (:134-135, :167-172).  direct7: every evaluation uses pclomp's DIRECT7 neighbourhood instead of the radius search.
+static void ndt_optimise(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, bool direct7,
+                         s3d_result* out) {
   const uint32_t np = ws.n_pairs;
   cudaStream_t st = ws.stream;
   const uint32_t tiles_per_pair = std::max<uint32_t>(1, (ws.max_na + kIterTile - 1) / kIterTile);
@@ -561,7 +613,8 @@ static void ndt_optimise(Workspace& ws, const std::vector<s3d_registration_param
     for (int e = 0; e < 4; ++e) {
       {
         StageTimer timer(ws, kStageIter);
-        ndt_eval_kernel<<<grid, kIterTile, 0, st>>>(slots, pairs, grids, ws.ndt_part.as<double>());
+        if (direct7) ndt_eval_kernel<true><<<grid, kIterTile, 0, st>>>(slots, pairs, grids, ws.ndt_part.as<double>());
+        else ndt_eval_kernel<false><<<grid, kIterTile, 0, st>>>(slots, pairs, grids, ws.ndt_part.as<double>());
         ++ws.launches;
       }
       {
@@ -621,21 +674,21 @@ static void ndt_optimise(Workspace& ws, const std::vector<s3d_registration_param
   }
 }
 
-void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, s3d_result* out) {
+void run_ndt(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, bool direct7, s3d_result* out) {
   std::vector<float> resolution(ws.n_pairs);
   for (uint32_t p = 0; p < ws.n_pairs; ++p) resolution[p] = params[p].resolution;
   run_ndt_grids(ws, kNdtFixedSlots, ws.n_pairs, resolution.data());
-  ndt_optimise(ws, params, guesses, out);
+  ndt_optimise(ws, params, guesses, direct7, out);
 }
 
 void run_ndt_prepared(Workspace& ws, const std::vector<s3d_registration_parameters>& params, const double* guesses, const NdtGrid* grids,
-                      s3d_result* out) {
+                      bool direct7, s3d_result* out) {
   const uint32_t np = ws.n_pairs;
   ws.ndt_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(np, 1));
   ws.h_grids.reserve(sizeof(NdtGrid) * std::max<uint32_t>(np, 1));
   memcpy(ws.h_grids.p, grids, sizeof(NdtGrid) * np);
   S3D_CUDA(cudaMemcpyAsync(ws.ndt_grids.p, ws.h_grids.p, sizeof(NdtGrid) * np, cudaMemcpyHostToDevice, ws.stream));
-  ndt_optimise(ws, params, guesses, out);
+  ndt_optimise(ws, params, guesses, direct7, out);
 }
 
 }  // namespace s3d

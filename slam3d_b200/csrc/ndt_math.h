@@ -29,12 +29,17 @@ constexpr int kNdtSums = 44;  // [0] score, [1..6] gradient, [7 + 6 i + j] Hessi
 
 // One voxel of the target grid (VoxelGridCovariance::Leaf).  cx,cy,cz = float centroid (a point of voxel_centroids_),
 // key = PCL's linear voxel index (ascending order == order of the centroid cloud), nr < 6: not part of the centroid cloud.
+// A leaf of >= 6 points that applyFilter marked invalid (nr_points = -1) carries kNdtLeafInvalid in its key: the radius search
+// still returns it, DIRECT7 does not.  PCL forms the index as an int, so bit 31 is free on every grid where PCL's arithmetic is
+// defined.
 struct NdtLeaf {
   float cx, cy, cz;
   uint32_t key;
   double mean[3];
   double icov[9];  // row-major (not exactly symmetric, as in PCL)
 };
+
+constexpr uint32_t kNdtLeafInvalid = 0x80000000u;
 
 S3D_HD void ndt_inv3(const double (&a)[3][3], double (&c)[3][3]) {  // Eigen 3x3 inverse: cofactors / determinant
   c[0][0] = a[1][1] * a[2][2] - a[1][2] * a[2][1];
@@ -82,6 +87,49 @@ S3D_HD bool ndt_finalize_leaf(int nr, const double ms[3], const double (&cs)[3][
   double ic[3][3];
   ndt_inv3(cov, ic);
   for (int r = 0; r < 3; ++r) for (int c = 0; c < 3; ++c) icov[3 * r + c] = ic[r][c];
+  return true;
+}
+
+// nr_points >= 0 after applyFilter for a leaf ndt_finalize_leaf accepted: PCL also marks the leaf invalid when
+// icov_.maxCoeff() == inf or icov_.minCoeff() == -inf (folded as std::max / std::min over the row-major entries, as the oracle does)
+S3D_HD bool ndt_icov_usable(const double icov[9]) {
+  double mx = -1.7976931348623157e308, mn = 1.7976931348623157e308;
+  for (int i = 0; i < 9; ++i) { mx = mx < icov[i] ? icov[i] : mx; mn = icov[i] < mn ? icov[i] : mn; }
+  return !(mx == INFINITY || mn == -INFINITY);
+}
+
+// ---- pclomp DIRECT7 neighbourhood (VoxelGridCovariance::getNeighborhoodAtPoint7) -------------------------------------------
+// Offsets in pclomp's order; a query reads its own voxel and the 6 face neighbours, each once, in this order.
+S3D_HD int ndt_direct7_offset(int i, int axis) {
+  return i == 0 ? 0 : ((i - 1) / 2 == axis ? ((i & 1) ? 1 : -1) : 0);
+}
+
+// ijk = (int) floor(p / leaf_size) per axis, float DIVISION (not applyFilter's * inverse_leaf_size).  Returns false for a
+// non-finite coordinate or a cell index outside int32 (PCL's cast is undefined there; here such a point has no neighbours).
+S3D_HD bool ndt_direct7_cell(float x, float y, float z, float leaf, long long ijk[3]) {
+  const float p[3] = {x, y, z};
+  for (int a = 0; a < 3; ++a) {
+#if defined(__CUDA_ARCH__)
+    const float f = floorf(__fdiv_rn(p[a], leaf));
+#else
+    const float f = floorf(p[a] / leaf);
+#endif
+    if (!(f >= -2147483648.0f && f < 2147483648.0f)) return false;
+    ijk[a] = (long long)f;
+  }
+  return true;
+}
+
+// The linear index (ijk + d - min_b) . divb_mul of offset i, or false when min_b <= ijk + d <= max_b fails on some axis
+// (max_b = min_b + div_b - 1).  The caller keeps the leaf under that key only if it exists with nr_points >= 6 and valid.
+S3D_HD bool ndt_direct7_key(const long long ijk[3], int i, const int32_t min_b[3], const int32_t div_b[3], uint32_t mul1, uint32_t mul2,
+                            uint32_t& key) {
+  long long c[3];
+  for (int a = 0; a < 3; ++a) {
+    c[a] = ijk[a] + ndt_direct7_offset(i, a) - min_b[a];
+    if (c[a] < 0 || c[a] >= div_b[a]) return false;
+  }
+  key = (uint32_t)c[0] + (uint32_t)c[1] * mul1 + (uint32_t)c[2] * mul2;
   return true;
 }
 

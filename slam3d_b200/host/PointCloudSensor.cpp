@@ -18,6 +18,9 @@ s3d_context* defaultContext() {
 #ifdef S3D_GICP_USE_BFGS  // built against PCL < 1.14 (shim/CMakeLists.txt): GICP runs that PCL's BFGS inner optimiser
     if (status == S3D_OK) status = s3d_set_gicp_optimizer(ctx, S3D_GICP_BFGS, nullptr);
 #endif
+#ifdef S3D_NDT_OMP_USE_DIRECT7  // shim/CMakeLists.txt: NDT_OMP runs pclomp's default DIRECT7 neighbour search
+    if (status == S3D_OK) status = s3d_set_ndt_omp_search(ctx, S3D_NDT_OMP_DIRECT7, nullptr);
+#endif
     if (status != S3D_OK) err = s3d_last_error();
   });
   if (!ctx) throw std::runtime_error("slam3d_b200: cannot create CUDA context: " + err);
