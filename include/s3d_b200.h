@@ -153,7 +153,7 @@ int s3d_gicp_align_loop_batch(s3d_context* ctx, const s3d_cloud* sources, const 
  *                    vector_bfgs2 with Fletcher's line search).  About 10x the evaluation passes of Newton (DESIGN.md 4).
  * The setting belongs to the context, not to s3d_registration_parameters (which mirrors slam3d's struct field for field): it is a
  * property of the PCL a build replaces.  It applies to every GICP (and GICP_OMP) entry point — s3d_gicp_align, _batch,
- * _loop_batch (coarse and fine), _prepared, _prepared_batch — and NDT ignores it; prepared clouds serve both.  Calls that start
+ * _loop_batch (coarse and fine), _prepared, _prepared_batch, _loop_batch_prepared — and NDT ignores it; prepared clouds serve both.  Calls that start
  * after it returns use the new setting: change it while no call is running on the context.  `previous` (may be NULL) receives the
  * setting it replaces.  Any other value returns S3D_INVALID_ARGUMENT and changes nothing. */
 enum { S3D_GICP_NEWTON = 0, S3D_GICP_BFGS = 1 };
@@ -166,7 +166,7 @@ int s3d_set_gicp_optimizer(s3d_context* ctx, int optimizer, int* previous);
  *                        doNDT): the query's own voxel and its 6 face neighbours, in the order (0,0,0) (+-1,0,0) (0,+-1,0)
  *                        (0,0,+-1), cell = floor(p / leaf size), leaves with >= 6 points that PCL did not mark invalid.
  * Like s3d_set_gicp_optimizer it belongs to the context: it applies to NDT_OMP in every align entry point — s3d_gicp_align,
- * _batch, _loop_batch (coarse and fine each by their own algorithm), _prepared, _prepared_batch — and NDT, GICP and GICP_OMP
+ * _batch, _loop_batch and _loop_batch_prepared (coarse and fine each by their own algorithm), _prepared, _prepared_batch — and NDT, GICP and GICP_OMP
  * ignore it.  Calls that start after it returns use the new setting: change it while no call is running on the context.
  * `previous` (may be NULL) receives the setting it replaces.  Any other value returns S3D_INVALID_ARGUMENT and changes nothing. */
 enum { S3D_NDT_OMP_KDTREE = 0, S3D_NDT_OMP_DIRECT7 = 1 };
@@ -268,6 +268,48 @@ int s3d_build_map(s3d_context* ctx, const s3d_cloud* clouds, const double* poses
  * patch_pose == NULL stops after the accumulation: PointCloudSensor::getAccumulatedCloud (:235-256). */
 int s3d_create_combined_measurement(s3d_context* ctx, const s3d_cloud* clouds, const double* poses, int n, const double patch_pose[16],
                                     float* out_xyzw, uint64_t* n_out);
+
+/* ---- loop closures on device-built patches ---------------------------------------------------------------------------------
+ * A loop-closure call with patches (ScanSensor::link with mPatchBuildingRange > 0) matches patches that share most of their scans,
+ * and one target patch with several candidates.  s3d_prepare_combined_measurements builds every patch of a call on the device, in
+ * one pass from the distinct scans, and prepares each patch under every spec without copying it to the host; the coarse and fine
+ * aligns then run on the handles with s3d_gicp_align_loop_batch_prepared.
+ *
+ * One spec = one kind of handle: exactly one of k and resolution is set.
+ *   k in [1, 4096], resolution 0   a GICP handle, as s3d_prepare_clouds(density, k) makes
+ *   k 0, resolution > 0 and finite an NDT handle, as s3d_prepare_clouds_ndt(density, resolution) makes
+ * density must not be NaN. */
+typedef struct s3d_prepare_spec {
+  double  density;
+  int32_t k;
+  float   resolution;
+} s3d_prepare_spec;
+
+/* n_patches patches from n_scans distinct scans.  Patch p has the members patch_first_member[p] .. patch_first_member[p + 1] - 1
+ * (patch_first_member holds n_patches + 1 entries, starts at 0 and does not decrease); member m is scan member_scan[m] at pose
+ * member_poses[16 m] (pose_i = vertex.correctedPose * measurement.sensorPose).  patch_poses = n_patches x 16 doubles, or NULL for
+ * the accumulated clouds only.  Each patch is exactly the cloud s3d_create_combined_measurement returns for the same list and
+ * patch pose, and is prepared under every spec: out[p * n_specs + s] receives the handle of patch p under specs[s], the same
+ * handle (size, and bit for bit every align on it) as s3d_prepare_clouds / s3d_prepare_clouds_ndt of that cloud gives.
+ * Every referenced scan is uploaded once however many patches hold it (host or device pointers, as everywhere); the patches stay
+ * on the device.  All-or-nothing like s3d_prepare_clouds.  A bad device slot, a bad spec, a member scan index out of range, a
+ * malformed patch_first_member or more than 2^31 - 1 patch points in all: S3D_INVALID_ARGUMENT and no handle. */
+int s3d_prepare_combined_measurements(s3d_context* ctx, int device_slot, const s3d_cloud* scans, int n_scans, const int32_t* member_scan,
+                                      const double* member_poses, const int32_t* patch_first_member, const double* patch_poses, int n_patches,
+                                      const s3d_prepare_spec* specs, int n_specs, s3d_prepared_cloud** out);
+
+/* s3d_gicp_align_loop_batch on prepared clouds: createConstraint(source, target, odometry, loop = true) (PointCloudSensor.cpp:286-292)
+ * for n_pairs pairs.  The coarse pass aligns coarse_sources[i] with coarse_targets[i] from guesses[16 i] with `coarse`; the fine
+ * pass aligns fine_sources[i] with fine_targets[i] from the coarse pose with `fine`.  out_fine[i] = out_coarse[i] when the coarse
+ * align of pair i fails (its fine align does not run); out_coarse may be NULL.  Each pass checks its handles against its own
+ * parameters as s3d_gicp_align_prepared_batch does (status 6 on a density, k or resolution that does not match, or on handles of
+ * different devices); the context's GICP optimiser and NDT_OMP search apply to each pass by its own algorithm.  Results are
+ * bit-identical to s3d_gicp_align_loop_batch on the raw clouds the handles were prepared from. */
+int s3d_gicp_align_loop_batch_prepared(s3d_context* ctx, const s3d_prepared_cloud* const* coarse_sources,
+                                       const s3d_prepared_cloud* const* coarse_targets, const s3d_prepared_cloud* const* fine_sources,
+                                       const s3d_prepared_cloud* const* fine_targets, const double* guesses,
+                                       const s3d_registration_parameters* coarse, const s3d_registration_parameters* fine, int n_pairs,
+                                       s3d_result* out_coarse, s3d_result* out_fine);
 
 /* ---- ground plane (PointCloudSensor::fillGroundPlane, PointCloudSensor.cpp:362-388) ---------------------------------------
  * pcl::RandomSampleConsensus + SampleConsensusModelPlane (DESIGN.md 6f): coefficients[4] = (a, b, c, d), unit normal.

@@ -10,7 +10,7 @@ import os
 import numpy as np
 
 from . import _abi
-from ._abi import Cloud, Counters, RegistrationParameters, Result  # noqa: F401
+from ._abi import Cloud, Counters, PrepareSpec, RegistrationParameters, Result  # noqa: F401
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("S3D_LIB_PATH", os.path.join(_HERE, "libs3d_b200.so"))  # override: kernel-variant experiments only
@@ -69,6 +69,11 @@ def lib():
         L.s3d_gicp_align_prepared.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RegistrationParameters), C.POINTER(Result)]
         L.s3d_gicp_align_prepared_batch.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_void_p,
                                                     C.POINTER(RegistrationParameters), C.c_int, C.POINTER(Result)]
+        L.s3d_prepare_combined_measurements.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                        C.c_void_p, C.c_int, C.POINTER(PrepareSpec), C.c_int, C.POINTER(C.c_void_p)]
+        L.s3d_gicp_align_loop_batch_prepared.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
+                                                         C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(RegistrationParameters),
+                                                         C.POINTER(RegistrationParameters), C.c_int, C.POINTER(Result), C.POINTER(Result)]
         _lib = L
     return _lib
 
@@ -350,6 +355,53 @@ def _gicp_align_prepared_batch(self, sources, targets, guesses=None, params=None
     return list(res)
 
 
+def _prepare_combined_measurements(self, scans, patches, specs, device_slot=0):
+    """createCombinedMeasurement of every patch, built on the device from `scans` (each uploaded once) and prepared under every
+    spec without a copy to the host (s3d_prepare_combined_measurements).  patches: list of (member scan indices, member poses,
+    patch_pose); patch_pose None for all patches stops after the accumulation (getAccumulatedCloud).  specs: list of
+    (density, k, resolution): k set and resolution None / 0 for a GICP handle, k 0 and resolution set for an NDT handle.
+    Returns PreparedClouds as [patch][spec]."""
+    n_scans, n_patches, n_specs = len(scans), len(patches), len(specs)
+    keep = []
+    cc = (Cloud * max(n_scans, 1))()
+    for i in range(n_scans):
+        a, c = _cloud(self, scans[i]); keep.append(a); cc[i] = c
+    with_pose = [p[2] is not None for p in patches]
+    if any(with_pose) and not all(with_pose):
+        raise ValueError("patch_pose must be given for every patch or for none")
+    members = [int(s) for p in patches for s in p[0]]
+    first = np.cumsum([0] + [len(p[0]) for p in patches]).astype(np.int32)
+    if any(len(p[0]) != len(p[1]) for p in patches):
+        raise ValueError("every member scan needs its pose")
+    ms = np.ascontiguousarray(np.asarray(members if members else [0], np.int32))
+    mp = np.ascontiguousarray(np.stack([_colmajor(T) for p in patches for T in p[1]])) if members else np.zeros((1, 4, 4))
+    pp = np.ascontiguousarray(np.stack([_colmajor(p[2]) for p in patches])) if n_patches and all(with_pose) else None
+    sp = (PrepareSpec * max(n_specs, 1))()
+    meta = []
+    for i, (density, k, resolution) in enumerate(specs):
+        r = float(resolution or 0.0)
+        sp[i] = PrepareSpec(float(density), int(k), r)
+        meta.append((float(density), int(k), float(C.c_float(r).value) if r else None))
+    hh = (C.c_void_p * max(n_patches * n_specs, 1))()
+    st = lib().s3d_prepare_combined_measurements(self._h, device_slot, cc, n_scans, ms.ctypes.data, mp.ctypes.data, first.ctypes.data,
+                                                  pp.ctypes.data if pp is not None else None, n_patches, sp, n_specs, hh)
+    self._check(st, "s3d_prepare_combined_measurements")
+    return [[PreparedCloud(self, C.c_void_p(hh[p * n_specs + s]), *meta[s]) for s in range(n_specs)] for p in range(n_patches)]
+
+
+def _gicp_align_loop_batch_prepared(self, coarse_sources, coarse_targets, fine_sources, fine_targets, guesses, coarse, fine):
+    """createConstraint(loop=true) on prepared clouds: coarse align on the coarse handles, then fine align on the fine handles from
+    the coarse pose (s3d_gicp_align_loop_batch_prepared).  Returns (coarse, fine) result lists."""
+    n = len(coarse_sources)
+    hs = [(C.c_void_p * max(n, 1))(*[h._h for h in x]) for x in (coarse_sources, coarse_targets, fine_sources, fine_targets)]
+    g = np.ascontiguousarray(np.stack([_colmajor(None if guesses is None else guesses[i]) for i in range(n)])) if n else np.zeros((1, 4, 4))
+    rc = (Result * max(n, 1))()
+    rf = (Result * max(n, 1))()
+    st = lib().s3d_gicp_align_loop_batch_prepared(self._h, hs[0], hs[1], hs[2], hs[3], g.ctypes.data, C.byref(coarse), C.byref(fine), n, rc, rf)
+    self._check(st, "s3d_gicp_align_loop_batch_prepared")
+    return list(rc)[:n], list(rf)[:n]
+
+
 def _transform_cloud(self, cloud, T):
     a, c = _cloud(self, cloud)
     t = _colmajor(T)
@@ -445,6 +497,8 @@ Context.prepare_cloud_ndt = _prepare_cloud_ndt
 Context.prepare_clouds_ndt = _prepare_clouds_ndt
 Context.gicp_align_prepared = _gicp_align_prepared
 Context.gicp_align_prepared_batch = _gicp_align_prepared_batch
+Context.prepare_combined_measurements = _prepare_combined_measurements
+Context.gicp_align_loop_batch_prepared = _gicp_align_loop_batch_prepared
 
 
 def last_error():

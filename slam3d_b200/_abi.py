@@ -73,5 +73,10 @@ class Result(C.Structure):
         return np.array(self.T[:], dtype=np.float64).reshape(4, 4).T.copy()  # column-major -> [row, col]
 
 
+class PrepareSpec(C.Structure):
+    """s3d_prepare_spec: one kind of prepared handle, GICP (k set, resolution 0) or NDT (k 0, resolution set)."""
+    _fields_ = [("density", C.c_double), ("k", C.c_int32), ("resolution", C.c_float)]
+
+
 class Counters(C.Structure):
     _fields_ = [("kernel_launches", C.c_uint64), ("h2d_bytes", C.c_uint64), ("d2h_bytes", C.c_uint64)]

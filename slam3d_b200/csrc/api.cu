@@ -835,11 +835,11 @@ static void align_prepared_chunk(s3d_context* ctx, int slot, const s3d_prepared_
 }
 }  // namespace s3d
 
-int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* const* sources, const s3d_prepared_cloud* const* targets,
-                                  const double* guesses, const s3d_registration_parameters* params, int n_pairs, s3d_result* out) {
-  if (!ctx || !params || !out || n_pairs < 0 || (n_pairs > 0 && (!sources || !targets || !guesses))) return S3D_INVALID_ARGUMENT;
-  if (n_pairs == 0) return S3D_OK;
-  const int slot = sources[0] ? sources[0]->device_slot : 0;
+namespace s3d {
+// The handle checks of an align on prepared clouds with `params`: every handle on device slot `slot`, of the density (and GICP: k;
+// NDT: the source's resolution) that `params` asks for.
+static int check_prepared(const s3d_prepared_cloud* const* sources, const s3d_prepared_cloud* const* targets, const s3d_registration_parameters* params,
+                          int n_pairs, int slot) {
   const int alg = effective_algorithm(params->registration_algorithm);
   for (int i = 0; i < n_pairs; ++i) {
     if (!sources[i] || !targets[i]) return S3D_INVALID_ARGUMENT;
@@ -859,6 +859,17 @@ int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* co
       return S3D_INVALID_ARGUMENT;
     }
   }
+  return S3D_OK;
+}
+
+// Chunks of the n_pairs pairs on `streams_small` worker threads.  With `fine` set, a chunk runs createConstraint's loop-closure
+// sequence (PointCloudSensor.cpp:286-292) on it: the pairs whose coarse align succeeded are aligned again with `fine` on the fine
+// handles from the coarse pose, the others keep the coarse result (the reference throws there), so one chunk's fine pass overlaps
+// the other chunks' coarse pass.
+static int align_prepared_impl(s3d_context* ctx, int slot, const s3d_prepared_cloud* const* sources, const s3d_prepared_cloud* const* targets,
+                               const double* guesses, const s3d_registration_parameters* params, int n_pairs, s3d_result* out,
+                               const s3d_prepared_cloud* const* fine_sources = nullptr, const s3d_prepared_cloud* const* fine_targets = nullptr,
+                               const s3d_registration_parameters* fine = nullptr, s3d_result* out_fine = nullptr) {
   const int W = std::max(1, ctx->streams_small);
   std::vector<int> st(W, S3D_OK);
   std::vector<std::string> errs(W);
@@ -874,6 +885,19 @@ int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* co
         if (b >= n_pairs) break;
         const int n = std::min(chunk, n_pairs - b);
         align_prepared_chunk(ctx, slot, sources + b, targets + b, guesses + 16 * (size_t)b, *params, n, out + b);
+        if (!fine) continue;
+        std::vector<const s3d_prepared_cloud*> fs, ft;
+        std::vector<double> g;
+        std::vector<int> idx;
+        for (int i = b; i < b + n; ++i) {
+          if (out[i].status != S3D_OK) { out_fine[i] = out[i]; continue; }  // :286-289: the coarse align threw
+          idx.push_back(i); fs.push_back(fine_sources[i]); ft.push_back(fine_targets[i]);
+          g.insert(g.end(), out[i].T, out[i].T + 16);
+        }
+        if (idx.empty()) continue;
+        std::vector<s3d_result> r(idx.size());
+        align_prepared_chunk(ctx, slot, fs.data(), ft.data(), g.data(), *fine, (int)idx.size(), r.data());
+        for (size_t j = 0; j < idx.size(); ++j) out_fine[idx[j]] = r[j];
       }
       return S3D_OK;
     });
@@ -885,6 +909,33 @@ int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* co
   for (int w = 0; w < W; ++w) if (st[w] != S3D_OK) { set_error(errs[w]); return st[w]; }
   for (int w = 0; w < W; ++w) if (!errs[w].empty()) { set_error(errs[w]); break; }
   return S3D_OK;
+}
+}  // namespace s3d
+
+int s3d_gicp_align_prepared_batch(s3d_context* ctx, const s3d_prepared_cloud* const* sources, const s3d_prepared_cloud* const* targets,
+                                  const double* guesses, const s3d_registration_parameters* params, int n_pairs, s3d_result* out) {
+  if (!ctx || !params || !out || n_pairs < 0 || (n_pairs > 0 && (!sources || !targets || !guesses))) return S3D_INVALID_ARGUMENT;
+  if (n_pairs == 0) return S3D_OK;
+  const int slot = sources[0] ? sources[0]->device_slot : 0;
+  if (const int st = check_prepared(sources, targets, params, n_pairs, slot)) return st;
+  return align_prepared_impl(ctx, slot, sources, targets, guesses, params, n_pairs, out);
+}
+
+int s3d_gicp_align_loop_batch_prepared(s3d_context* ctx, const s3d_prepared_cloud* const* coarse_sources,
+                                       const s3d_prepared_cloud* const* coarse_targets, const s3d_prepared_cloud* const* fine_sources,
+                                       const s3d_prepared_cloud* const* fine_targets, const double* guesses,
+                                       const s3d_registration_parameters* coarse, const s3d_registration_parameters* fine, int n_pairs,
+                                       s3d_result* out_coarse, s3d_result* out_fine) {
+  if (!ctx || !coarse || !fine || !out_fine || n_pairs < 0 ||
+      (n_pairs > 0 && (!coarse_sources || !coarse_targets || !fine_sources || !fine_targets || !guesses)))
+    return S3D_INVALID_ARGUMENT;
+  if (n_pairs == 0) return S3D_OK;
+  const int slot = coarse_sources[0] ? coarse_sources[0]->device_slot : 0;
+  if (const int st = check_prepared(coarse_sources, coarse_targets, coarse, n_pairs, slot)) return st;
+  if (const int st = check_prepared(fine_sources, fine_targets, fine, n_pairs, slot)) return st;
+  std::vector<s3d_result> tmp;
+  if (!out_coarse) { tmp.resize(n_pairs); out_coarse = tmp.data(); }
+  return align_prepared_impl(ctx, slot, coarse_sources, coarse_targets, guesses, coarse, n_pairs, out_coarse, fine_sources, fine_targets, fine, out_fine);
 }
 
 int s3d_gicp_align_prepared(s3d_context* ctx, const s3d_prepared_cloud* source, const s3d_prepared_cloud* target, const double guess[16],
@@ -899,6 +950,15 @@ int s3d_gicp_align_prepared(s3d_context* ctx, const s3d_prepared_cloud* source, 
 }
 
 // ---- patch and map building ------------------------------------------------------------------------------------------
+namespace s3d {
+// pose.inverse() of an Eigen::Isometry3d: [R^T | -R^T t]  (the patch_pose.inverse() of createCombinedMeasurement, :264)
+static void isometry_inverse(const double* T, double* inv) {
+  for (int r = 0; r < 3; ++r) for (int c = 0; c < 3; ++c) inv[c * 4 + r] = T[r * 4 + c];
+  for (int r = 0; r < 3; ++r) { double s = 0; for (int c = 0; c < 3; ++c) s += inv[c * 4 + r] * T[12 + c]; inv[12 + r] = -s; }
+  inv[3] = inv[7] = inv[11] = 0; inv[15] = 1;
+}
+}  // namespace s3d
+
 int s3d_transform_cloud(s3d_context* ctx, s3d_cloud in, const double T[16], float* out_xyzw) {
   if (!ctx || !T || (in.n && !out_xyzw)) return S3D_INVALID_ARGUMENT;
   if (in.n == 0) return S3D_OK;
@@ -923,18 +983,68 @@ int s3d_create_combined_measurement(s3d_context* ctx, const s3d_cloud* clouds, c
     std::vector<const float*> ptrs(n);
     std::vector<uint64_t> sizes(n);
     for (int i = 0; i < n; ++i) { ptrs[i] = clouds[i].xyzw; sizes[i] = clouds[i].n; }
-    // pose.inverse() of an Eigen::Isometry3d: [R^T | -R^T t]
     double inv[16];
-    if (patch_pose) {
-      for (int r = 0; r < 3; ++r) for (int c = 0; c < 3; ++c) inv[c * 4 + r] = patch_pose[r * 4 + c];
-      for (int r = 0; r < 3; ++r) { double s = 0; for (int c = 0; c < 3; ++c) s += inv[c * 4 + r] * patch_pose[12 + c]; inv[12 + r] = -s; }
-      inv[3] = inv[7] = inv[11] = 0; inv[15] = 1;
-    }
+    if (patch_pose) isometry_inverse(patch_pose, inv);
     const uint32_t m = run_accumulate(ws, ptrs, sizes, poses, patch_pose ? inv : nullptr);
     if (m && !out_xyzw) return S3D_INVALID_ARGUMENT;
     copy_out(ws, out_xyzw, ws.accu.p, 16 * (size_t)m);
     ws.sync();
     *n_out = m;
+    return S3D_OK;
+  });
+}
+
+int s3d_prepare_combined_measurements(s3d_context* ctx, int device_slot, const s3d_cloud* scans, int n_scans, const int32_t* member_scan,
+                                      const double* member_poses, const int32_t* patch_first_member, const double* patch_poses, int n_patches,
+                                      const s3d_prepare_spec* specs, int n_specs, s3d_prepared_cloud** out) {
+  if (!ctx || !out || n_patches < 0 || n_specs < 0 || n_scans < 0) return S3D_INVALID_ARGUMENT;
+  const size_t n_out = (size_t)n_patches * (size_t)n_specs;
+  for (size_t i = 0; i < n_out; ++i) out[i] = nullptr;
+  auto invalid = [](const char* msg) { set_error(msg); return (int)S3D_INVALID_ARGUMENT; };
+  if (device_slot < 0 || device_slot >= (int)ctx->devs.size()) return invalid("bad device slot");
+  if ((n_specs > 0 && !specs) || (n_patches > 0 && !patch_first_member) || (n_scans > 0 && !scans)) return invalid("missing table");
+  for (int s = 0; s < n_specs; ++s) {
+    const s3d_prepare_spec& sp = specs[s];
+    if (std::isnan(sp.density)) return invalid("point_cloud_density must not be NaN");
+    if (!std::isfinite(sp.resolution) || sp.resolution < 0.f) return invalid("NDT resolution must be positive and finite");
+    if (sp.resolution > 0.f ? sp.k != 0 : (sp.k < 1 || sp.k > kMaxK))
+      return invalid("a spec sets either k in [1, 4096] (GICP) or a positive resolution (NDT)");
+  }
+  for (int i = 0; i < n_scans; ++i) if (scans[i].n && !scans[i].xyzw) return invalid("scan without points pointer");
+  if (n_patches == 0) return S3D_OK;
+  if (patch_first_member[0] != 0) return invalid("patch_first_member[0] must be 0");
+  for (int p = 0; p < n_patches; ++p) if (patch_first_member[p + 1] < patch_first_member[p]) return invalid("patch_first_member decreases");
+  const int32_t n_members = patch_first_member[n_patches];
+  if (n_members > 0 && (!member_scan || !member_poses)) return invalid("missing member table");
+  uint64_t total = 0;
+  for (int32_t m = 0; m < n_members; ++m) {
+    if (member_scan[m] < 0 || member_scan[m] >= n_scans) return invalid("member scan index out of range");
+    total += scans[member_scan[m]].n;
+  }
+  if (total >= (1ull << 31)) return invalid("patches too large: more than 2^31 - 1 points");
+  if (n_specs == 0) return S3D_OK;
+  return guarded([&]() -> int {
+    WsLease lease(ctx, device_slot);  // holds the patches (ws.accu) until every spec is prepared
+    Workspace& ws = *lease;
+    std::vector<double> inv(patch_poses ? 16 * (size_t)n_patches : 0);
+    for (int p = 0; patch_poses && p < n_patches; ++p) isometry_inverse(patch_poses + 16 * (size_t)p, &inv[16 * (size_t)p]);
+    std::vector<uint64_t> off;
+    const float4* pts = run_patch_gather(ws, scans, member_scan, member_poses, patch_first_member, patch_poses ? inv.data() : nullptr,
+                                         (uint32_t)n_patches, off);
+    std::vector<s3d_cloud> patches(n_patches);
+    for (int p = 0; p < n_patches; ++p) patches[p] = s3d_cloud{reinterpret_cast<const float*>(pts + off[p]), off[p + 1] - off[p]};
+    std::vector<s3d_prepared_cloud*> h(n_patches);
+    for (int s = 0; s < n_specs; ++s) {
+      const s3d_prepare_spec& sp = specs[s];
+      const int st = prepare_clouds(ctx, device_slot, patches.data(), n_patches, sp.density, sp.resolution > 0.f ? 0 : sp.k, sp.resolution, h.data());
+      if (st != S3D_OK) {
+        const std::string err = s3d_last_error();
+        for (size_t i = 0; i < n_out; ++i) { s3d_release_cloud(ctx, out[i]); out[i] = nullptr; }
+        set_error(err);
+        return st;
+      }
+      for (int p = 0; p < n_patches; ++p) out[(size_t)p * n_specs + s] = h[p];
+    }
     return S3D_OK;
   });
 }

@@ -6,6 +6,7 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdint>
+#include <cstring>
 #include <map>
 #include <mutex>
 #include <string>
@@ -267,6 +268,10 @@ void run_expand_cov(Workspace& ws, double* cov_out);  // full 3x3 covariances pe
 void run_nn_stage(Workspace& ws, uint32_t ref_slot, uint32_t qry_slot, const float* T16_dev, uint32_t* nn_index, float* nn_dist2);
 uint32_t run_accumulate(Workspace& ws, const std::vector<const float*>& clouds, const std::vector<uint64_t>& sizes, const double* poses,
                         const double* second = nullptr);  // -> ws.accu; second: one more 4x4 applied to every (float-rounded) point
+// map.cu: every patch of s3d_prepare_combined_measurements (arguments as there, validated) into ws.accu; patch p is
+// [patch_off[p], patch_off[p + 1]).  patch_inv: n_patches x 16 doubles of patch_pose.inverse(), or NULL.  Synchronises ws.
+const float4* run_patch_gather(Workspace& ws, const s3d_cloud* scans, const int32_t* member_scan, const double* member_poses,
+                               const int32_t* patch_first_member, const double* patch_inv, uint32_t n_patches, std::vector<uint64_t>& patch_off);
 uint32_t run_radius_filter(Workspace& ws, const float4* dev_in, uint32_t n, double radius, unsigned min_pts, float4* dev_out);
 // map.cu: exclusive scan of n_tiles per-tile counts in place (one warp); *total = their sum
 __global__ void keep_scan_kernel(uint32_t n_tiles, uint32_t* __restrict__ tile_counts, uint32_t* __restrict__ total);

@@ -12,36 +12,63 @@
 namespace s3d {
 
 // pcl::transformPointCloud(cloud, out, Matrix4d): double se3 form  x*c0 + (y*c1 + (z*c2 + c3)), cast to float.
-// poses: n_slots x 16 doubles (column-major); out_off: first output index of every slot (clouds are concatenated unpadded).
 // second: optional 16 doubles applied to the (float-rounded) result of the first transform — createCombinedMeasurement's
 // transformPointCloud(accumulated, shifted, pose.inverse()) fused into the same pass, with both float roundings kept.
+// The one body of both kernels below: the patch path gives the points of s3d_create_combined_measurement bit for bit.
+struct Se3d { double t0, t1, t2, t4, t5, t6, t8, t9, t10, t12, t13, t14; };
+__device__ __forceinline__ Se3d load_se3d(const double* T) {
+  return Se3d{T[0], T[1], T[2], T[4], T[5], T[6], T[8], T[9], T[10], T[12], T[13], T[14]};
+}
+__device__ __forceinline__ float4 combined_point(float4 p, const Se3d& T, const double* __restrict__ second) {
+  const double x = p.x, y = p.y, z = p.z;
+  float4 o;
+  o.x = (float)__dadd_rn(__dmul_rn(x, T.t0), __dadd_rn(__dmul_rn(y, T.t4), __dadd_rn(__dmul_rn(z, T.t8), T.t12)));
+  o.y = (float)__dadd_rn(__dmul_rn(x, T.t1), __dadd_rn(__dmul_rn(y, T.t5), __dadd_rn(__dmul_rn(z, T.t9), T.t13)));
+  o.z = (float)__dadd_rn(__dmul_rn(x, T.t2), __dadd_rn(__dmul_rn(y, T.t6), __dadd_rn(__dmul_rn(z, T.t10), T.t14)));
+  o.w = 1.0f;
+  if (second) {
+    const double u = o.x, v = o.y, w = o.z;
+    o.x = (float)__dadd_rn(__dmul_rn(u, second[0]), __dadd_rn(__dmul_rn(v, second[4]), __dadd_rn(__dmul_rn(w, second[8]), second[12])));
+    o.y = (float)__dadd_rn(__dmul_rn(u, second[1]), __dadd_rn(__dmul_rn(v, second[5]), __dadd_rn(__dmul_rn(w, second[9]), second[13])));
+    o.z = (float)__dadd_rn(__dmul_rn(u, second[2]), __dadd_rn(__dmul_rn(v, second[6]), __dadd_rn(__dmul_rn(w, second[10]), second[14])));
+  }
+  return o;
+}
+
+// poses: n_slots x 16 doubles (column-major); out_off: first output index of every slot (clouds are concatenated unpadded).
 __global__ void __launch_bounds__(kSortThreads) transform_concat_kernel(const SlotInfo* __restrict__ slots, TileMap tm, const double* __restrict__ poses,
                                                                         const uint32_t* __restrict__ out_off, float4* __restrict__ out,
                                                                         const double* __restrict__ second) {
   const uint32_t t = blockIdx.x;
   const uint32_t slot = tm.tile_slot[t], first = tm.tile_first[t];
   const SlotInfo& si = slots[slot];
-  const double* T = poses + 16 * (size_t)slot;
-  const double t0 = T[0], t1 = T[1], t2 = T[2], t4 = T[4], t5 = T[5], t6 = T[6], t8 = T[8], t9 = T[9], t10 = T[10], t12 = T[12], t13 = T[13], t14 = T[14];
+  const Se3d T = load_se3d(poses + 16 * (size_t)slot);
 #pragma unroll
   for (int j = 0; j < kSortTile / kSortThreads; ++j) {
     const uint32_t e = first + j * kSortThreads + threadIdx.x;
-    if (e < si.n_raw) {
-      const float4 p = si.raw[e];
-      const double x = p.x, y = p.y, z = p.z;
-      float4 o;
-      o.x = (float)__dadd_rn(__dmul_rn(x, t0), __dadd_rn(__dmul_rn(y, t4), __dadd_rn(__dmul_rn(z, t8), t12)));
-      o.y = (float)__dadd_rn(__dmul_rn(x, t1), __dadd_rn(__dmul_rn(y, t5), __dadd_rn(__dmul_rn(z, t9), t13)));
-      o.z = (float)__dadd_rn(__dmul_rn(x, t2), __dadd_rn(__dmul_rn(y, t6), __dadd_rn(__dmul_rn(z, t10), t14)));
-      o.w = 1.0f;
-      if (second) {
-        const double u = o.x, v = o.y, w = o.z;
-        o.x = (float)__dadd_rn(__dmul_rn(u, second[0]), __dadd_rn(__dmul_rn(v, second[4]), __dadd_rn(__dmul_rn(w, second[8]), second[12])));
-        o.y = (float)__dadd_rn(__dmul_rn(u, second[1]), __dadd_rn(__dmul_rn(v, second[5]), __dadd_rn(__dmul_rn(w, second[9]), second[13])));
-        o.z = (float)__dadd_rn(__dmul_rn(u, second[2]), __dadd_rn(__dmul_rn(v, second[6]), __dadd_rn(__dmul_rn(w, second[10]), second[14])));
-      }
-      out[out_off[slot] + e] = o;
-    }
+    if (e < si.n_raw) out[out_off[slot] + e] = combined_point(si.raw[e], T, second);
+  }
+}
+
+// Member m of a multi-patch build: distinct scan `scan` (a slot of the batch), its pose at poses[16 m], its patch's
+// patch_pose.inverse() at patch_inv[16 patch] (patch_inv NULL: getAccumulatedCloud), first output index `out`.
+struct PatchMember { uint32_t scan, patch, out, reserved; };
+
+// Every patch of a call in one launch: tile t covers points [tile_first, +kSortTile) of member tile_slot[t].  Each scan is read
+// from where it was staged once, however many patches it belongs to; the patches land back to back in `out`.
+__global__ void __launch_bounds__(kSortThreads) patch_gather_kernel(const SlotInfo* __restrict__ scans, TileMap tm, const PatchMember* __restrict__ members,
+                                                                    const double* __restrict__ poses, const double* __restrict__ patch_inv,
+                                                                    float4* __restrict__ out) {
+  const uint32_t t = blockIdx.x;
+  const uint32_t m = tm.tile_slot[t], first = tm.tile_first[t];
+  const PatchMember pm = members[m];
+  const SlotInfo& si = scans[pm.scan];
+  const Se3d T = load_se3d(poses + 16 * (size_t)m);
+  const double* second = patch_inv ? patch_inv + 16 * (size_t)pm.patch : nullptr;
+#pragma unroll
+  for (int j = 0; j < kSortTile / kSortThreads; ++j) {
+    const uint32_t e = first + j * kSortThreads + threadIdx.x;
+    if (e < si.n_raw) out[pm.out + e] = combined_point(si.raw[e], T, second);
   }
 }
 
@@ -157,6 +184,62 @@ uint32_t run_accumulate(Workspace& ws, const std::vector<const float*>& clouds, 
   S3D_CUDA(cudaGetLastError());
   ws.sync();  // `off` and the pageable `poses` must outlive the copies
   return (uint32_t)total;
+}
+
+// Patches of s3d_prepare_combined_measurements -> ws.accu (device), patch p at patch_off[p] (n_patches + 1 entries).  Only the
+// scans some member references are staged (setup_batch: pinned bounce for pageable memory, device pointers read in place), each
+// once; the tables go up in one copy.  Returns after the kernel has finished, so other streams may read ws.accu.
+const float4* run_patch_gather(Workspace& ws, const s3d_cloud* scans, const int32_t* member_scan, const double* member_poses,
+                               const int32_t* patch_first_member, const double* patch_inv, uint32_t n_patches, std::vector<uint64_t>& patch_off) {
+  const uint32_t n_members = (uint32_t)patch_first_member[n_patches];
+  std::map<int32_t, uint32_t> slot_of;  // scan index -> slot of the staged batch, in first-use order
+  std::vector<const float*> ptrs;
+  std::vector<uint64_t> sizes;
+  std::vector<PatchMember> members(n_members);
+  patch_off.assign(n_patches + 1, 0);
+  uint64_t total = 0;
+  for (uint32_t p = 0; p < n_patches; ++p) {
+    patch_off[p] = total;
+    for (int32_t m = patch_first_member[p]; m < patch_first_member[p + 1]; ++m) {
+      const int32_t s = member_scan[m];
+      auto it = slot_of.find(s);
+      if (it == slot_of.end()) {
+        it = slot_of.emplace(s, (uint32_t)ptrs.size()).first;
+        ptrs.push_back(scans[s].xyzw); sizes.push_back(scans[s].n);
+      }
+      members[m] = PatchMember{it->second, p, (uint32_t)total, 0};
+      total += scans[s].n;
+    }
+  }
+  patch_off[n_patches] = total;
+  if (total >= (1ull << 31)) throw CudaError{"patches too large: more than 2^31 points"};
+  setup_batch(ws, ptrs, sizes, 0);
+  ws.accu.reserve(16 * std::max<uint64_t>(total, 4));
+  if (total == 0) return ws.accu.as<float4>();
+  std::vector<uint32_t> tile_slot, tile_first;
+  for (uint32_t m = 0; m < n_members; ++m)
+    for (uint64_t f = 0; f < sizes[members[m].scan]; f += kSortTile) { tile_slot.push_back(m); tile_first.push_back((uint32_t)f); }
+  const uint32_t n_tiles = (uint32_t)tile_slot.size();
+  // one table block: member poses | patch inverses | members | tile_slot | tile_first
+  const size_t b_pose = 128 * (size_t)n_members, b_inv = patch_inv ? 128 * (size_t)n_patches : 0, b_mem = sizeof(PatchMember) * n_members;
+  std::vector<char> tab(b_pose + b_inv + b_mem + 8 * (size_t)n_tiles);
+  memcpy(tab.data(), member_poses, b_pose);
+  if (patch_inv) memcpy(tab.data() + b_pose, patch_inv, b_inv);
+  memcpy(tab.data() + b_pose + b_inv, members.data(), b_mem);
+  memcpy(tab.data() + b_pose + b_inv + b_mem, tile_slot.data(), 4 * (size_t)n_tiles);
+  memcpy(tab.data() + b_pose + b_inv + b_mem + 4 * (size_t)n_tiles, tile_first.data(), 4 * (size_t)n_tiles);
+  ws.map_aux.reserve(tab.size());
+  char* d = ws.map_aux.as<char>();
+  S3D_CUDA(cudaMemcpyAsync(d, tab.data(), tab.size(), cudaMemcpyHostToDevice, ws.stream));
+  ws.h2d += tab.size();
+  TileMap tm{reinterpret_cast<const uint32_t*>(d + b_pose + b_inv + b_mem), reinterpret_cast<const uint32_t*>(d + b_pose + b_inv + b_mem) + n_tiles, n_tiles};
+  patch_gather_kernel<<<n_tiles, kSortThreads, 0, ws.stream>>>(ws.slots.as<SlotInfo>(), tm, reinterpret_cast<const PatchMember*>(d + b_pose + b_inv),
+                                                               reinterpret_cast<const double*>(d), patch_inv ? reinterpret_cast<const double*>(d + b_pose) : nullptr,
+                                                               ws.accu.as<float4>());
+  ++ws.launches;
+  S3D_CUDA(cudaGetLastError());
+  ws.sync();  // `tab` must outlive the copy, and the prepare pass reads the patches from other streams
+  return ws.accu.as<float4>();
 }
 
 // RadiusOutlierRemoval of the n points at dev_in (device) into dev_out (device, capacity n); returns the number kept

@@ -11,7 +11,9 @@
 // mPatchBuildingRange hops of a vertex (BoostGraph::getVerticesInRange, graph/boost/BoostGraph.cpp:274-299, vertex-id order),
 // accumulated and re-expressed in the vertex' frame by PointCloudSensor::createCombinedMeasurement.
 // linkLastToNeighbors(true) hands all candidates of a vertex to PointCloudSensor::createConstraints — ONE device batch through
-// s3d_gicp_align_loop_batch — instead of one createConstraint per candidate; edges and warnings are the same.
+// s3d_gicp_align_loop_batch — instead of one createConstraint per candidate; edges and warnings are the same.  With
+// setDevicePatches(true) and patches, that batch goes through PointCloudSensor::createLoopConstraints: the patches are built and
+// prepared on the device and never copied to the host.
 #pragma once
 
 #include <cmath>
@@ -98,6 +100,12 @@ class MiniHost {
   // ScanSensor::buildPatch(source)  :215-270 with mPatchSolver == NULL
   Measurement::Ptr buildPatch(unsigned source) const {
     if (mPatchBuildingRange == 0) return mMeasurements[source];  // :217-220
+    const PointCloudSensor::Patch p = patchOf(source);
+    return mSensor->createCombinedMeasurement(p.vertices, p.pose);  // :269
+  }
+
+  // the arguments buildPatch hands to createCombinedMeasurement (mPatchBuildingRange > 0)
+  PointCloudSensor::Patch patchOf(unsigned source) const {
     // Graph::getVerticesInRange: breadth-first search to depth mPatchBuildingRange, result in vertex order (std::map<Vertex, depth>)
     std::map<unsigned, unsigned> depth;
     depth[source] = 0;
@@ -109,7 +117,7 @@ class MiniHost {
     }
     PointCloudSensor::PosedMeasurements v_objects;
     for (const auto& d : depth) v_objects.emplace_back(std::dynamic_pointer_cast<PointCloudMeasurement>(mMeasurements[d.first]), mCorrected[d.first]);
-    return mSensor->createCombinedMeasurement(v_objects, mCorrected[source]);  // :269
+    return PointCloudSensor::Patch{v_objects, mCorrected[source]};
   }
 
   // ScanSensor::link(source_id, target_id, guess)  :144-168
@@ -152,10 +160,17 @@ class MiniHost {
     if (batched) {
       for (auto i = neighbors.rbegin(); i != neighbors.rend() && (int)batch.size() < mMaxNeighorLinks; ++i) if (qualifies(*i)) batch.push_back(*i);
       if (batch.empty()) return;
-      std::vector<PointCloudSensor::ConstraintRequest> req;
-      Measurement::Ptr target_m = buildPatch(vertex);
-      for (unsigned index : batch) req.push_back({buildPatch(index), target_m, mCorrected[index].inverse() * mCorrected[vertex]});
-      res = mSensor->createConstraints(req, true);
+      if (mDevicePatches && mPatchBuildingRange > 0) {  // the patches are built and prepared on the device
+        std::vector<PointCloudSensor::LoopRequest> req;
+        const PointCloudSensor::Patch target_p = patchOf(vertex);
+        for (unsigned index : batch) req.push_back({patchOf(index), target_p, mCorrected[index].inverse() * mCorrected[vertex]});
+        res = mSensor->createLoopConstraints(req);
+      } else {
+        std::vector<PointCloudSensor::ConstraintRequest> req;
+        Measurement::Ptr target_m = buildPatch(vertex);
+        for (unsigned index : batch) req.push_back({buildPatch(index), target_m, mCorrected[index].inverse() * mCorrected[vertex]});
+        res = mSensor->createConstraints(req, true);
+      }
     }
     int count = 0;
     for (auto i = neighbors.rbegin(); i != neighbors.rend() && count < mMaxNeighorLinks; ++i) {
@@ -174,6 +189,9 @@ class MiniHost {
   void setNeighborRadius(float r, int max_links) { mNeighborRadius = r; mMaxNeighorLinks = max_links; }  // ScanSensor.hpp setters
   void setMinLoopLength(unsigned l) { mMinLoopLength = l; }
   void setPatchBuildingRange(unsigned r) { mPatchBuildingRange = r; }
+  // linkLastToNeighbors(true) with patches: build the patches on the device from their scans (PointCloudSensor::createLoopConstraints)
+  // instead of on the host (createCombinedMeasurement + createConstraints).  Same edges and warnings; off by default.
+  void setDevicePatches(bool on) { mDevicePatches = on; }
   const Transform& correctedPose(unsigned v) const { return mCorrected[v]; }
 
   std::vector<RecordedEdge> edges;
@@ -204,6 +222,7 @@ class MiniHost {
   int mMaxNeighorLinks = 1;
   unsigned mMinLoopLength = 10;
   unsigned mPatchBuildingRange = 0;                 // ScanSensor.hpp: Sensor::mPatchBuildingRange (core/Sensor.hpp)
+  bool mDevicePatches = false;                      // setDevicePatches
   float mMinTranslation = 0.f, mMinRotation = 0.f;  // Sensor::mMinTranslation / mMinRotation (0: every scan qualifies)
   Transform mLastTransform;                         // ScanSensor::mLastTransform
   PointCloudSensor* mSensor;

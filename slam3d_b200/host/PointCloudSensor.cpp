@@ -3,7 +3,9 @@
 #include "PointCloudSensor.hpp"
 
 #include <cmath>
+#include <cstring>
 #include <list>
+#include <map>
 #include <stdexcept>
 
 namespace slam3d_b200 {
@@ -288,16 +290,117 @@ std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createConstrai
   const int st = loop ? s3d_gicp_align_loop_batch(defaultContext(), src.data(), tgt.data(), guesses.data(), &cc, &cf, n, coarse.data(), fine.data())  // :286-292
                       : s3d_gicp_align_batch(defaultContext(), src.data(), tgt.data(), guesses.data(), &cf, n, fine.data());                           // :292
   if (st != S3D_OK) throw std::runtime_error(s3d_last_error());
-  for (int k = 0; k < n; ++k) {
-    ConstraintResult& r = out[idx[k]];
-    if (loop && coarse[k].status != S3D_OK) { failureOf(coarse[k].status, coarse[k], mCoarseConfiguration, r.error, r.message); continue; }  // the coarse align threw
-    if (fine[k].status != S3D_OK) { failureOf(fine[k].status, fine[k], mFineConfiguration, r.error, r.message); continue; }
-    Transform icp_result;
-    for (int j = 0; j < 16; ++j) icp_result.m[j] = fine[k].T[j];
-    const Transform tf = requests[idx[k]].source->getSensorPose() * icp_result * requests[idx[k]].target->getInverseSensorPose();  // :295
-    Covariance<6> covariance = Covariance<6>::Identity() * mCovarianceScale;                                                      // :296
-    r.constraint.reset(new SE3Constraint(mName, tf, covariance.inverseDiagonal()));
+  for (int k = 0; k < n; ++k)
+    out[idx[k]] = resultOf(coarse[k], fine[k], loop, requests[idx[k]].source->getSensorPose(), requests[idx[k]].target->getInverseSensorPose());
+  return out;
+}
+
+PointCloudSensor::ConstraintResult PointCloudSensor::resultOf(const s3d_result& coarse, const s3d_result& fine, bool loop,
+                                                              const Transform& source_sensor_pose, const Transform& target_inverse_sensor_pose) const {
+  ConstraintResult r;
+  if (loop && coarse.status != S3D_OK) { failureOf(coarse.status, coarse, mCoarseConfiguration, r.error, r.message); return r; }  // the coarse align threw
+  if (fine.status != S3D_OK) { failureOf(fine.status, fine, mFineConfiguration, r.error, r.message); return r; }
+  Transform icp_result;
+  for (int j = 0; j < 16; ++j) icp_result.m[j] = fine.T[j];
+  const Transform tf = source_sensor_pose * icp_result * target_inverse_sensor_pose;  // :295
+  Covariance<6> covariance = Covariance<6>::Identity() * mCovarianceScale;          // :296
+  r.constraint.reset(new SE3Constraint(mName, tf, covariance.inverseDiagonal()));
+  return r;
+}
+
+// the spec of the prepared handles an align() with `c` runs on (the cases in which align() takes the prepared path)
+static bool preparedSpec(const RegistrationParameters& c, s3d_prepare_spec& spec) {
+  if (std::isnan(c.point_cloud_density)) return false;
+  if ((c.registration_algorithm == GICP || c.registration_algorithm == GICP_OMP) && c.correspondence_randomness >= 1 && c.correspondence_randomness <= 4096) {
+    spec = s3d_prepare_spec{c.point_cloud_density, c.correspondence_randomness, 0.f};
+    return true;
   }
+  if ((c.registration_algorithm == NDT || c.registration_algorithm == NDT_OMP) && c.resolution > 0.f && std::isfinite(c.resolution)) {
+    spec = s3d_prepare_spec{c.point_cloud_density, 0, c.resolution};
+    return true;
+  }
+  return false;
+}
+
+std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createLoopConstraints(const std::vector<LoopRequest>& requests) {
+  std::vector<ConstraintResult> out(requests.size());
+  if (requests.empty()) return out;
+  s3d_prepare_spec coarse_spec, fine_spec;
+  if (!preparedSpec(mCoarseConfiguration, coarse_spec) || !preparedSpec(mFineConfiguration, fine_spec)) {
+    std::vector<ConstraintRequest> req;
+    for (const LoopRequest& r : requests)
+      req.push_back({createCombinedMeasurement(r.source.vertices, r.source.pose), createCombinedMeasurement(r.target.vertices, r.target.pose), r.odometry});
+    return createConstraints(req, true);
+  }
+  // distinct scans by cloud object, distinct patches by (member scans, member poses, patch pose) as bit patterns
+  std::vector<s3d_cloud> scans;
+  std::map<const PointCloud*, int32_t> scan_of;
+  std::vector<int32_t> member_scan, first{0};
+  std::vector<double> member_poses, patch_poses;
+  std::vector<uint64_t> patch_points;
+  std::map<std::vector<uint64_t>, int32_t> patch_of;
+  auto bits = [](std::vector<uint64_t>& key, const Transform& t) {
+    for (double d : t.m) { uint64_t b; std::memcpy(&b, &d, sizeof b); key.push_back(b); }
+  };
+  auto patchIndex = [&](const Patch& p) {
+    std::vector<uint64_t> key;
+    std::vector<int32_t> ms;
+    std::vector<Transform> mp;
+    uint64_t n = 0;
+    for (const auto& v : p.vertices) {
+      const PointCloud::Ptr& c = v.first->getPointCloud();
+      auto it = scan_of.find(c.get());
+      if (it == scan_of.end()) { it = scan_of.emplace(c.get(), (int32_t)scans.size()).first; scans.push_back(asCloud(c)); }
+      mp.push_back(v.second * v.first->getSensorPose());  // :248
+      ms.push_back(it->second);
+      key.push_back((uint64_t)it->second);
+      bits(key, mp.back());
+      n += c ? c->size() : 0;
+    }
+    bits(key, p.pose);
+    const auto ins = patch_of.emplace(key, (int32_t)patch_points.size());
+    if (ins.second) {
+      member_scan.insert(member_scan.end(), ms.begin(), ms.end());
+      for (const Transform& t : mp) member_poses.insert(member_poses.end(), t.m.begin(), t.m.end());
+      first.push_back((int32_t)member_scan.size());
+      patch_poses.insert(patch_poses.end(), p.pose.m.begin(), p.pose.m.end());
+      patch_points.push_back(n);
+      if (mLogger) mLogger->message(DEBUG, "Patch pointcloud has " + std::to_string(n) + " points.");  // :258-266
+    }
+    return ins.first->second;
+  };
+  std::vector<int32_t> src(requests.size()), tgt(requests.size());
+  for (size_t i = 0; i < requests.size(); ++i) { src[i] = patchIndex(requests[i].source); tgt[i] = patchIndex(requests[i].target); }
+  const int n_patches = (int)patch_points.size();
+  std::vector<s3d_prepare_spec> specs{coarse_spec};
+  if (fine_spec.density != coarse_spec.density || fine_spec.k != coarse_spec.k || fine_spec.resolution != coarse_spec.resolution) specs.push_back(fine_spec);
+  const int ns = (int)specs.size();
+  struct Handles {  // released when the batch is done, whatever happens
+    std::vector<s3d_prepared_cloud*> h;
+    ~Handles() { for (s3d_prepared_cloud* p : h) s3d_release_cloud(defaultContext(), p); }
+  } hh;
+  hh.h.assign((size_t)n_patches * ns, nullptr);
+  if (s3d_prepare_combined_measurements(defaultContext(), 0, scans.data(), (int)scans.size(), member_scan.data(), member_poses.data(), first.data(),
+                                        patch_poses.data(), n_patches, specs.data(), ns, hh.h.data()) != S3D_OK)
+    throw std::runtime_error(s3d_last_error());
+  // a patch's sensor pose is the identity (createCombinedMeasurement :265); the guess and the edge are formed as createConstraint
+  // forms them (:274, :295)
+  const Transform identity = Transform::Identity();
+  const int n = (int)requests.size();
+  std::vector<const s3d_prepared_cloud*> cs(n), ct(n), fs(n), ft(n);
+  std::vector<double> guesses;
+  for (int i = 0; i < n; ++i) {
+    cs[i] = hh.h[(size_t)src[i] * ns]; ct[i] = hh.h[(size_t)tgt[i] * ns];
+    fs[i] = hh.h[(size_t)src[i] * ns + ns - 1]; ft[i] = hh.h[(size_t)tgt[i] * ns + ns - 1];
+    const Transform guess = identity.inverse() * requests[i].odometry * identity;
+    guesses.insert(guesses.end(), guess.m.begin(), guess.m.end());
+  }
+  std::vector<s3d_result> coarse(n), fine(n);
+  const s3d_registration_parameters cc = mCoarseConfiguration.toC(), cf = mFineConfiguration.toC();
+  if (s3d_gicp_align_loop_batch_prepared(defaultContext(), cs.data(), ct.data(), fs.data(), ft.data(), guesses.data(), &cc, &cf, n, coarse.data(),
+                                         fine.data()) != S3D_OK)
+    throw std::runtime_error(s3d_last_error());
+  for (int i = 0; i < n; ++i) out[i] = resultOf(coarse[i], fine[i], true, identity, identity.inverse());
   return out;
 }
 

@@ -76,6 +76,17 @@ class PointCloudSensor {
   };
   std::vector<ConstraintResult> createConstraints(const std::vector<ConstraintRequest>& requests, bool loop);
 
+  // Loop closures between patches (extension): request i gives the same constraint — or fails with the same exception type and
+  // message — as createConstraint(createCombinedMeasurement(source_i), createCombinedMeasurement(target_i), odometry_i, true),
+  // but the patches never exist on the host: one s3d_prepare_combined_measurements call builds every distinct patch on the device
+  // from the distinct scans (each uploaded once) and prepares it for the coarse and the fine configuration, and one
+  // s3d_gicp_align_loop_batch_prepared runs all coarse and fine aligns.  Scans are told apart by cloud object, patches by
+  // (members, their poses, patch pose); each distinct patch logs createCombinedMeasurement's DEBUG line.  A configuration that no
+  // prepared handle serves (ICP, k or resolution out of range) takes the host patches and createConstraints instead.
+  struct Patch { PosedMeasurements vertices; Transform pose; };  // the arguments of createCombinedMeasurement
+  struct LoopRequest { Patch source, target; Transform odometry; };
+  std::vector<ConstraintResult> createLoopConstraints(const std::vector<LoopRequest>& requests);
+
  protected:
   std::string mName;
   Logger* mLogger;
@@ -86,6 +97,11 @@ class PointCloudSensor {
   double mMapResolution;
   double mMapOutlierRadius;
   unsigned mMapOutlierNeighbors;
+
+ private:
+  // the ConstraintResult of one batched createConstraint from its align results (:286-299)
+  ConstraintResult resultOf(const s3d_result& coarse, const s3d_result& fine, bool loop, const Transform& source_sensor_pose,
+                            const Transform& target_inverse_sensor_pose) const;
 };
 
 }  // namespace slam3d_b200

@@ -1,5 +1,6 @@
 // host_capi.cpp — flat C entry points over the C++ host mirror so the pytest suite can drive it through ctypes.
 // (Test/driver glue only; a slam3d application uses the C++ classes directly.)
+#include <chrono>
 #include <cstring>
 #include <thread>
 
@@ -32,6 +33,8 @@ struct OtherMeasurement : Measurement {
 extern "C" {
 
 const char* s3dhost_last_message() { return g_msg.c_str(); }
+// the process-wide context of the host mirror (counters, stage times of everything the mirror ran)
+void* s3dhost_context() { return defaultContext(); }
 void s3dhost_set_cache_capacity(uint64_t n) { setPreparedCacheCapacity((size_t)n); }
 uint64_t s3dhost_cache_hits() { return (uint64_t)preparedCacheHits(); }
 
@@ -121,6 +124,11 @@ int s3dhost_run_odometry(void* s, const float* const* scans, const uint64_t* siz
   return (int)all[0].size();
 }
 
+// seconds spent in linkLastToNeighbors() calls that matched at least one candidate, and their number, of the last trajectory run
+static double g_link_seconds = 0;
+static int g_link_calls = 0;
+void s3dhost_link_stats(double* seconds, int* calls) { *seconds = g_link_seconds; *calls = g_link_calls; }
+
 // BASELINE configs[4] (trajectory): n scans through addMeasurement(m, odom) + linkLastToNeighbors() after every new vertex.
 // edges_out: per recorded edge {source, target, loop} as 3 ints followed by nothing; T_out: 16 doubles per edge (relative pose);
 // poses_out: n x 16 doubles (corrected poses).  Returns the number of edges (<= max_edges) or -1.
@@ -133,9 +141,18 @@ static int run_trajectory(void* s, const float* const* scans, const uint64_t* si
     host.setNeighborRadius((float)neighbor_radius, max_links);
     host.setMinLoopLength((unsigned)min_loop_length);
     host.setPatchBuildingRange((unsigned)patch_range);
+    host.setDevicePatches(batched == 2);
+    g_link_seconds = 0; g_link_calls = 0;
     for (int i = 0; i < n; ++i) {
       Measurement::Ptr m(new PointCloudMeasurement(makeCloud(scans[i], sizes[i]), "robot", sensor->getName(), Transform()));
-      if (host.addMeasurement(m, makeTransform(odoms + 16 * i))) host.linkLastToNeighbors(batched != 0);
+      if (!host.addMeasurement(m, makeTransform(odoms + 16 * i))) continue;
+      const size_t seen = host.edges.size() + host.warnings.size();
+      const auto t0 = std::chrono::steady_clock::now();
+      host.linkLastToNeighbors(batched != 0);
+      if (host.edges.size() + host.warnings.size() != seen) {
+        g_link_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
+        ++g_link_calls;
+      }
     }
     const int ne = (int)std::min<size_t>(host.edges.size(), (size_t)max_edges);
     for (int e = 0; e < ne; ++e) {
@@ -158,7 +175,8 @@ int s3dhost_run_trajectory(void* s, const float* const* scans, const uint64_t* s
 }
 
 // the same with Sensor::mPatchBuildingRange = patch_range (loop closures match patches of scans, ScanSensor.cpp:215-270) and,
-// when batched != 0, all candidates of a vertex matched in one device batch (PointCloudSensor::createConstraints)
+// when batched != 0, all candidates of a vertex matched in one device batch (PointCloudSensor::createConstraints); batched == 2
+// builds those patches on the device (MiniHost::setDevicePatches, PointCloudSensor::createLoopConstraints)
 int s3dhost_run_trajectory2(void* s, const float* const* scans, const uint64_t* sizes, int n, const double* odoms, double neighbor_radius,
                             int max_links, int min_loop_length, int patch_range, int batched, int max_edges, int* edges_out, double* T_out,
                             double* poses_out, int* n_warnings) {
