@@ -11,7 +11,8 @@
  *   - plain C, no C++/torch types; all pointers are caller-owned and only read/written during the call;
  *   - point clouds are arrays of 16-byte points {x,y,z,w} == pcl::PointXYZ memory
  *     (PointCloudSensor.hpp:43-44); `w` is ignored on input and written as 1.0f on output;
- *   - cloud pointers may be HOST or DEVICE pointers (the library asks cudaPointerGetAttributes);
+ *   - cloud pointers may be HOST or DEVICE pointers (the library asks cudaPointerGetAttributes); device memory of the GPU a call
+ *     runs on is read in place, device memory of another GPU is first copied device to device onto the call's GPU;
  *     result structs and 4x4 poses are always host memory.  Host clouds may be pageable (a std::vector, a pcl::PointCloud);
  *     pinned memory (cudaHostRegister on the cloud's buffer, or cudaMallocHost) roughly doubles the upload rate;
  *   - DEVICE inputs are read in place on the library's own (non-blocking) streams: they must be complete before the call.
@@ -229,9 +230,25 @@ int s3d_prepare_cloud_ndt(s3d_context* ctx, int device_slot, s3d_cloud cloud, do
                           s3d_prepared_cloud** out);
 int s3d_release_cloud(s3d_context* ctx, s3d_prepared_cloud* cloud);
 uint64_t s3d_prepared_cloud_size(const s3d_prepared_cloud* cloud); /* points after filtering */
-/* Device blocks of prepared clouds since context creation, over all devices: obtained from cudaMalloc, and reused from
- * released handles (s3d_release_cloud hands a block back to its device; a later prepare takes it when it fits). */
+/* Device blocks since context creation, over all devices: obtained from cudaMalloc, and reused from released handles.  One pool
+ * per device serves prepared clouds and resident scans (s3d_upload_scans): s3d_release_cloud and s3d_release_scan hand a block back
+ * to its device, and a later prepare or upload takes it when it fits. */
 int s3d_get_prepared_block_stats(s3d_context* ctx, uint64_t* allocated, uint64_t* reused);
+
+/* ---- resident scans ---------------------------------------------------------------------------------------------------------
+ * A slam3d measurement is matched, patched and mapped many times over its life, and every call with a host cloud uploads it again.
+ * s3d_upload_scans copies clouds once into library-owned device memory of `device_slot` (blocks of the pool above); the caller keeps
+ * the handles as long as the measurements live.  s3d_resident_scan_cloud returns a handle's device view: an s3d_cloud that every
+ * entry point taking a cloud accepts (it is a device cloud like any other; results are bit for bit those of the host cloud).
+ * The copy is verbatim (16 bytes per point, `w` included).  Host clouds go through the same staging as every call's host inputs and
+ * add 16 n bytes each to h2d_bytes; device clouds (of any device) are copied device to device and add nothing.  Synchronous like
+ * every call: the views are complete on return.  All-or-nothing like s3d_prepare_clouds.  A bad device slot, a NULL pointer, n < 0
+ * or a cloud of 2^31 points or more: S3D_INVALID_ARGUMENT and no handle.  An empty cloud gets a handle of size 0 (view: NULL, 0).
+ * Handles are immutable and may be shared by threads; release every handle before s3d_destroy_context. */
+typedef struct s3d_resident_scan s3d_resident_scan;
+int s3d_upload_scans(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, s3d_resident_scan** out);
+int s3d_release_scan(s3d_context* ctx, s3d_resident_scan* scan);
+s3d_cloud s3d_resident_scan_cloud(const s3d_resident_scan* scan); /* {NULL, 0} for NULL */
 /* Align on prepared clouds; the algorithm comes from params->registration_algorithm as in s3d_gicp_align.
  *   GICP / GICP_OMP  both handles from s3d_prepare_cloud(s) with k == correspondence_randomness (an NDT handle: status 6).
  *   NDT / NDT_OMP    the source (the scan whose grid NDT matches against) from s3d_prepare_cloud(s)_ndt with

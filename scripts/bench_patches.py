@@ -1,18 +1,21 @@
 #!/usr/bin/env python
 """Config 5 with patches (SURVEY 8d: mPatchBuildingRange = 2, 3 links per vertex, candidates batched): the same figure-eight
-trajectory as scripts/run_c5.py, through the MiniHost twice per repetition, alternating in one process:
+trajectory as scripts/run_c5.py, through the MiniHost three times per repetition, alternating in one process:
 
   host    linkLastToNeighbors(true) builds every patch with createCombinedMeasurement (to the host) and matches the host patches
           with createConstraints (s3d_gicp_align_loop_batch: uploads and preprocesses every pair slot, coarse and fine pass)
   device  setDevicePatches(true): createLoopConstraints builds the distinct patches on the device from the distinct scans,
           prepares each once per pass setting and runs s3d_gicp_align_loop_batch_prepared
+  resident  device patches with the host mirror's resident-scan store on (setResidentScanBudget): every scan is uploaded once,
+          on its first use, and every later call (odometry prepares, patch builds) reads its device copy
 
-Both runs must record the same edges bit for bit and the same warnings.  Reported per mode: scans/s over the whole trajectory
+All runs must record the same edges bit for bit and the same warnings.  Reported per mode: scans/s over the whole trajectory
 (odometry included), H2D / D2H bytes and kernel launches of the library, and the mean time of one vertex's loop-closure call
 (linkLastToNeighbors of a vertex that matched at least one candidate).  A last profiled run of each mode gives the device-time
-split by stage (s3d_get_stage_times).
+split by stage (s3d_get_stage_times).  Last, one buildMap over the whole trajectory (s3d_build_map, the sensor's default map
+settings) is timed from host scans and from resident scans (s3d_upload_scans), alternating.
 
-    python scripts/bench_patches.py --scans 600 --reps 2 --out profiles/r03_bench_patches.json
+    python scripts/bench_patches.py --scans 600 --reps 2 --out profiles/r04_bench_resident.json
 """
 import argparse
 import ctypes as C
@@ -28,7 +31,8 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 
-MODES = {"host": 1, "device": 2}  # s3dhost_run_trajectory2's `batched`
+MODES = {"host": 1, "device": 2, "resident": 2}  # s3dhost_run_trajectory2's `batched`
+RESIDENT_BUDGET = 1 << 36  # holds every scan of the trajectory: nothing is evicted
 
 
 def workload(n):
@@ -58,6 +62,34 @@ def workload(n):
     return scans, odoms
 
 
+def time_build_map(scans, poses, reps):
+    """one s3d_build_map over every scan of the trajectory (outlier radius 0.2, 3 neighbours, 0.1 m: the sensor's defaults), from
+    host scans and from resident scans, alternating; both maps must be equal bit for bit"""
+    import slam3d_b200
+    ctx = slam3d_b200.Context()
+    t0 = time.perf_counter()
+    views = ctx.upload_scans(scans)
+    upload_s = time.perf_counter() - t0
+    times = {"host": [], "resident": []}
+    maps = {}
+    for rep in range(reps + 1):  # repetition 0 warms up
+        for mode in (("host", "resident") if rep % 2 == 0 else ("resident", "host")):
+            h0 = ctx.counters()["h2d_bytes"]
+            t0 = time.perf_counter()
+            m = ctx.build_map(views if mode == "resident" else scans, poses)
+            dt = time.perf_counter() - t0
+            maps[mode] = (m.shape[0], m.tobytes())
+            print(json.dumps({"build_map": mode, "rep": rep, "seconds": dt, "h2d_bytes": ctx.counters()["h2d_bytes"] - h0}), flush=True)
+            if rep > 0:
+                times[mode].append(dt)
+    assert maps["host"] == maps["resident"], "maps differ"
+    for v in views:
+        v.release()
+    ctx.close()
+    return {"scans": len(scans), "map_points": maps["host"][0], "upload_once_s": upload_s,
+            **{f"{m}_s": float(np.median(t)) for m, t in times.items()}, "runs": times}
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--scans", type=int, default=600)
@@ -76,6 +108,8 @@ def main():
                                              C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_int)]
     host.s3dhost_context.restype = C.c_void_p
     host.s3dhost_link_stats.argtypes = [C.POINTER(C.c_double), C.POINTER(C.c_int)]
+    host.s3dhost_set_resident_budget.argtypes = [C.c_uint64]
+    host.s3dhost_resident_stats.argtypes = [C.POINTER(C.c_uint64)] * 3
     hctx = C.c_void_p(host.s3dhost_context())
     n = args.scans
     scans, odoms = workload(n)
@@ -93,20 +127,27 @@ def main():
         L.s3d_get_counters(hctx, C.byref(c))
         return np.array([c.kernel_launches, c.h2d_bytes, c.d2h_bytes], np.int64)
 
+    def uploads():
+        u, h, b = C.c_uint64(0), C.c_uint64(0), C.c_uint64(0)
+        host.s3dhost_resident_stats(C.byref(u), C.byref(h), C.byref(b))
+        return u.value
+
     def run(mode):
         edges = np.zeros((4 * n, 3), np.int32); T = np.zeros((4 * n, 16)); nw = C.c_int(0)
-        c0 = counters()
+        host.s3dhost_set_resident_budget(RESIDENT_BUDGET if mode == "resident" else 0)
+        c0, u0 = counters(), uploads()
         t0 = time.perf_counter()
         ne = host.s3dhost_run_trajectory2(sensor, ptrs, sizes, n, od.ctypes.data, args.radius, args.max_links, 10, args.patch_range,
                                           MODES[mode], 4 * n, edges.ctypes.data, T.ctypes.data, None, C.byref(nw))
         dt = time.perf_counter() - t0
-        c1 = counters()
+        c1, u1 = counters(), uploads()
+        host.s3dhost_set_resident_budget(0)
         assert ne >= 0, host.s3dhost_last_message()
         ls, lc = C.c_double(0), C.c_int(0)
         host.s3dhost_link_stats(C.byref(ls), C.byref(lc))
         d = c1 - c0
         return {"seconds": dt, "scans_per_s": n / dt, "kernel_launches": int(d[0]), "h2d_bytes": int(d[1]), "d2h_bytes": int(d[2]),
-                "loop_calls": lc.value, "loop_call_ms": 1e3 * ls.value / max(lc.value, 1)}, \
+                "loop_calls": lc.value, "loop_call_ms": 1e3 * ls.value / max(lc.value, 1), "scans_uploaded_to_store": u1 - u0}, \
                (edges[:ne].copy(), T[:ne].copy(), nw.value, host.s3dhost_last_message().decode())
 
     gpu = {}
@@ -117,12 +158,12 @@ def main():
         pass
     runs = {m: [] for m in MODES}
     ref = {}
-    for rep in range(args.reps + 1):  # repetition 0 warms up both modes (module load, workspace growth, loop graphs)
-        for mode in (("host", "device") if rep % 2 == 0 else ("device", "host")):
+    order = list(MODES)
+    for rep in range(args.reps + 1):  # repetition 0 warms up every mode (module load, workspace growth, loop graphs)
+        for mode in order[rep % 3:] + order[:rep % 3]:
             r, out = run(mode)
             ref.setdefault(mode, out)
-            other = ref.get("device" if mode == "host" else "host")
-            if other is not None:
+            for other in ref.values():
                 assert np.array_equal(out[0], other[0]) and np.array_equal(out[1], other[1]) and out[2:] == other[2:], "edges differ"
             if rep > 0:
                 runs[mode].append(r)
@@ -138,12 +179,14 @@ def main():
         L.s3d_get_stage_times(hctx, ms, nl, 1)
         L.s3d_set_profiling(hctx, 0)
         stages[mode] = {"wall_s": r["seconds"], **{k: {"ms": ms[i], "launches": int(nl[i])} for i, k in enumerate(names)}}
+    build_map = time_build_map(scans, odoms, args.reps)
     e = ref["host"][0]
     summary = {
         "workload": f"config 5: {n}-scan figure-eight, patch range {args.patch_range}, {args.max_links} links per vertex, batched",
         "gpu": gpu, "edges": int(len(e)), "loop_edges": int(e[:, 2].sum()), "warnings": ref["host"][2], "edges_equal": True,
+        "scan_bytes": int(sum(16 * s.shape[0] for s in scans)),
         **{m: {k: float(np.median([r[k] for r in runs[m]])) for k in runs[m][0]} for m in MODES},
-        "runs": runs, "stages_profiled": stages,
+        "runs": runs, "stages_profiled": stages, "build_map": build_map,
     }
     print(json.dumps(summary))
     if args.out:

@@ -71,6 +71,10 @@ def lib():
                                                     C.POINTER(RegistrationParameters), C.c_int, C.POINTER(Result)]
         L.s3d_prepare_combined_measurements.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                                         C.c_void_p, C.c_int, C.POINTER(PrepareSpec), C.c_int, C.POINTER(C.c_void_p)]
+        L.s3d_upload_scans.argtypes = [C.c_void_p, C.c_int, C.POINTER(Cloud), C.c_int, C.POINTER(C.c_void_p)]
+        L.s3d_release_scan.argtypes = [C.c_void_p, C.c_void_p]
+        L.s3d_resident_scan_cloud.argtypes = [C.c_void_p]
+        L.s3d_resident_scan_cloud.restype = Cloud
         L.s3d_gicp_align_loop_batch_prepared.argtypes = [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.POINTER(C.c_void_p),
                                                          C.POINTER(C.c_void_p), C.c_void_p, C.POINTER(RegistrationParameters),
                                                          C.POINTER(RegistrationParameters), C.c_int, C.POINTER(Result), C.POINTER(Result)]
@@ -99,6 +103,10 @@ def _is_torch(a):
 
 
 def _cloud(ctx, a):
+    if isinstance(a, ResidentScan):  # a device cloud: the library reads it in place (or copies it to the GPU a call runs on)
+        if not a._h:
+            raise ValueError("ResidentScan was released")
+        return a, lib().s3d_resident_scan_cloud(a._h)
     a = as_xyzw(a)
     if _is_torch(a):
         if a.is_cuda:
@@ -289,6 +297,44 @@ class PreparedCloud:
                 self.release()
         except Exception:
             pass
+
+
+class ResidentScan:
+    """A scan copied once into library-owned device memory of one device slot (s3d_upload_scans).  Every Context method that takes a
+    cloud takes a ResidentScan in its place, with the same result as the host cloud and without uploading it again.  release()
+    hands the memory back to the context's block pool."""
+
+    def __init__(self, ctx, handle, size):
+        self._ctx, self._h, self.size = ctx, handle, size
+
+    @property
+    def shape(self):
+        return (self.size, 4)
+
+    def release(self):
+        if self._h:
+            lib().s3d_release_scan(self._ctx._h, self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            if self._ctx._h:
+                self.release()
+        except Exception:
+            pass
+
+
+def _upload_scans(self, clouds, device_slot=0):
+    """Copies each cloud (numpy array, torch tensor on the host or a GPU) verbatim to device memory of `device_slot`; returns one
+    ResidentScan per cloud (all-or-nothing)."""
+    n = len(clouds)
+    keep = []
+    cc = (Cloud * max(n, 1))()
+    for i in range(n):
+        a, c = _cloud(self, clouds[i]); keep.append(a); cc[i] = c
+    hh = (C.c_void_p * max(n, 1))()
+    self._check(lib().s3d_upload_scans(self._h, int(device_slot), cc, n, hh), "s3d_upload_scans")
+    return [ResidentScan(self, C.c_void_p(hh[i]), int(cc[i].n)) for i in range(n)]
 
 
 def _prepare_cloud(self, cloud, density, k=20, device_slot=0):
@@ -485,6 +531,7 @@ def _fill_ground_plane(self, cloud, radius, map_resolution=0.1):
     return out[:n].copy()
 
 
+Context.upload_scans = _upload_scans
 Context.fit_plane_ransac = _fit_plane_ransac
 Context.fill_ground_plane = _fill_ground_plane
 Context.combined_measurement = _combined_measurement

@@ -95,6 +95,13 @@ struct s3d_prepared_cloud {
   s3d::NdtGrid grid{};       // NDT handles: the VoxelGridCovariance; leaves / table point into `block`
 };
 
+struct s3d_resident_scan {
+  int device_slot = 0;
+  void* block = nullptr;     // the n points, a block of the device's pool (NULL for an empty scan)
+  size_t block_bytes = 0;
+  uint64_t n = 0;
+};
+
 struct s3d_context {
   std::vector<std::unique_ptr<s3d::DeviceCtx>> devs;
   std::mutex mu;
@@ -771,6 +778,67 @@ int s3d_get_prepared_block_stats(s3d_context* ctx, uint64_t* allocated, uint64_t
   return S3D_OK;
 }
 
+// ---- resident scans ---------------------------------------------------------------------------------------------------
+int s3d_upload_scans(s3d_context* ctx, int device_slot, const s3d_cloud* clouds, int n, s3d_resident_scan** out) {
+  auto invalid = [](const char* msg) { set_error(msg); return (int)S3D_INVALID_ARGUMENT; };
+  if (!ctx || !out || n < 0) return invalid("s3d_upload_scans: NULL context or output, or n < 0");
+  for (int i = 0; i < n; ++i) out[i] = nullptr;
+  if (n > 0 && !clouds) return invalid("s3d_upload_scans: NULL cloud list");
+  if (device_slot < 0 || device_slot >= (int)ctx->devs.size()) return invalid("bad device slot");
+  for (int i = 0; i < n; ++i) {
+    if (clouds[i].n >= (1ull << 31)) return invalid("s3d_upload_scans: a cloud of 2^31 points or more");
+    if (clouds[i].n && !clouds[i].xyzw) return invalid("s3d_upload_scans: cloud without points pointer");
+  }
+  if (n == 0) return S3D_OK;
+  return guarded([&]() -> int {
+    WsLease lease(ctx, device_slot);
+    Workspace& ws = *lease;
+    DeviceCtx* dc = ctx->devs[device_slot].get();
+    std::vector<std::unique_ptr<s3d_resident_scan>> hh(n);
+    struct BlockGuard {  // a failure below hands the blocks back instead of leaking them
+      std::vector<std::unique_ptr<s3d_resident_scan>>& hh; DeviceCtx* dc; bool armed = true;
+      ~BlockGuard() {
+        if (!armed) return;
+        std::lock_guard<std::mutex> g(dc->mu);
+        for (auto& h : hh) if (h && h->block) dc->free_blocks.emplace_back(h->block, h->block_bytes);
+      }
+    } guard{hh, dc};
+    std::vector<const float*> src;
+    std::vector<uint64_t> sizes;
+    std::vector<float4*> dst;
+    for (int i = 0; i < n; ++i) {
+      hh[i].reset(new s3d_resident_scan());
+      hh[i]->device_slot = device_slot;
+      hh[i]->n = clouds[i].n;
+      if (!clouds[i].n) continue;
+      hh[i]->block = block_alloc(dc, 16 * size_t(clouds[i].n), &hh[i]->block_bytes);
+      src.push_back(clouds[i].xyzw); sizes.push_back(clouds[i].n); dst.push_back(static_cast<float4*>(hh[i]->block));
+    }
+    upload_clouds(ws, src, sizes, dst);
+    guard.armed = false;
+    for (int i = 0; i < n; ++i) out[i] = hh[i].release();
+    return S3D_OK;
+  });
+}
+
+int s3d_release_scan(s3d_context* ctx, s3d_resident_scan* scan) {
+  if (!scan) return S3D_OK;
+  if (!ctx || scan->device_slot >= (int)ctx->devs.size()) return S3D_INVALID_ARGUMENT;
+  if (scan->block) {
+    DeviceCtx* dc = ctx->devs[scan->device_slot].get();
+    std::lock_guard<std::mutex> g(dc->mu);
+    dc->free_blocks.emplace_back(scan->block, scan->block_bytes);  // recycled by the next prepare or upload; freed with the context
+  }
+  delete scan;
+  return S3D_OK;
+}
+
+s3d_cloud s3d_resident_scan_cloud(const s3d_resident_scan* scan) {
+  s3d_cloud c{nullptr, 0};
+  if (scan) { c.xyzw = static_cast<const float*>(scan->block); c.n = scan->n; }
+  return c;
+}
+
 namespace s3d {
 // One sub-batch of align() calls on prepared clouds (all on device slot `slot`).  GICP runs every pair; NDT runs the pairs whose
 // fixed cloud (the source, slot 2p) is an NDT handle, and the others end as align() ends for an algorithm without its data.
@@ -1116,7 +1184,8 @@ int s3d_build_map(s3d_context* ctx, const s3d_cloud* clouds, const double* poses
 namespace {
 constexpr uint64_t kMaxGroundFill = (1ull << 31) - 1;
 
-// the cloud in ws.accu (device): the sampler and the counting kernel read it many times, whatever memory it came from
+// the cloud in ws.accu (device): the sampler and the counting kernel read it many times, whatever memory it came from (the copy of
+// another GPU's memory, such as a scan resident on another device slot, is a device-to-device copy onto ws.device)
 const float4* stage_cloud(Workspace& ws, s3d_cloud cloud) {
   S3D_CUDA(cudaSetDevice(ws.device));
   ws.order_after_input();

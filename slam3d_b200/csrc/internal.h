@@ -261,6 +261,8 @@ struct StageTimer {
 
 // ---- stage launchers (each enqueues kernels on ws.stream; no host synchronisation inside) -----------------
 void setup_batch(Workspace& ws, const std::vector<const float*>& clouds, const std::vector<uint64_t>& sizes, uint32_t n_pairs);
+// voxel.cu: clouds[i] (host or device memory of any GPU, sizes[i] points) copied verbatim to dst[i] on ws.device; synchronises ws
+void upload_clouds(Workspace& ws, const std::vector<const float*>& clouds, const std::vector<uint64_t>& sizes, const std::vector<float4*>& dst);
 void run_voxel(Workspace& ws, float leaf, uint32_t* leaf_keys = nullptr);  // leaf <= 0: working cloud = raw cloud; leaf_keys: unsorted voxel keys (device, total)
 void run_grid(Workspace& ws, float leaf_hint);      // NN grid on the working clouds
 void run_knn_covariances(Workspace& ws, int k, uint32_t* knn_index, float* knn_dist2);  // outputs optional (device, slot-concatenated)

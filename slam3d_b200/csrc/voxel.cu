@@ -158,6 +158,64 @@ class CopyPool {
   bool stop_ = false;
 };
 
+static cudaPointerAttributes pointer_attributes(const void* p) {
+  cudaPointerAttributes at{};
+  if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
+  return at;
+}
+
+// Pageable host clouds (a std::vector, the points of a pcl::PointCloud): cudaMemcpyAsync from pageable memory is staged by the
+// driver through one small pinned buffer and blocks the calling thread (~10 GB/s, measured: e2e 1800 against 2430
+// registrations/s from pinned memory).  The chunk's host thread copies them into the workspace's own pinned buffer instead —
+// the host threads of the other chunks do the same in parallel, before they queue for the upload turn — and the DMA runs from there.
+static bool pinned_bounce_enabled() {
+  static const bool enabled = [] { const char* e = getenv("S3D_PINNED_BOUNCE"); return !e || atoi(e) != 0; }();  // 0: A/B measurements
+  return enabled;
+}
+
+// s3d_upload_scans: verbatim copies of clouds[i] into dst[i] (device memory of ws.device), staged as setup_batch stages its inputs.
+// Pageable clouds are copied in rounds of at most kRound bytes through the pinned bounce buffer, so it stays bounded however many
+// scans one call uploads.  Host bytes count in ws.h2d; device clouds (of this or another GPU) are copied device to device.
+void upload_clouds(Workspace& ws, const std::vector<const float*>& clouds, const std::vector<uint64_t>& sizes, const std::vector<float4*>& dst) {
+  constexpr size_t kRound = size_t(256) << 20;
+  S3D_CUDA(cudaSetDevice(ws.device));
+  ws.order_after_input();
+  const size_t n = clouds.size();
+  std::vector<int> host(n, 0), via_bounce(n, 0);
+  for (size_t i = 0; i < n; ++i) {
+    if (!sizes[i]) continue;
+    const cudaPointerAttributes at = pointer_attributes(clouds[i]);
+    host[i] = at.type != cudaMemoryTypeDevice && at.type != cudaMemoryTypeManaged;
+    via_bounce[i] = at.type == cudaMemoryTypeUnregistered && pinned_bounce_enabled();
+  }
+  std::vector<size_t> at_bounce(n, 0);  // offset of a pageable cloud in the bounce buffer during its round
+  for (size_t b = 0; b < n;) {
+    size_t e = b, pinned = 0;  // this round: clouds [b, e), `pinned` bytes of them through the bounce buffer
+    std::vector<std::pair<void*, std::pair<const void*, size_t>>> spans;
+    for (; e < n; ++e) {
+      const size_t bytes = 16 * size_t(sizes[e]);
+      if (!via_bounce[e]) continue;
+      if (pinned && pinned + bytes > kRound) break;
+      at_bounce[e] = pinned;
+      pinned += bytes;
+    }
+    if (pinned) {
+      ws.h_bounce.reserve(pinned);
+      for (size_t i = b; i < e; ++i)
+        if (via_bounce[i]) spans.push_back({ws.h_bounce.as<char>() + at_bounce[i], {clouds[i], 16 * size_t(sizes[i])}});
+      CopyPool::get().copy(spans);
+    }
+    for (size_t i = b; i < e; ++i) {
+      if (!sizes[i]) continue;
+      const void* from = via_bounce[i] ? static_cast<const void*>(ws.h_bounce.as<char>() + at_bounce[i]) : static_cast<const void*>(clouds[i]);
+      S3D_CUDA(cudaMemcpyAsync(dst[i], from, 16 * size_t(sizes[i]), cudaMemcpyDefault, ws.stream));
+      if (host[i]) ws.h2d += 16 * size_t(sizes[i]);
+    }
+    ws.sync();  // the bounce buffer is refilled by the next round
+    b = e;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------------------
 // Batch set-up: slot table, tile table, input staging.  clouds[2p] = slam3d source of pair p, clouds[2p+1] = target
 // (or any list of clouds for the stage-level entry points).
@@ -208,26 +266,21 @@ void setup_batch(Workspace& ws, const std::vector<const float*>& clouds, const s
   ws.h_slots.reserve(sizeof(SlotInfo) * ns);
   ws.h_tiles.reserve(4 * (2 * size_t(n_tiles) + ns + 1));
 
-  // classify input pointers; host memory (pinned or pageable) and misaligned device memory go through raw_stage
+  // classify input pointers; host memory (pinned or pageable), misaligned device memory and device memory of another GPU (a view
+  // of a scan resident on one device inside a batch sharded over several) go through raw_stage
   bool need_stage = false, need_bounce = false;
-  std::vector<int> on_device(ns, 0), pageable(ns, 0);
+  std::vector<int> on_device(ns, 0), pageable(ns, 0), other_device(ns, 0);
   for (uint32_t s = 0; s < ns; ++s) {
     if (sizes[s] == 0) continue;
-    cudaPointerAttributes at{};
-    cudaError_t e = cudaPointerGetAttributes(&at, clouds[s]);
-    if (e != cudaSuccess) { cudaGetLastError(); at.type = cudaMemoryTypeUnregistered; }
-    on_device[s] = (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && (reinterpret_cast<uintptr_t>(clouds[s]) & 15) == 0;
+    const cudaPointerAttributes at = pointer_attributes(clouds[s]);
+    other_device[s] = at.type == cudaMemoryTypeDevice && at.device != ws.device;
+    on_device[s] = (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) && !other_device[s] && (reinterpret_cast<uintptr_t>(clouds[s]) & 15) == 0;
     pageable[s] = at.type == cudaMemoryTypeUnregistered;
     if (!on_device[s]) need_stage = true;
     if (pageable[s]) need_bounce = true;
   }
   if (need_stage) ws.raw_stage.reserve(16 * tot);
-  // Pageable host clouds (a std::vector, the points of a pcl::PointCloud): cudaMemcpyAsync from pageable memory is staged by the
-  // driver through one small pinned buffer and blocks the calling thread (~10 GB/s, measured: e2e 1800 against 2430
-  // registrations/s from pinned memory).  The chunk's host thread copies them into the workspace's own pinned buffer instead —
-  // the host threads of the other chunks do the same in parallel, before they queue for the upload turn — and the DMA runs from there.
-  static const bool bounce_enabled = [] { const char* e = getenv("S3D_PINNED_BOUNCE"); return !e || atoi(e) != 0; }();  // 0: A/B measurements
-  if (need_bounce && bounce_enabled) {
+  if (need_bounce && pinned_bounce_enabled()) {
     ws.h_bounce.reserve(16 * tot);
     std::vector<std::pair<void*, std::pair<const void*, size_t>>> spans;
     for (uint32_t s = 0; s < ns; ++s)
@@ -258,8 +311,8 @@ void setup_batch(Workspace& ws, const std::vector<const float*>& clouds, const s
     else {
       si.raw = ws.raw_stage.as<float4>() + si.off;
       const void* from = (need_bounce && pageable[s]) ? static_cast<const void*>(ws.h_bounce.as<char>() + 16 * size_t(si.off)) : static_cast<const void*>(clouds[s]);
-      S3D_CUDA(cudaMemcpyAsync(ws.raw_stage.as<float4>() + si.off, from, 16 * sizes[s], cudaMemcpyDefault, ws.stream));
-      ws.h2d += 16 * sizes[s];
+      S3D_CUDA(cudaMemcpyAsync(ws.raw_stage.as<float4>() + si.off, from, 16 * sizes[s], cudaMemcpyDefault, ws.stream));  // another GPU's memory: device to device
+      if (!other_device[s]) ws.h2d += 16 * sizes[s];
     }
     h_begin[s] = t;
     for (uint64_t f = 0; f < sizes[s]; f += kSortTile) { h_tile_slot[t] = s; h_tile_first[t] = static_cast<uint32_t>(f); ++t; }

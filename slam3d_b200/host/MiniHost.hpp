@@ -193,6 +193,12 @@ class MiniHost {
   // instead of on the host (createCombinedMeasurement + createConstraints).  Same edges and warnings; off by default.
   void setDevicePatches(bool on) { mDevicePatches = on; }
   const Transform& correctedPose(unsigned v) const { return mCorrected[v]; }
+  // every vertex with its corrected pose, in vertex order: the list a slam3d application hands to PointCloudSensor::buildMap
+  PointCloudSensor::PosedMeasurements vertices() const {
+    PointCloudSensor::PosedMeasurements v;
+    for (size_t i = 0; i < mMeasurements.size(); ++i) v.emplace_back(std::dynamic_pointer_cast<PointCloudMeasurement>(mMeasurements[i]), mCorrected[i]);
+    return v;
+  }
 
   std::vector<RecordedEdge> edges;
   std::vector<std::string> warnings;

@@ -49,7 +49,103 @@ void setPreparedCacheCapacity(size_t capacity) {
 }
 size_t preparedCacheHits() { std::lock_guard<std::mutex> g(g_cache_mutex); return g_cache_hits; }
 
-static s3d_cloud asCloud(const PointCloud::Ptr& c);
+static s3d_cloud asCloud(const PointCloud::Ptr& c) {
+  s3d_cloud o;
+  o.xyzw = c && c->size() ? &c->points[0].x : nullptr;
+  o.n = c ? c->size() : 0;
+  return o;
+}
+
+namespace {
+struct Resident {
+  s3d_resident_scan* h = nullptr;
+  ~Resident() { if (h) s3d_release_scan(defaultContext(), h); }
+};
+struct StoreEntry { const PointCloud* key; std::weak_ptr<PointCloud> alive; size_t bytes; std::shared_ptr<Resident> scan; };
+std::mutex g_store_mutex;
+std::list<StoreEntry> g_store;  // front = most recently used
+size_t g_store_budget = 0, g_store_bytes = 0;
+uint64_t g_store_uploads = 0, g_store_hits = 0;
+
+// under g_store_mutex: entries whose measurement is gone, then least-recently-used ones while the bytes exceed the budget.  A call
+// that still holds an evicted scan keeps it until the call ends.
+void storeTrim() {
+  for (auto it = g_store.begin(); it != g_store.end();) {
+    if (it->alive.expired()) { g_store_bytes -= it->bytes; it = g_store.erase(it); } else ++it;
+  }
+  while (g_store_bytes > g_store_budget) { g_store_bytes -= g_store.back().bytes; g_store.pop_back(); }
+}
+
+// The clouds one call reads, as device views of stored scans where the store holds (or now takes) them; host clouds otherwise.
+// The misses of the call are uploaded together, once each.  `hold` keeps the scans of the views alive until the call is done.
+struct Views {
+  std::vector<s3d_cloud> clouds;
+  std::vector<std::shared_ptr<Resident>> hold;
+};
+Views residentViews(const std::vector<PointCloud::Ptr>& clouds) {
+  Views v;
+  v.hold.resize(clouds.size());
+  for (const PointCloud::Ptr& c : clouds) v.clouds.push_back(asCloud(c));
+  std::map<const PointCloud*, size_t> miss;  // cloud -> index of its first occurrence in `clouds`
+  {
+    std::lock_guard<std::mutex> g(g_store_mutex);
+    if (g_store_budget == 0) return v;
+    storeTrim();
+    for (size_t i = 0; i < clouds.size(); ++i) {
+      const size_t bytes = 16 * size_t(v.clouds[i].n);
+      if (bytes == 0 || bytes > g_store_budget || miss.count(clouds[i].get())) continue;
+      auto it = g_store.begin();
+      while (it != g_store.end() && it->key != clouds[i].get()) ++it;
+      if (it == g_store.end()) { miss.emplace(clouds[i].get(), i); continue; }
+      ++g_store_hits;
+      g_store.splice(g_store.begin(), g_store, it);
+      v.hold[i] = it->scan;
+    }
+  }
+  if (!miss.empty()) {
+    std::vector<s3d_cloud> up;
+    for (const auto& m : miss) up.push_back(v.clouds[m.second]);
+    std::vector<s3d_resident_scan*> h(up.size(), nullptr);
+    if (s3d_upload_scans(defaultContext(), 0, up.data(), (int)up.size(), h.data()) != S3D_OK) throw std::runtime_error(s3d_last_error());
+    std::lock_guard<std::mutex> g(g_store_mutex);
+    size_t k = 0;
+    for (const auto& m : miss) {
+      std::shared_ptr<Resident> r(new Resident());
+      r->h = h[k++];
+      v.hold[m.second] = r;
+      ++g_store_uploads;
+      bool stored = false;  // another thread may have stored the same cloud meanwhile
+      for (const StoreEntry& e : g_store) stored = stored || e.key == m.first;
+      if (stored) continue;
+      g_store.push_front({m.first, clouds[m.second], 16 * size_t(up[k - 1].n), r});
+      g_store_bytes += g_store.front().bytes;
+    }
+    storeTrim();
+  }
+  for (size_t i = 0; i < clouds.size(); ++i) {
+    if (!v.hold[i]) {  // a later occurrence of a cloud uploaded by this call
+      auto m = miss.find(clouds[i].get());
+      if (m != miss.end()) v.hold[i] = v.hold[m->second];
+    }
+    if (v.hold[i]) v.clouds[i] = s3d_resident_scan_cloud(v.hold[i]->h);
+  }
+  return v;
+}
+}  // namespace
+
+void setResidentScanBudget(size_t bytes) {
+  std::lock_guard<std::mutex> g(g_store_mutex);
+  g_store_budget = bytes;
+  storeTrim();
+}
+
+ResidentScanStats residentScanStats() {
+  std::lock_guard<std::mutex> g(g_store_mutex);
+  storeTrim();
+  ResidentScanStats s;
+  s.uploads = g_store_uploads; s.hits = g_store_hits; s.bytes_resident = g_store_bytes;
+  return s;
+}
 
 // the prepared form of `cloud` for (density, k) — or, with resolution > 0, its NDT form for (density, resolution): from the
 // cache, or built now and remembered
@@ -67,20 +163,14 @@ static std::shared_ptr<Prepared> prepared(const PointCloud::Ptr& cloud, double d
     }
   }
   std::shared_ptr<Prepared> p(new Prepared());
-  const int st = resolution > 0.f ? s3d_prepare_cloud_ndt(defaultContext(), 0, asCloud(cloud), density, resolution, &p->h)
-                                  : s3d_prepare_cloud(defaultContext(), 0, asCloud(cloud), density, k, &p->h);
+  const Views v = residentViews({cloud});
+  const int st = resolution > 0.f ? s3d_prepare_cloud_ndt(defaultContext(), 0, v.clouds[0], density, resolution, &p->h)
+                                  : s3d_prepare_cloud(defaultContext(), 0, v.clouds[0], density, k, &p->h);
   if (st != S3D_OK) throw std::runtime_error(s3d_last_error());
   std::lock_guard<std::mutex> g(g_cache_mutex);
   g_cache.push_front({cloud.get(), cloud, density, k, resolution, p});
   while (g_cache.size() > g_cache_capacity) g_cache.pop_back();
   return p;
-}
-
-static s3d_cloud asCloud(const PointCloud::Ptr& c) {
-  s3d_cloud o;
-  o.xyzw = c && c->size() ? &c->points[0].x : nullptr;
-  o.n = c ? c->size() : 0;
-  return o;
 }
 
 // :119-174
@@ -101,7 +191,8 @@ Transform align(PointCloudMeasurement::Ptr source, PointCloudMeasurement::Ptr ta
     std::shared_ptr<Prepared> pt = prepared(target->getPointCloud(), config.point_cloud_density, 0, config.resolution);
     st = s3d_gicp_align_prepared(defaultContext(), ps->h, pt->h, guess.data(), &c, &res);
   } else {
-    st = s3d_gicp_align(defaultContext(), asCloud(source->getPointCloud()), asCloud(target->getPointCloud()), guess.data(), &c, &res);
+    const Views v = residentViews({source->getPointCloud(), target->getPointCloud()});
+    st = s3d_gicp_align(defaultContext(), v.clouds[0], v.clouds[1], guess.data(), &c, &res);
   }
   if (result_info) *result_info = res;
   switch (st) {
@@ -183,21 +274,29 @@ void PointCloudSensor::fillGroundPlane(PointCloud::Ptr cloud, ScalarType radius)
 
 // :235-256  (pose = vertex.correctedPose * measurement.sensorPose, accumulated in list order)
 PointCloud::Ptr PointCloudSensor::getAccumulatedCloud(const PosedMeasurements& vertices) const {
+  std::vector<PointCloud::Ptr> clouds;
+  for (const auto& v : vertices) clouds.push_back(v.first->getPointCloud());
+  const Views views = residentViews(clouds);
   PointCloud::Ptr accu(new PointCloud);
-  for (size_t i = 0; i < vertices.size(); ++i) {
-    PointCloud::Ptr t = transform(vertices[i].first->getPointCloud(), vertices[i].second * vertices[i].first->getSensorPose());
-    accu->points.insert(accu->points.end(), t->points.begin(), t->points.end());
+  for (size_t i = 0; i < vertices.size(); ++i) {  // transform(cloud_i, pose_i) of every vertex, appended
+    const size_t at = accu->size();
+    accu->points.resize(at + views.clouds[i].n);
+    const Transform tf = vertices[i].second * vertices[i].first->getSensorPose();
+    if (views.clouds[i].n && s3d_transform_cloud(defaultContext(), views.clouds[i], tf.data(), &accu->points[at].x) != S3D_OK)
+      throw std::runtime_error(s3d_last_error());
   }
   return accu;
 }
 
 // :258-266  one device pass: transform(cloud_i, pose_i) appended in list order, then transformPointCloud(pose.inverse())
 Measurement::Ptr PointCloudSensor::createCombinedMeasurement(const PosedMeasurements& vertices, Transform pose) const {
-  std::vector<s3d_cloud> clouds(vertices.size());
+  std::vector<PointCloud::Ptr> scans;
+  for (const auto& v : vertices) scans.push_back(v.first->getPointCloud());
+  const Views views = residentViews(scans);
+  const std::vector<s3d_cloud>& clouds = views.clouds;
   std::vector<double> poses(16 * vertices.size());
   size_t total = 0;
   for (size_t i = 0; i < vertices.size(); ++i) {
-    clouds[i] = asCloud(vertices[i].first->getPointCloud());
     const Transform p = vertices[i].second * vertices[i].first->getSensorPose();  // :248
     for (int j = 0; j < 16; ++j) poses[16 * i + j] = p.m[j];
     total += clouds[i].n;
@@ -216,11 +315,13 @@ Measurement::Ptr PointCloudSensor::createCombinedMeasurement(const PosedMeasurem
 // :301-318  one device pass: accumulate -> removeOutliers -> downsample
 PointCloud::Ptr PointCloudSensor::buildMap(const PosedMeasurements& vertices) const {
   PointCloud::Ptr map(new PointCloud);
-  std::vector<s3d_cloud> clouds(vertices.size());
+  std::vector<PointCloud::Ptr> scans;
+  for (const auto& v : vertices) scans.push_back(v.first->getPointCloud());
+  const Views views = residentViews(scans);
+  const std::vector<s3d_cloud>& clouds = views.clouds;
   std::vector<double> poses(16 * vertices.size());
   size_t total = 0;
   for (size_t i = 0; i < vertices.size(); ++i) {
-    clouds[i] = asCloud(vertices[i].first->getPointCloud());
     const Transform p = vertices[i].second * vertices[i].first->getSensorPose();
     for (int j = 0; j < 16; ++j) poses[16 * i + j] = p.m[j];
     total += clouds[i].n;
@@ -269,7 +370,7 @@ static void failureOf(int st, const s3d_result& r, const RegistrationParameters&
 std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createConstraints(const std::vector<ConstraintRequest>& requests, bool loop) {
   std::vector<ConstraintResult> out(requests.size());
   std::vector<size_t> idx;
-  std::vector<s3d_cloud> src, tgt;
+  std::vector<PointCloud::Ptr> clouds;  // source, target of each request that reaches the batch
   std::vector<double> guesses;
   for (size_t i = 0; i < requests.size(); ++i) {
     PointCloudMeasurement::Ptr sc = std::dynamic_pointer_cast<PointCloudMeasurement>(requests[i].source);
@@ -280,11 +381,14 @@ std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createConstrai
       continue;
     }
     const Transform guess = requests[i].source->getInverseSensorPose() * requests[i].odometry * requests[i].target->getSensorPose();  // :274
-    idx.push_back(i); src.push_back(asCloud(sc->getPointCloud())); tgt.push_back(asCloud(tc->getPointCloud()));
+    idx.push_back(i); clouds.push_back(sc->getPointCloud()); clouds.push_back(tc->getPointCloud());
     guesses.insert(guesses.end(), guess.m.begin(), guess.m.end());
   }
   const int n = (int)idx.size();
   if (n == 0) return out;
+  const Views views = residentViews(clouds);
+  std::vector<s3d_cloud> src, tgt;
+  for (int k = 0; k < n; ++k) { src.push_back(views.clouds[2 * k]); tgt.push_back(views.clouds[2 * k + 1]); }
   std::vector<s3d_result> coarse(n), fine(n);
   const s3d_registration_parameters cc = mCoarseConfiguration.toC(), cf = mFineConfiguration.toC();
   const int st = loop ? s3d_gicp_align_loop_batch(defaultContext(), src.data(), tgt.data(), guesses.data(), &cc, &cf, n, coarse.data(), fine.data())  // :286-292
@@ -333,7 +437,7 @@ std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createLoopCons
     return createConstraints(req, true);
   }
   // distinct scans by cloud object, distinct patches by (member scans, member poses, patch pose) as bit patterns
-  std::vector<s3d_cloud> scans;
+  std::vector<PointCloud::Ptr> scans;
   std::map<const PointCloud*, int32_t> scan_of;
   std::vector<int32_t> member_scan, first{0};
   std::vector<double> member_poses, patch_poses;
@@ -350,7 +454,7 @@ std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createLoopCons
     for (const auto& v : p.vertices) {
       const PointCloud::Ptr& c = v.first->getPointCloud();
       auto it = scan_of.find(c.get());
-      if (it == scan_of.end()) { it = scan_of.emplace(c.get(), (int32_t)scans.size()).first; scans.push_back(asCloud(c)); }
+      if (it == scan_of.end()) { it = scan_of.emplace(c.get(), (int32_t)scans.size()).first; scans.push_back(c); }
       mp.push_back(v.second * v.first->getSensorPose());  // :248
       ms.push_back(it->second);
       key.push_back((uint64_t)it->second);
@@ -380,7 +484,8 @@ std::vector<PointCloudSensor::ConstraintResult> PointCloudSensor::createLoopCons
     ~Handles() { for (s3d_prepared_cloud* p : h) s3d_release_cloud(defaultContext(), p); }
   } hh;
   hh.h.assign((size_t)n_patches * ns, nullptr);
-  if (s3d_prepare_combined_measurements(defaultContext(), 0, scans.data(), (int)scans.size(), member_scan.data(), member_poses.data(), first.data(),
+  const Views views = residentViews(scans);
+  if (s3d_prepare_combined_measurements(defaultContext(), 0, views.clouds.data(), (int)scans.size(), member_scan.data(), member_poses.data(), first.data(),
                                         patch_poses.data(), n_patches, specs.data(), ns, hh.h.data()) != S3D_OK)
     throw std::runtime_error(s3d_last_error());
   // a patch's sensor pose is the identity (createCombinedMeasurement :265); the guess and the edge are formed as createConstraint

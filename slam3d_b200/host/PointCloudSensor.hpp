@@ -33,6 +33,17 @@ s3d_context* defaultContext();
 void setPreparedCacheCapacity(size_t capacity);
 size_t preparedCacheHits();
 
+// Resident scans (optional, off by default).  With a budget > 0 the cloud of a PointCloudMeasurement is uploaded once, on its first
+// use, with s3d_upload_scans, and every later call that reads it (align() on the raw path and on prepared-cache misses,
+// createConstraints, createLoopConstraints, getAccumulatedCloud, createCombinedMeasurement, buildMap) passes the device view instead
+// of uploading it again.  Results are bit for bit those of the host clouds.  Free-standing clouds (the arguments of downsample,
+// downsampleScan, transform, removeOutliers, fillGroundPlane) are never stored.  Keyed by the cloud object like the prepared cache;
+// an entry is released when its measurement is gone, and least-recently-used entries are released while the stored bytes exceed
+// the budget.  A cloud larger than the budget is not stored.  Budget 0 releases every entry and reads host clouds again.
+void setResidentScanBudget(size_t bytes);
+struct ResidentScanStats { uint64_t uploads = 0, hits = 0, bytes_resident = 0; };  // scans uploaded, lookups served, 16 B per stored point
+ResidentScanStats residentScanStats();
+
 // align(source, target, guess, config) — PointCloudSensor.cpp:119-174.  Throws NoMatch / std::runtime_error exactly
 // where the reference does.  `result_info` (optional) receives the C-ABI result (fitness, iterations...).
 Transform align(PointCloudMeasurement::Ptr source, PointCloudMeasurement::Ptr target, const Transform& guess,

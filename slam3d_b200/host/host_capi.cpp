@@ -37,6 +37,11 @@ const char* s3dhost_last_message() { return g_msg.c_str(); }
 void* s3dhost_context() { return defaultContext(); }
 void s3dhost_set_cache_capacity(uint64_t n) { setPreparedCacheCapacity((size_t)n); }
 uint64_t s3dhost_cache_hits() { return (uint64_t)preparedCacheHits(); }
+void s3dhost_set_resident_budget(uint64_t bytes) { setResidentScanBudget((size_t)bytes); }
+void s3dhost_resident_stats(uint64_t* uploads, uint64_t* hits, uint64_t* bytes_resident) {
+  const ResidentScanStats s = residentScanStats();
+  *uploads = s.uploads; *hits = s.hits; *bytes_resident = s.bytes_resident;
+}
 
 void* s3dhost_sensor_create(const char* name) { return new PointCloudSensor(name, nullptr); }
 void s3dhost_sensor_destroy(void* s) { delete static_cast<PointCloudSensor*>(s); }
@@ -128,15 +133,29 @@ int s3dhost_run_odometry(void* s, const float* const* scans, const uint64_t* siz
 static double g_link_seconds = 0;
 static int g_link_calls = 0;
 void s3dhost_link_stats(double* seconds, int* calls) { *seconds = g_link_seconds; *calls = g_link_calls; }
+// seconds spent in the periodic buildMap calls of the last trajectory run, and their number
+static double g_map_seconds = 0;
+static int g_map_calls = 0;
+void s3dhost_map_stats(double* seconds, int* calls) { *seconds = g_map_seconds; *calls = g_map_calls; }
+
+// FNV-1a over the bytes of a map: tells maps apart without copying them out
+static uint64_t mapHash(const PointCloud& map) {
+  uint64_t h = 1469598103934665603ull;
+  const unsigned char* p = map.size() ? reinterpret_cast<const unsigned char*>(&map.points[0].x) : nullptr;
+  for (size_t i = 0; i < 16 * map.size(); ++i) { h ^= p[i]; h *= 1099511628211ull; }
+  return h;
+}
 
 // BASELINE configs[4] (trajectory): n scans through addMeasurement(m, odom) + linkLastToNeighbors() after every new vertex.
 // edges_out: per recorded edge {source, target, loop} as 3 ints followed by nothing; T_out: 16 doubles per edge (relative pose);
 // poses_out: n x 16 doubles (corrected poses).  Returns the number of edges (<= max_edges) or -1.
 static int run_trajectory(void* s, const float* const* scans, const uint64_t* sizes, int n, const double* odoms, double neighbor_radius,
                           int max_links, int min_loop_length, int patch_range, int batched, int max_edges, int* edges_out, double* T_out,
-                          double* poses_out, int* n_warnings) {
+                          double* poses_out, int* n_warnings, int map_every = 0, int max_maps = 0, uint64_t* map_sizes = nullptr,
+                          uint64_t* map_hashes = nullptr) {
   PointCloudSensor* sensor = static_cast<PointCloudSensor*>(s);
   try {
+    g_map_seconds = 0; g_map_calls = 0;
     MiniHost host(sensor);
     host.setNeighborRadius((float)neighbor_radius, max_links);
     host.setMinLoopLength((unsigned)min_loop_length);
@@ -152,6 +171,13 @@ static int run_trajectory(void* s, const float* const* scans, const uint64_t* si
       if (host.edges.size() + host.warnings.size() != seen) {
         g_link_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
         ++g_link_calls;
+      }
+      if (map_every > 0 && host.vertices().size() % (size_t)map_every == 0) {  // the application's periodic map over the whole graph
+        const auto m0 = std::chrono::steady_clock::now();
+        const PointCloud::Ptr map = sensor->buildMap(host.vertices());
+        g_map_seconds += std::chrono::duration<double>(std::chrono::steady_clock::now() - m0).count();
+        if (g_map_calls < max_maps) { map_sizes[g_map_calls] = map->size(); map_hashes[g_map_calls] = mapHash(*map); }
+        ++g_map_calls;
       }
     }
     const int ne = (int)std::min<size_t>(host.edges.size(), (size_t)max_edges);
@@ -181,6 +207,16 @@ int s3dhost_run_trajectory2(void* s, const float* const* scans, const uint64_t* 
                             int max_links, int min_loop_length, int patch_range, int batched, int max_edges, int* edges_out, double* T_out,
                             double* poses_out, int* n_warnings) {
   return run_trajectory(s, scans, sizes, n, odoms, neighbor_radius, max_links, min_loop_length, patch_range, batched, max_edges, edges_out, T_out, poses_out, n_warnings);
+}
+
+// the same, and every `map_every` vertices (0: never) PointCloudSensor::buildMap over all vertices with their corrected poses, as a
+// slam3d application refreshes its map while the graph grows.  map_sizes / map_hashes receive the size and an FNV-1a hash of the
+// first max_maps maps; s3dhost_map_stats gives their number and time.
+int s3dhost_run_trajectory_maps(void* s, const float* const* scans, const uint64_t* sizes, int n, const double* odoms, double neighbor_radius,
+                                int max_links, int min_loop_length, int patch_range, int batched, int map_every, int max_maps, uint64_t* map_sizes,
+                                uint64_t* map_hashes, int max_edges, int* edges_out, double* T_out, double* poses_out, int* n_warnings) {
+  return run_trajectory(s, scans, sizes, n, odoms, neighbor_radius, max_links, min_loop_length, patch_range, batched, max_edges, edges_out, T_out,
+                        poses_out, n_warnings, map_every, max_maps, map_sizes, map_hashes);
 }
 
 // ScanSensor::addMeasurement(m) without odometry (core/ScanSensor.cpp:49-79): the guess is chained from the previous result and
